@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the render hot path (BASELINE.json metric: audio-seconds rendered per second).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config {1,2,3,4,5}] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config {1,2,3,4,5}] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workloads = BASELINE.json `configs` with the shapes and ranges of SURVEY 8(d):
@@ -389,6 +389,23 @@ def bit_checksum(torch, t):
     return int(t.contiguous().view(torch.int32).to(torch.int64).sum().item())
 
 
+DUMP_BYTES = 32 << 20       # --dump-outputs: above this, a sample of rows (a config-4 step returns 4.3 GB)
+
+
+def dump_outputs(path, outputs):
+    """--dump-outputs: each batch-first tensor of `outputs` as <path>/<name>.npy in float32.  All rows when the outputs
+    fit in DUMP_BYTES together, else the same rows of each: sorted(RandomState(0).choice(B, k, replace=False))."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    B = len(next(iter(outputs.values())))
+    row_bytes = sum(t[0].numel() * 4 for t in outputs.values())
+    k = min(B, max(1, DUMP_BYTES // row_bytes))
+    rows = np.sort(np.random.RandomState(0).choice(B, k, replace=False))
+    for name, t in outputs.items():
+        sample = t.index_select(0, torch.from_numpy(rows).to(t.device))
+        np.save(os.path.join(path, name + ".npy"), sample.float().cpu().numpy())
+
+
 # --------------------------------------------------------------------------------------------- config 4
 
 def make_batch4(cx, R, Bg, seed, lo, hi):
@@ -493,6 +510,8 @@ def run_config4(cx, args):
     step = step_of(wb)
     sampler = ClockSampler(cx.local_rank) if rank == 0 else None
     ms_per_step, clocks = cx.timed(step, args.steps, args.warmup, sampler)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"wet": wb["wet"], "logmel": wb["logmel"]})
     value = world * B * (N / SR) / (ms_per_step * 1e-3)
     checksum = float(wb["wet"].double().abs().mean().item())
     # algorithmic bytes of the step: dry audio read once (a phaser example up to the end of its window: start + N
@@ -825,6 +844,9 @@ def run_small_configs(cx, args):
         dominant = ("flanger", f_fl, B * n * 8)
     sampler = ClockSampler(cx.local_rank) if rank == 0 else None
     ms_per_step, clocks = cx.timed(step, args.steps, args.warmup, sampler)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("dry", "wet", "mod_sig"), holder["out"][:3])) if cfg == 2 else
+                     {"wet": out})
     value = audio_s / (ms_per_step * 1e-3)
     dname, dfn, dbytes = dominant
     kernels[dname] = {"ms": cx.kernel_ms(dfn, 3 if cfg == 5 else 10), "algorithmic_bytes": dbytes}
@@ -870,7 +892,14 @@ def main():
     ap.add_argument("--no-e2e-full", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true", help="do not pin the process to the GPU-local CPUs")
     ap.add_argument("--e2e-chunk", type=int, default=512, help="examples per pipelined chunk of the host-buffer path")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float32; a fixed sample of rows when "
+                         "the outputs exceed 32 MiB), rank 0's rows, to compare two builds on the same inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; --impl reference has none")
     args.warmup = max(args.warmup, 3)
 
     rank = env_int("RANK", 0)
