@@ -256,7 +256,7 @@ int modfx_phaser_f32(const float* x, float* y, int32_t B, int64_t N, float sr, c
  * proc_n = n_out + round(sr / rate_hz[b]) samples ("one extra LFO period", rows padded to the common pitch N); the
  * phaser runs over the row from its first sample and the window [start[b], start[b] + n_out) of the wet signal AND of
  * the dry input is delivered (datasets.py:445-447): y (B, n_out), dry_out (B, n_out) or NULL.  Samples past the window
- * are never processed (the effect is causal).  Needs a host block size that is a multiple of 128 samples.
+ * are never processed (the effect is causal).
  * With an example_index list and x_compact = 1, x is a compact (n_items, N) array whose row i belongs to example
  * example_index[i] (every other array stays indexed by the example id): an interleaved batch keeps the long phaser
  * rows apart from its (B, n_out) dry / wet tensors, into which y / dry_out may point.

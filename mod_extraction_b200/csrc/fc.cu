@@ -4,35 +4,26 @@
 // python loop costs ~105 us per time step.  Bit-exact with it: every float32 operation of the
 // reference is one IEEE-RN operation here (explicit __f*_rn intrinsics, never contracted).
 //
-// Three kernels share the per-sample arithmetic (=> the same bits): fc_cta_kernel (default: a CTA of three producer
-// warps + one consumer warp per delay line), fc_wide_kernel (a CTA per delay line whose every tap lies more than 384
-// samples back: the chorus) and fc_kernel (one warp per delay line: the first schedule, kept as the cross-check);
-// fc_allpass_kernel is the all-pass interpolation mode.
+// Two kernels share the per-sample arithmetic (=> the same bits): fc_cta_kernel (default: a CTA of three producer
+// warps + one consumer warp per delay line, for every modulation source) and fc_wide_kernel (a CTA per delay line
+// whose every tap lies more than 384 samples back: the chorus); fc_allpass_kernel is the all-pass interpolation mode.
 //
 // Parallelisation (DESIGN.md "E1"): the recurrence v[n] = x[n] + fb*interp(v[n-kp], v[n-kq]) is
 // sequential in time per delay line, but a sample only depends on samples at least
-// `near = min(kp,kq)` steps back.  In fc_kernel one warp owns one delay line (example x channel); the written
-// values v live in a shared-memory ring indexed by time.  A tile of 128 samples (4 per lane) is
-// rendered in one shot when every dependency falls before the tile (always true for chorus,
-// true for flanger while the delay exceeds 128 samples); otherwise 32-sample blocks are resolved
-// as "waves" of independent prefixes, and stretches with a 1-2 sample delay fall back to a
-// lock-step serial loop with register forwarding.  Only the schedule changes, never the
+// `near = min(kp,kq)` steps back.  The written values v live in a shared-memory ring indexed by time.
+// A tile of 128 samples is rendered in one shot when every dependency falls before the tile (always
+// true for chorus, true for flanger while the delay exceeds 128 samples); otherwise 32-sample blocks
+// are resolved as "waves" of independent prefixes, and stretches with a delay of a few samples fall
+// back to a lock-step serial loop with register forwarding.  Only the schedule changes, never the
 // arithmetic of a sample, so the result is identical in all modes.
 #include "common.cuh"
-
-#include <stdlib.h>
 
 namespace modfx {
 namespace {
 
 constexpr int kTile = 128;          // samples per tile (4 sub-steps x 32 lanes)
 constexpr int kSub = kTile / kWarp; // 4
-constexpr int kLoWin = 512;         // control-rate LFO points staged in shared memory at a time
-constexpr int kStages = 8;          // dry-audio tiles in flight per warp (cp.async ring)
-#ifndef MODFX_FC_POLL_NS
-#define MODFX_FC_POLL_NS 128   // producers polling for the consumer: 32 / 100 / 300 ns measured within noise of each other (1.17-1.26 ms), longer leaves more issue slots
-#endif
-constexpr int kSerialMaxK = 7;      // register-history serial run covers tap distances up to this (+1)
+constexpr int kPollNs = 128;        // producers polling for the consumer: 32 / 100 / 300 ns measured within noise of each other (1.17-1.26 ms), longer leaves more issue slots
 
 struct FcArgs {
     const float* x;
@@ -59,7 +50,6 @@ struct FcArgs {
     const int32_t* index;
     int n_items;
     int wide;                       // 1: examples that qualify for fc_wide_kernel are rendered there and skipped here
-    long long* stats;               // MODFX_FC_STATS builds only: per-CTA schedule counters of fc_cta_kernel
 };
 
 enum ModMode { kAudioRate = 0, kControlRate = 1, kDirectLfo = 2 };
@@ -105,9 +95,6 @@ __device__ __forceinline__ void fc_sample(const Samp& s, float vp, float vq, con
 // ---- cp.async staging of the dry audio (and the audio-rate mod_sig) ---------------------
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 
-__device__ __forceinline__ void cp_async_16(void* dst, const void* src, int src_bytes) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(smem_u32(dst)), "l"(src), "r"(src_bytes));
-}
 __device__ __forceinline__ void cp_async_4(void* dst, const void* src, int src_bytes) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;\n" ::"r"(smem_u32(dst)), "l"(src), "r"(src_bytes));
 }
@@ -115,60 +102,14 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
 
-// Stage samples [n0, n0 + kTile) of `row` into `dst` (zero-filled past N).
-__device__ __forceinline__ void stage_tile(float* dst, const float* row, int n0, int N, int lane, bool vec16) {
-    if (n0 >= N) return;
-    if (vec16) {
-        const int n = n0 + 4 * lane;
-        if (n < N) cp_async_16(dst + 4 * lane, row + n, min(16, (N - n) * 4));
-        else *reinterpret_cast<float4*>(dst + 4 * lane) = make_float4(0.f, 0.f, 0.f, 0.f);
-    } else {
-#pragma unroll
-        for (int k = 0; k < kSub; ++k) {
-            const int n = n0 + k * kWarp + lane;
-            if (n < N) cp_async_4(dst + k * kWarp + lane, row + n, 4);
-            else dst[k * kWarp + lane] = 0.0f;
-        }
-    }
-}
-
-// ---- lock-step serial run over one full 32-sample block whose tap distances are all K or K+1 -------
-// Delays of a few samples make the recurrence truly serial: 4 dependent float ops per sample.  Every
-// lane executes the same code (no divergence): per sample one 16-byte broadcast read of the
-// pre-computed {x, fraction, 1-fraction, stale tap}, a 2-way select between history REGISTERS (the taps
-// are among the last K+1 values, so they never travel through shared memory on the critical path),
-// the 4 float ops of fx.py:113-114, and two stores (ring + interpolated value for the per-lane epilogue).
-template <int K>
-__device__ __noinline__ void serial_block(float* __restrict__ ring, int mask, int nb, const float4* __restrict__ coef,
-                                          unsigned sel_mask, float fb, float* __restrict__ it_out) {
-    float h[K + 2];
-#pragma unroll
-    for (int j = 1; j <= K + 1; ++j) h[j] = ring[(nb - j) & mask];
-    float* dst = ring + (nb & mask);            // blocks are 32-aligned and the ring is a multiple of 32: no wrap inside
-#pragma unroll
-    for (int i = 0; i < kWarp; ++i) {
-        const float4 cf = coef[i];
-        const bool sel = (sel_mask >> i) & 1u;  // tap p at distance K (else K+1)
-        const float vp = sel ? h[K] : h[K + 1];
-        const float vq = sel ? ((K == 1) ? cf.w : h[K - 1]) : h[K];
-        const float it = __fadd_rn(__fmul_rn(cf.y, vq), __fmul_rn(cf.z, vp));       // fx.py:113
-        const float v = __fadd_rn(cf.x, __fmul_rn(fb, it));                           // fx.py:114
-        dst[i] = v;
-        it_out[i] = it;
-#pragma unroll
-        for (int j = K + 1; j >= 2; --j) h[j] = h[j - 1];
-        h[1] = v;
-    }
-}
-
 // ---- wide path: delay lines whose every tap lies more than a tile back (chorus) ------------------------------
 // With a minimum delay of D0 = min_delay_width * Mmin samples (485 for the reference's chorus) a sample never depends on
-// the previous kWideTile samples, so a whole CTA can render 384 samples of ONE delay line at a time -- four times the
-// warps per example of the one-warp kernel, which at 1365 examples leaves an SM with 9 warps.  Same per-sample
-// arithmetic (the branch-free form of fx.py:95-118 used by the one-warp kernel's fast path), so the bits are identical.
+// the previous kWideTile samples, so a whole CTA can render 384 samples of ONE delay line at a time, with one barrier
+// per tile and no producer / consumer hand-off.  Same per-sample arithmetic (the branch-free form of fx.py:95-118 used
+// by fc_cta_kernel's producers), so the bits are identical.
 // Whether an example qualifies is decided from its parameters and the extremes of its control-rate row by
-// wide_pred(), evaluated identically by both kernels: the wide kernel renders the example iff it holds, the one-warp
-// kernel iff it does not.
+// wide_pred(), evaluated identically by both kernels: the wide kernel renders the example iff it holds, fc_cta_kernel
+// iff it does not.
 constexpr int kWideThreads = 128;
 constexpr int kWideSub = 3;
 constexpr int kWideTile = kWideThreads * kWideSub;      // 384
@@ -227,7 +168,7 @@ __global__ void __launch_bounds__(kWideThreads) fc_wide_kernel(const FcArgs a, i
     mn = red[0][0]; mx = red[1][0];
 #pragma unroll
     for (int w = 1; w < kWideThreads / kWarp; ++w) { mn = fminf(mn, red[0][w]); mx = fmaxf(mx, red[1][w]); }
-    if (!wide_pred(c, mn, mx)) return;                      // left to the one-warp kernel (CTA-uniform)
+    if (!wide_pred(c, mn, mx)) return;                      // left to fc_cta_kernel (CTA-uniform)
 
     const float* xs = a.x + ((int64_t)b * a.C + ch) * (int64_t)N;
     float* ys = a.y + ((int64_t)b * a.C + ch) * (int64_t)N;
@@ -286,291 +227,8 @@ __global__ void __launch_bounds__(kWideThreads) fc_wide_kernel(const FcArgs a, i
     }
 }
 
-template <int MODE>
-__global__ void __launch_bounds__(kWarp) fc_kernel(const FcArgs a) {
-    extern __shared__ __align__(16) float smem[];
-    const int lane = threadIdx.x;
-    const int item = blockIdx.x / a.C;
-    const int ch = blockIdx.x - item * a.C;
-    const int b = a.index ? a.index[item] : item;
-    const int N = a.N;
-
-    // shared memory: [x stages][serial scratch][mod stages (audio-rate) | LFO window (control-rate)][ring]
-    float* xst = smem;
-    float4* coef = reinterpret_cast<float4*>(smem + kStages * kTile);       // 32 x {x, fr, omfr, stale}
-    float* itbuf = smem + kStages * kTile + 4 * kWarp;                      // 32 interpolated values
-    float* mst = itbuf + kWarp;
-    float* lo = mst;
-    float* ring = mst + ((MODE == kAudioRate) ? kStages * kTile : ((MODE == kControlRate) ? (kLoWin + 4) : 0));
-
-    Coef c = make_coef(a, b);
-    if (MODE == kControlRate && a.wide) {
-        // examples whose every tap lies more than a wide tile back were rendered by fc_wide_kernel (same predicate)
-        const float* row = a.mod + (int64_t)b * a.n_lo;
-        float mn = INFINITY, mx = -INFINITY;
-        for (int i = lane; i < a.n_lo; i += kWarp) {
-            const float v = __ldg(row + i);
-            mn = fminf(mn, v);
-            mx = fmaxf(mx, v);
-            if (!(v == v)) mx = INFINITY;
-        }
-        warp_minmax(mn, mx);
-        if (wide_pred(c, mn, mx)) return;
-    }
-    // With 0 <= mod <= 1 and these bounds the delay stays in [0, M], so (w - d) + M lies in [0, 2M) and
-    // the reference's remainder is a single conditional subtraction (exact by Sterbenz).
-    const bool coef_ok = (c.A >= 0.0f) && (c.D0 >= 0.0f) && (__fadd_rn(c.A, c.D0) <= c.Mf) && (a.M >= kTile);
-
-    const float* xs = a.x + ((int64_t)b * a.C + ch) * (int64_t)N;
-    float* ys = a.y + ((int64_t)b * a.C + ch) * (int64_t)N;
-    const float* ms = nullptr;
-    if (MODE == kAudioRate) ms = a.mod + (a.mod_has_ch ? ((int64_t)b * a.C + ch) : (int64_t)b) * (int64_t)N;
-    const bool xvec = (((uintptr_t)xs) & 15) == 0;
-    const bool mvec = (MODE == kAudioRate) && ((((uintptr_t)ms) & 15) == 0);
-
-    // prologue of the copy pipeline: tiles 0 .. kStages-2
-#pragma unroll
-    for (int t = 0; t < kStages - 1; ++t) {
-        stage_tile(xst + t * kTile, xs, t * kTile, N, lane, xvec);
-        if (MODE == kAudioRate) stage_tile(mst + t * kTile, ms, t * kTile, N, lane, mvec);
-        cp_async_commit();
-    }
-
-    for (int i = lane; i <= a.ring_mask; i += kWarp) ring[i] = 0.0f;                // fx.py:92
-
-    LfoDesc lfo;
-    if (MODE == kDirectLfo || (MODE == kControlRate && a.lfo_freq)) {
-        lfo = make_lfo_desc(a.lfo_freq[b], a.lfo_phase[b], a.lfo_shape[b],
-                            a.lfo_exp ? a.lfo_exp[b] : 1.0f, a.sr_lo);
-    }
-    int lo_base = 0, lo_end = 0;    // control points [lo_base, lo_end) are staged in lo[] (+1 duplicate at the end)
-    bool lo_ok = true;              // every staged control point lies in [0, 1]
-    __syncwarp();
-
-    int wk[kSub];                   // (n mod M) of this lane's sample in each 32-sample block of the tile
-#pragma unroll
-    for (int k = 0; k < kSub; ++k) wk[k] = (k * kWarp + lane) % c.M;
-    int stage = 0;                  // tile index mod kStages
-    for (int n0 = 0; n0 < N; n0 += kTile) {
-        {   // keep kStages-1 tiles of dry audio in flight
-            int ps = stage + kStages - 1;
-            if (ps >= kStages) ps -= kStages;
-            const int pn = n0 + (kStages - 1) * kTile;
-            stage_tile(xst + ps * kTile, xs, pn, N, lane, xvec);
-            if (MODE == kAudioRate) stage_tile(mst + ps * kTile, ms, pn, N, lane, mvec);
-            cp_async_commit();
-        }
-        if (MODE == kControlRate) {
-            // Slide the staged window of the control-rate LFO (882 points per 2 s clip in the
-            // reference pipeline) so that it covers every tap this tile interpolates from.
-            const int last_n = min(n0 + kTile - 1, N - 1);
-            const int need_hi = min((int)__fmul_rn(a.up_scale, (float)last_n) + 1, a.n_lo - 1);
-            if (need_hi >= lo_end) {
-                __syncwarp();
-                lo_base = min((int)__fmul_rn(a.up_scale, (float)n0), a.n_lo - 1);
-                lo_end = min(lo_base + kLoWin, a.n_lo);
-                bool ok = true;
-                // one extra slot duplicates the last point so that tap i0+1 needs no clamp
-                for (int i = lo_base + lane; i <= lo_end; i += kWarp) {
-                    const int ii = min(i, a.n_lo - 1);
-                    const float v = a.lfo_freq ? lfo_value(lfo, ii) : a.mod[(int64_t)b * a.n_lo + ii];
-                    lo[i - lo_base] = v;
-                    ok = ok && (v >= 0.0f) && (v <= 1.0f);
-                }
-                lo_ok = __all_sync(kFull, ok);
-            }
-        }
-        cp_async_wait<kStages - 1>();       // this tile's copies (issued kStages-1 tiles ago) landed
-        __syncwarp();
-
-        const float* xt = xst + stage * kTile;
-        const float* mt = mst + stage * kTile;
-        Samp s[kSub];
-        bool indep = true;
-        bool fast = coef_ok && (n0 + kTile <= N) && (MODE != kControlRate || lo_ok);
-        if (fast) {
-            // ---- branch-free per-sample arithmetic of fx.py:95-102 (+ the x100 upsample) ----
-            const float* lo_shift = lo - lo_base;
-            bool bad = false;
-#pragma unroll
-            for (int k = 0; k < kSub; ++k) {
-                const int j = k * kWarp + lane;
-                const int n = n0 + j;
-                s[k].x = xt[j];
-                float m;
-                if (MODE == kAudioRate) {
-                    m = mt[j];
-                    bad = bad || !(m >= 0.0f && m <= 1.0f);
-                } else if (MODE == kControlRate) {
-                    const float src = __fmul_rn(a.up_scale, (float)n);
-                    const int i0 = (int)src;
-                    const float l1 = __fsub_rn(src, (float)i0);
-                    const float l0 = __fsub_rn(1.0f, l1);
-                    m = __fmaf_rn(l0, lo_shift[i0], __fmul_rn(l1, lo_shift[i0 + 1]));
-                } else {
-                    m = lfo_value(lfo, n);
-                }
-                const float d = __fadd_rn(__fmul_rn(c.A, m), c.D0);                 // fx.py:98
-                const float t = __fadd_rn(__fsub_rn((float)wk[k], d), c.Mf);        // fx.py:99
-                const float r = (t >= c.Mf) ? __fsub_rn(t, c.Mf) : t;               // % M
-                const float pf = floorf(r);
-                s[k].fr = __fsub_rn(r, pf);                                          // fx.py:100
-                s[k].omfr = __fsub_rn(1.0f, s[k].fr);
-                int kp = wk[k] - (int)pf;                                            // fx.py:101
-                if (kp <= 0) kp += c.M;
-                s[k].kp = kp;
-                indep = indep && (kp >= ((j == 0) ? 1 : j + 2));                     // min(kp,kq) > j
-            }
-            if (MODE == kAudioRate && __any_sync(kFull, bad)) fast = false;          // mod outside [0,1]: exact remainder path
-        }
-        if (!fast) {
-            indep = true;
-#pragma unroll
-            for (int k = 0; k < kSub; ++k) {
-                const int j = k * kWarp + lane;
-                const int n = n0 + j;
-                const bool valid = n < N;
-                float m;
-                s[k].x = xt[j];
-                if (MODE == kAudioRate) m = mt[j];
-                else if (MODE == kControlRate) m = upsample_ac(lo - lo_base, a.n_lo, a.up_scale, min(n, N - 1));
-                else m = valid ? lfo_value(lfo, n) : 0.0f;
-                fc_index(m, wk[k], c, s[k].fr, s[k].omfr, s[k].kp);
-                const int near = max(s[k].kp - 1, 1);          // = min(kp, kq)
-                indep = indep && (!valid || near > j);
-            }
-        }
-
-        if (__all_sync(kFull, indep)) {
-            // ---- whole tile independent of itself: 128 samples in one shot ----
-            float vp[kSub], vq[kSub];
-#pragma unroll
-            for (int k = 0; k < kSub; ++k) {
-                const int n = n0 + k * kWarp + lane;
-                vp[k] = ring[(n - s[k].kp) & c.mask];
-                vq[k] = ring[(n - kq_of(s[k].kp, c.M)) & c.mask];
-            }
-#pragma unroll
-            for (int k = 0; k < kSub; ++k) {
-                const int n = n0 + k * kWarp + lane;
-                float v, out;
-                fc_sample(s[k], vp[k], vq[k], c, v, out);
-                ring[n & c.mask] = v;
-                if (n < N) ys[n] = out;
-            }
-        } else {
-#pragma unroll
-            for (int k = 0; k < kSub; ++k) {
-                // ---- one 32-sample block ----
-                const int nb = n0 + k * kWarp;
-                const int cnt = min(kWarp, N - nb);
-                if (cnt <= 0) break;
-                const Samp me = s[k];
-                const int n = nb + lane;
-                const bool mine = lane < cnt;
-                const int near = mine ? max(me.kp - 1, 1) : 0x7fffffff;
-                // smallest dependency distance relative to the block start, over the block
-                const int slack = __reduce_min_sync(kFull, mine ? (near - lane) : 0x7fffffff);
-                const int kmin = __reduce_min_sync(kFull, mine ? me.kp : 0x7fffffff);
-                float my_out = 0.0f;
-                if (slack > 0) {
-                    // every sample depends only on samples before the block: one wave
-                    const float vp = ring[(n - me.kp) & c.mask];
-                    const float vq = ring[(n - kq_of(me.kp, c.M)) & c.mask];
-                    float v;
-                    fc_sample(me, vp, vq, c, v, my_out);
-                    __syncwarp();
-                    if (mine) ring[n & c.mask] = v;
-                } else {
-                    const int kmax = __reduce_max_sync(kFull, mine ? me.kp : 0);
-                    if (cnt == kWarp && kmax - kmin <= 1 && kmin <= kSerialMaxK && c.M >= 2 * kWarp) {
-                        // ---- delays of K..K+1 samples: register-history serial run ----
-                        const float stale = ring[(n - c.M) & c.mask];        // tap q of a sub-sample delay (kp == 1)
-                        coef[lane] = make_float4(me.x, me.fr, me.omfr, stale);
-                        const unsigned sel = __ballot_sync(kFull, me.kp == kmin);
-                        __syncwarp();
-                        switch (kmin) {
-                            case 1: serial_block<1>(ring, c.mask, nb, coef, sel, c.fb, itbuf); break;
-                            case 2: serial_block<2>(ring, c.mask, nb, coef, sel, c.fb, itbuf); break;
-                            case 3: serial_block<3>(ring, c.mask, nb, coef, sel, c.fb, itbuf); break;
-                            case 4: serial_block<4>(ring, c.mask, nb, coef, sel, c.fb, itbuf); break;
-                            case 5: serial_block<5>(ring, c.mask, nb, coef, sel, c.fb, itbuf); break;
-                            case 6: serial_block<6>(ring, c.mask, nb, coef, sel, c.fb, itbuf); break;
-                            default: serial_block<7>(ring, c.mask, nb, coef, sel, c.fb, itbuf); break;
-                        }
-                        __syncwarp();
-                        const float it = itbuf[lane];
-                        const float o = __fadd_rn(me.x, __fmul_rn(c.depth, it));                 // fx.py:115
-                        const float r = __fadd_rn(__fmul_rn(c.omm, me.x), __fmul_rn(c.mix, o));  // fx.py:117
-                        my_out = fminf(fmaxf(r, -1.0f), 1.0f);
-                    } else if (kmin >= 3) {
-                        // waves of mn consecutive samples: sample j depends on samples <= j - mn
-                        const int mn = kmin - 1;
-                        for (int done = 0; done < cnt; done += mn) {
-                            if (lane >= done && lane < done + mn && mine) {
-                                const float vp = ring[(n - me.kp) & c.mask];
-                                const float vq = ring[(n - kq_of(me.kp, c.M)) & c.mask];
-                                float v;
-                                fc_sample(me, vp, vq, c, v, my_out);
-                                ring[n & c.mask] = v;
-                            }
-                            __syncwarp();
-                        }
-                    } else {
-                        // ---- anything else with a 1-2 sample delay in it (irregular modulation): generic
-                        // lock-step serial run; taps at distance 1 and 2 come from registers, older taps are
-                        // loaded two samples ahead. ----
-                        float p1 = ring[(nb - 1) & c.mask];
-                        float p2 = ring[(nb - 2) & c.mask];
-                        int kpa = __shfl_sync(kFull, me.kp, 0);
-                        int kpb = __shfl_sync(kFull, me.kp, 1);
-                        float lpa = ring[(nb - kpa) & c.mask];
-                        float lqa = ring[(nb - kq_of(kpa, c.M)) & c.mask];
-                        float lpb = ring[(nb + 1 - kpb) & c.mask];
-                        float lqb = ring[(nb + 1 - kq_of(kpb, c.M)) & c.mask];
-                        float my_it = 0.0f;
-#pragma unroll 4
-                        for (int i = 0; i < cnt; ++i) {
-                            // taps of sample i+2 (valid when their distance is >= 3: already stored)
-                            const int kpc = __shfl_sync(kFull, me.kp, (i + 2) & 31);
-                            const float lpc = ring[(nb + i + 2 - kpc) & c.mask];
-                            const float lqc = ring[(nb + i + 2 - kq_of(kpc, c.M)) & c.mask];
-                            const float xi = __shfl_sync(kFull, me.x, i);
-                            const float fri = __shfl_sync(kFull, me.fr, i);
-                            const float omi = __shfl_sync(kFull, me.omfr, i);
-                            const int kqa = kq_of(kpa, c.M);
-                            const float vp = (kpa == 1) ? p1 : ((kpa == 2) ? p2 : lpa);
-                            const float vq = (kqa == 1) ? p1 : ((kqa == 2) ? p2 : lqa);
-                            const float it = __fadd_rn(__fmul_rn(fri, vq), __fmul_rn(omi, vp));     // fx.py:113
-                            const float v = __fadd_rn(xi, __fmul_rn(c.fb, it));                      // fx.py:114
-                            ring[(nb + i) & c.mask] = v;        // every lane stores the same value
-                            if (lane == i) my_it = it;
-                            p2 = p1; p1 = v;
-                            kpa = kpb; lpa = lpb; lqa = lqb;
-                            kpb = kpc; lpb = lpc; lqb = lqc;
-                        }
-                        const float o = __fadd_rn(me.x, __fmul_rn(c.depth, my_it));
-                        const float r = __fadd_rn(__fmul_rn(c.omm, me.x), __fmul_rn(c.mix, o));
-                        my_out = fminf(fmaxf(r, -1.0f), 1.0f);
-                    }
-                }
-                if (mine) ys[n] = my_out;
-                __syncwarp();
-            }
-        }
-        __syncwarp();
-#pragma unroll
-        for (int k = 0; k < kSub; ++k) {
-            wk[k] += kTile;
-            if (wk[k] >= c.M) { wk[k] -= c.M; if (wk[k] >= c.M) wk[k] %= c.M; }
-        }
-        if (++stage == kStages) stage = 0;
-    }
-    cp_async_wait<0>();
-}
-
 // ---- CTA per delay line, warp-specialised: the latency-oriented schedule (DESIGN.md "E1") ------------------
-// The one-warp kernel above spends ~1400 cycles per 128-sample tile because one warp does everything in turn: index
+// A single warp per delay line spends ~1400 cycles per 128-sample tile because it does everything in turn: index
 // arithmetic, x100 upsample, taps, the recurrence, the mix.  Only the recurrence v[n] = x[n] + fb * it[n] is
 // sequential; everything else is a function of n alone.  Here a CTA of 4 warps owns one delay line:
 //   * 3 PRODUCER warps run ahead, a 128-sample tile each in turn: they fill a ring of tile slots with
@@ -591,7 +249,7 @@ constexpr int kCtaProd = 3;
 constexpr int kCtaThreads = (kCtaProd + 1) * kWarp;     // 128
 constexpr int kNT = 2 * kCtaProd;                       // tile slots in flight (two per producer)
 constexpr int kXDepth = 4;                              // dry-audio tiles in flight per producer warp (cp.async)
-constexpr int kLoSmemMax = 2048;                        // in-kernel synthesised control rows up to this many points
+constexpr int kLoSmemMax = 2048;                        // in-kernel synthesised control rows staged in shared memory up to this many points
 constexpr int kSlotFloats = 4 * kTile + kTile + 8;      // float4 coef[128] | it[128] | slack of the four blocks, schedule codes
 constexpr int kSerialK = 8;                             // register-history serial runs cover tap distances up to this (+1)
 
@@ -614,18 +272,10 @@ __device__ __forceinline__ int ld_acquire(const int* p) {
 // operations of fx.py:113-114.  A real loop (the body stays in the instruction cache); the records of the next group
 // are pulled into registers ahead of the dependent chain, the taps come from history REGISTERS, results leave as two
 // 16-byte stores per group from one lane.
-#ifdef MODFX_FC_STATS
-}  // namespace
-__device__ unsigned long long g_serial_stats[4];     // calls, cycles inside the sample loop, cycles of the whole call
-namespace {
-#endif
 
 template <int K>
 __device__ __noinline__ void serial_run(float* __restrict__ ring, int mask, int nb, const float4* __restrict__ coef,
                                         float fb, float* __restrict__ it_out, int lane, int ngroups) {
-#ifdef MODFX_FC_STATS
-    const long long sr_t0 = clock64();
-#endif
     // Four groups of 4 samples per loop iteration over ONE register window w[]: for a group with base `o`,
     // w[o + 3 - u] is sample u of the group and w[o + 3 + j] the sample j before the group, so the tap of sample u at
     // distance d is w[o + 3 - u + d] whether it lies before the group or inside it.  The groups work at o = 12, 8, 4, 0
@@ -640,9 +290,6 @@ __device__ __noinline__ void serial_run(float* __restrict__ ring, int mask, int 
     float4 ca[4], cb[4];
 #pragma unroll
     for (int u = 0; u < 4; ++u) ca[u] = coef[u];
-#ifdef MODFX_FC_STATS
-    const long long sr_t1 = clock64();
-#endif
 #define MODFX_SERIAL_GROUP(O, CF, ITS)                                                                              \
     _Pragma("unroll") for (int u = 0; u < 4; ++u) {                                                                 \
         const float4 cf = CF[u];                                                                                    \
@@ -686,18 +333,18 @@ __device__ __noinline__ void serial_run(float* __restrict__ ring, int mask, int 
     }
 #undef MODFX_SERIAL_STEP
 #undef MODFX_SERIAL_GROUP
-#ifdef MODFX_FC_STATS
-    if (lane == 0) {
-        const long long sr_t2 = clock64();
-        atomicAdd(&g_serial_stats[0], 1ull);
-        atomicAdd(&g_serial_stats[1], (unsigned long long)ngroups);
-        atomicAdd(&g_serial_stats[2], (unsigned long long)(sr_t2 - sr_t0));
-        atomicAdd(&g_serial_stats[3], (unsigned long long)(sr_t2 - sr_t1));
-    }
-#endif
 }
 
-template <int MODE, bool SYNTH>
+// Where fc_cta_kernel's producers take the modulation from: memory (an audio-rate or control-rate mod_sig), or the LFO
+// parameters -- synthesised into shared memory first (control rows up to kLoSmemMax points) or evaluated where it is
+// needed (every sample of kDirectLfo, the two taps of every sample of a longer control row).
+enum Synth { kRead = 0, kStaged = 1, kAtTap = 2 };
+
+// lfo_value out of line, for the two taps of kAtTap control rows: inlined twice into the producer loop, its
+// double-precision cos makes ptxas spill
+__device__ __noinline__ float lfo_at(LfoDesc d, int i) { return lfo_value(d, i); }
+
+template <int MODE, int SYNTH>
 __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int lo_smem) {
     extern __shared__ __align__(16) float smem[];
     int* filled = reinterpret_cast<int*>(smem);                            // [kCtaProd] tiles filled by producer p
@@ -706,7 +353,7 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
     float* slots = smem + 16;                                              // [kNT][kSlotFloats]
     float* xstage = slots + kNT * kSlotFloats;                             // [kCtaProd][kXDepth][128] dry audio in flight
     float* mstage = xstage + kCtaProd * kXDepth * kTile;                   // same for an audio-rate mod_sig
-    float* lo_s = mstage + ((MODE == kAudioRate) ? kCtaProd * kXDepth * kTile : 0);   // [lo_smem] synthesised control row
+    float* lo_s = mstage + ((MODE == kAudioRate) ? kCtaProd * kXDepth * kTile : 0);   // [lo_smem] synthesised control row (or none)
     float* ring = lo_s + lo_smem;                                          // written samples, indexed by time & mask
     const int ring_w = (int)(ring - smem);                                 // word index of the ring inside smem[]
 
@@ -717,9 +364,9 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
     const int N = a.N;
     const Coef c = make_coef(a, b);
     const int mask = c.mask;
-    const float* lo = (MODE == kControlRate) ? (SYNTH ? lo_s : a.mod + (int64_t)b * a.n_lo) : nullptr;
+    const float* lo = (MODE == kControlRate) ? (SYNTH == kStaged ? lo_s : a.mod + (int64_t)b * a.n_lo) : nullptr;
 
-    if (MODE == kControlRate && !SYNTH && a.wide) {
+    if (MODE == kControlRate && SYNTH == kRead && a.wide) {
         // examples whose every tap lies more than a wide tile back were rendered by fc_wide_kernel (same predicate)
         float mn = INFINITY, mx = -INFINITY;
         for (int i = tid; i < a.n_lo; i += kCtaThreads) {
@@ -737,10 +384,10 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
     }
     if (tid < 8) filled[tid] = 0;
     for (int i = tid; i <= mask; i += kCtaThreads) ring[i] = 0.0f;                   // fx.py:92
-    if (MODE == kControlRate && SYNTH) {
-        const LfoDesc lfo = make_lfo_desc(a.lfo_freq[b], a.lfo_phase[b], a.lfo_shape[b], a.lfo_exp ? a.lfo_exp[b] : 1.0f, a.sr_lo);
+    LfoDesc lfo{};
+    if (SYNTH != kRead) lfo = make_lfo_desc(a.lfo_freq[b], a.lfo_phase[b], a.lfo_shape[b], a.lfo_exp ? a.lfo_exp[b] : 1.0f, a.sr_lo);
+    if (SYNTH == kStaged)
         for (int i = tid; i < a.n_lo; i += kCtaThreads) lo_s[i] = lfo_value(lfo, i);
-    }
     __syncthreads();
 
     const int ntiles = (N + kTile - 1) / kTile;
@@ -776,13 +423,6 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
         const int wstep = (kCtaProd * kTile) % c.M;
         int q = 0;                                          // stage of this warp's current tile
         int done_seen = 0;
-#ifdef MODFX_FC_STATS
-        long long pr_cyc[4] = {0, 0, 0, 0};                 // wait for the consumer, epilogue, audio wait, fill
-        long long pr_t0 = clock64();
-#define PR_STAT(k) do { const long long t1_ = clock64(); pr_cyc[k] += t1_ - pr_t0; pr_t0 = t1_; } while (0)
-#else
-#define PR_STAT(k) do { } while (0)
-#endif
         for (int t = p; t < ntiles + kNT; t += kCtaProd) {
             float* slot = slots + (t % kNT) * kSlotFloats;
             float4* cs = reinterpret_cast<float4*>(slot);
@@ -793,9 +433,8 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
                 const int td = t - kNT;
                 while (done_seen <= td) {
                     done_seen = ld_acquire(done);
-                    if (done_seen <= td) __nanosleep(MODFX_FC_POLL_NS);   // leave the issue slots to the warps that have work
+                    if (done_seen <= td) __nanosleep(kPollNs);   // leave the issue slots to the warps that have work
                 }
-                PR_STAT(0);
 #pragma unroll
                 for (int k = 0; k < kSub; ++k) {
                     const float x = cs[k * kWarp + lane].x;
@@ -806,7 +445,6 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
                     if (nj < N) ys[nj] = fminf(fmaxf(r, -1.0f), 1.0f);                          // fx.py:118
                 }
                 __syncwarp();
-                PR_STAT(1);
             }
             if (t < ntiles) {
                 {   // keep kXDepth - 1 tiles in flight
@@ -823,7 +461,6 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
                     cp_async_commit();
                 }
                 cp_async_wait<kXDepth - 1>();               // every lane reads back only what it copied itself
-                PR_STAT(2);
                 // straight-line arithmetic for the four 32-sample blocks of the tile (independent chains interleave);
                 // the exact-remainder path of fc_index is taken afterwards for the whole tile if any sample needs it
                 float xv[kSub], mv[kSub], frv[kSub], omv[kSub];
@@ -837,13 +474,18 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
                     float m;
                     if (MODE == kAudioRate) {
                         m = mine ? mq[q * kTile + k * kWarp + lane] : 0.0f;
+                    } else if (MODE == kDirectLfo) {
+                        m = lfo_value(lfo, min(n, N - 1));
                     } else {
                         const float src = __fmul_rn(a.up_scale, (float)min(n, N - 1));          // util.py:15-29
                         const int i0 = min((int)src, last_lo);
+                        const int i1 = min(i0 + 1, last_lo);
                         const float l1 = __fsub_rn(src, (float)i0);
                         const float l0 = __fsub_rn(1.0f, l1);
-                        const float m0 = SYNTH ? lo[i0] : __ldg(lo + i0);
-                        const float m1 = SYNTH ? lo[min(i0 + 1, last_lo)] : __ldg(lo + min(i0 + 1, last_lo));
+                        float m0, m1;
+                        if (SYNTH == kRead) { m0 = __ldg(lo + i0); m1 = __ldg(lo + i1); }
+                        else if (SYNTH == kStaged) { m0 = lo[i0]; m1 = lo[i1]; }
+                        else { m0 = lfo_at(lfo, i0); m1 = lfo_at(lfo, i1); }
                         m = __fmaf_rn(l0, m0, __fmul_rn(l1, m1));
                     }
                     mv[k] = m;
@@ -921,27 +563,13 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
                 __syncwarp();
                 if (lane == 0) st_release(filled + p, t / kCtaProd + 1);
                 if (++q == kXDepth) q = 0;
-                PR_STAT(3);
             }
         }
         cp_async_wait<0>();
-#ifdef MODFX_FC_STATS
-        if (lane == 0 && p == 0 && a.stats) {
-            long long* o = a.stats + (long long)gridDim.x * 12 + (long long)blockIdx.x * 4;
-            for (int k = 0; k < 4; ++k) o[k] = pr_cyc[k];
-        }
-#endif
         return;
     }
 
     // ================================ consumer ================================
-#ifdef MODFX_FC_STATS
-    long long st_cnt[6] = {0, 0, 0, 0, 0, 0}, st_cyc[6] = {0, 0, 0, 0, 0, 0};   // wait, one-shot / 4 x one-wave tiles, wave1, serial, waves, generic
-    long long st_t0 = clock64();
-#define FC_STAT(k) do { const long long t1_ = clock64(); st_cnt[k]++; st_cyc[k] += t1_ - st_t0; st_t0 = t1_; } while (0)
-#else
-#define FC_STAT(k) do { } while (0)
-#endif
     int avail = 0;                                          // tiles [0, avail) are known to be filled
     int sl = 0;
     for (int t = 0; t < ntiles; ++t) {
@@ -949,7 +577,6 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
             const int f0 = ld_acquire(filled), f1 = ld_acquire(filled + 1), f2 = ld_acquire(filled + 2);
             avail = min(min(kCtaProd * f0, kCtaProd * f1 + 1), kCtaProd * f2 + 2);
         }
-        FC_STAT(0);
         float* slot = slots + sl * kSlotFloats;
         float4* cs = reinterpret_cast<float4*>(slot);
         float* itb = slot + 4 * kTile;
@@ -1016,7 +643,6 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
                     __syncwarp();
                 }
             }
-            FC_STAT(1);
         } else {
             // ---- some block has a tap inside itself: the producer left a schedule code per block
             const unsigned codes = (unsigned)reinterpret_cast<const int*>(slot + 5 * kTile)[4];
@@ -1056,10 +682,6 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
                         default: serial_run<8>(ring, mask, nb, cb, c.fb, ito, lane, 8 * L); break;
                     }
                     __syncwarp();
-#ifdef MODFX_FC_STATS
-                    st_cnt[3] += L - 1;
-#endif
-                    FC_STAT(3);
                     j += L;
                     continue;
                 }
@@ -1073,7 +695,6 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
                     if (mine) ring[n & mask] = __fadd_rn(r.x, __fmul_rn(c.fb, my_it));
                     itb[j * kWarp + lane] = my_it;
                     __syncwarp();
-                    FC_STAT(2);
                 } else if (code == 14) {
                     // waves of kmin - 1 consecutive samples: sample i depends on samples <= i - (kmin - 1).  Every lane
                     // computes in every wave (no divergence); only the lanes of the wave keep and store their result.
@@ -1089,7 +710,6 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
                         __syncwarp();
                     }
                     itb[j * kWarp + lane] = my_it;
-                    FC_STAT(4);
                 } else {
                     // ---- anything else with a 1-2 sample delay in it: generic lock-step serial run; taps at
                     // distance 1 and 2 come from registers, older taps are loaded two samples ahead ----
@@ -1124,7 +744,6 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
                     }
                     itb[j * kWarp + lane] = my_it;
                     __syncwarp();
-                    FC_STAT(5);
                 }
                 ++j;
             }
@@ -1133,12 +752,6 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
         if (lane == 0) st_release(done, t + 1);
         if (++sl == kNT) sl = 0;
     }
-#ifdef MODFX_FC_STATS
-    if (lane == 0 && a.stats) {
-        long long* o = a.stats + (long long)blockIdx.x * 12;
-        for (int k = 0; k < 6; ++k) { o[k] = st_cnt[k]; o[6 + k] = st_cyc[k]; }
-    }
-#endif
 }
 
 // ---- all-pass fractional-delay interpolation (north_star: "per-sample linear or all-pass interpolation") -----------
@@ -1347,17 +960,21 @@ extern "C" int modfx_flanger_chorus_f32(const float* x, float* y, int32_t B, int
     if (a.n_items == 0) return MODFX_OK;
     MODFX_REQUIRE(a.n_items > 0, "n_items=%d", a.n_items);
 
-    const size_t smem = sizeof(float) * ((size_t)ring + (size_t)kStages * kTile + 5 * kWarp +
-                                         (mode == kAudioRate ? (size_t)kStages * kTile : (mode == kControlRate ? (size_t)kLoWin + 4 : 0)));
-    if (smem > 200 * 1024)
-        return fail(MODFX_ERR_UNSUPPORTED, "delay line of %d samples (+%d control points) needs %zu B of shared memory",
-                    a.M, a.n_lo, smem);
+    // The CTA-per-delay-line kernel renders every modulation source; a control row synthesised in-kernel is staged in
+    // shared memory up to kLoSmemMax points and evaluated at the taps beyond that.
+    const bool synth = a.lfo_freq != nullptr;
+    const int lo_smem = (mode == kControlRate && synth && a.n_lo <= kLoSmemMax) ? ((a.n_lo + 3) & ~3) : 0;
+    const size_t csmem = sizeof(float) * (16 + (size_t)kNT * kSlotFloats +
+                                          (size_t)kCtaProd * kXDepth * kTile * (mode == kAudioRate ? 2 : 1) +
+                                          (size_t)lo_smem + (size_t)ring);
+    if (csmem > 200 * 1024)
+        return fail(MODFX_ERR_UNSUPPORTED, "delay line of %d samples needs %zu B of shared memory", a.M, csmem);
     const dim3 grid((unsigned)((int64_t)a.n_items * C));
     cudaStream_t s = as_stream(stream);
     // Delay lines that can never reach back less than a wide tile (min_delay_width * Mmin >= 388 samples: the chorus) go
-    // through the CTA-per-example kernel first; the one-warp kernel then skips exactly those examples.
+    // through the CTA-per-example kernel first; fc_cta_kernel then skips exactly those examples.
     a.wide = 0;
-    if (mode == kControlRate && !a.lfo_freq && Mmin >= kWideTile + kWideMargin) {
+    if (mode == kControlRate && !synth && Mmin >= kWideTile + kWideMargin) {
         const int wring = next_pow2(a.M + kWideTile);
         const size_t wsmem = sizeof(float) * (size_t)wring;
         if (wsmem <= 200 * 1024) {
@@ -1368,52 +985,18 @@ extern "C" int modfx_flanger_chorus_f32(const float* x, float* y, int32_t B, int
             MODFX_CUDA_OK(cudaGetLastError());
         }
     }
-    // The latency-oriented CTA-per-delay-line kernel covers a modulation signal read from memory (audio rate or control
-    // rate) and control rows synthesised in-kernel up to kLoSmemMax points; the one-warp kernel keeps the rest (an
-    // audio-rate LFO synthesised per sample, very long synthesised control rows) and MODFX_FC_KERNEL=warp forces it.
-#ifdef MODFX_FC_STATS
-    {
-        const char* sp = getenv("MODFX_FC_STATS_PTR");
-        a.stats = sp ? reinterpret_cast<long long*>(strtoull(sp, nullptr, 0)) : nullptr;
-    }
-#endif
-    const char* force = getenv("MODFX_FC_KERNEL");
-    const bool force_warp = force && force[0] == 'w';
-    const bool cta_ok = !force_warp && (mode == kAudioRate || (mode == kControlRate && (!a.lfo_freq || a.n_lo <= kLoSmemMax)));
-    if (cta_ok) {
-        const int lo_smem = (mode == kControlRate && a.lfo_freq) ? ((a.n_lo + 3) & ~3) : 0;
-        const size_t csmem = sizeof(float) * (16 + (size_t)kNT * kSlotFloats +
-                                              (size_t)kCtaProd * kXDepth * kTile * (mode == kAudioRate ? 2 : 1) +
-                                              (size_t)lo_smem + (size_t)ring);
-        if (csmem > 200 * 1024)
-            return fail(MODFX_ERR_UNSUPPORTED, "delay line of %d samples needs %zu B of shared memory", a.M, csmem);
-#define LAUNCH_CTA(MODE)                                                                                  \
+#define LAUNCH_CTA(MODE, SYNTH)                                                                           \
     do {                                                                                                  \
         if (csmem > 48 * 1024)                                                                            \
             MODFX_CUDA_OK(cudaFuncSetAttribute(fc_cta_kernel<MODE, SYNTH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)csmem)); \
         fc_cta_kernel<MODE, SYNTH><<<grid, kCtaThreads, csmem, s>>>(a, lo_smem);                          \
     } while (0)
-#define SYNTH false
-        if (mode == kAudioRate) LAUNCH_CTA(kAudioRate);
-        else if (!a.lfo_freq) LAUNCH_CTA(kControlRate);
-#undef SYNTH
-#define SYNTH true
-        else LAUNCH_CTA(kControlRate);
-#undef SYNTH
+    if (mode == kAudioRate) LAUNCH_CTA(kAudioRate, kRead);
+    else if (mode == kDirectLfo) LAUNCH_CTA(kDirectLfo, kAtTap);
+    else if (!synth) LAUNCH_CTA(kControlRate, kRead);
+    else if (lo_smem > 0) LAUNCH_CTA(kControlRate, kStaged);
+    else LAUNCH_CTA(kControlRate, kAtTap);
 #undef LAUNCH_CTA
-        MODFX_CUDA_OK(cudaGetLastError());
-        return MODFX_OK;
-    }
-#define LAUNCH_FC(MODE)                                                                                   \
-    do {                                                                                                  \
-        if (smem > 48 * 1024)                                                                             \
-            MODFX_CUDA_OK(cudaFuncSetAttribute(fc_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        fc_kernel<MODE><<<grid, kWarp, smem, s>>>(a);                                                     \
-    } while (0)
-    if (mode == kAudioRate) LAUNCH_FC(kAudioRate);
-    else if (mode == kControlRate) LAUNCH_FC(kControlRate);
-    else LAUNCH_FC(kDirectLfo);
-#undef LAUNCH_FC
     MODFX_CUDA_OK(cudaGetLastError());
     return MODFX_OK;
 }
@@ -1462,13 +1045,6 @@ extern "C" int modfx_flanger_chorus_allpass_f32(const float* x, float* y, int32_
     MODFX_CUDA_OK(cudaGetLastError());
     return MODFX_OK;
 }
-
-#ifdef MODFX_FC_STATS
-extern "C" int modfx_fc_serial_stats(unsigned long long* out4) {
-    cudaDeviceSynchronize();
-    return (int)cudaMemcpyFromSymbol(out4, modfx::g_serial_stats, sizeof(unsigned long long) * 4);
-}
-#endif
 
 extern "C" int modfx_tremolo_f32(const float* x, float* y, int32_t B, int32_t C, int64_t N,
                                  const modfx_mod_source* mod, modfx_param mix, void* stream) {

@@ -5,19 +5,11 @@
 //
 // The filter is a 7-state linear time-varying recurrence (6 all-pass states + the fed-back output),
 // strictly serial per example: ~100 dependent cycles per sample.  It is parallelised over time with
-// a chunked affine scan (DESIGN.md "P1"):
-//   K0  control-rate cutoff: the oscillator phase is accumulated in float32 exactly like the
-//       reference (sequentially inside each 8192-sample host block) and mapped to the all-pass
-//       coefficient c = 2G-1 for every 4th sample;
-//   K1  for every chunk of 128 samples, 8 independent runs give the chunk's state-transition matrix
-//       (7 homogeneous runs from the unit states) and its zero-state response (1 run with the audio);
-//   K2  the 7x7 maps are chained to get the true state at every chunk start: groups of 32 maps are composed
-//       in parallel, the group maps chained serially, and every group re-chained from its initial state;
-//   K3  every chunk is re-run from its true initial state and writes the mixed, clipped output.
-// K1 and K3 stage audio through shared memory so global traffic stays coalesced.
+// a chunked affine scan (DESIGN.md "P1"): phaser_phase_kernel accumulates the oscillator phase in float32
+// exactly like the reference (sequentially inside each host block), and phaser_fused_kernel renders one
+// 4096-sample segment per CTA out of shared memory -- coefficients, per-sub-chunk affine maps, their chain
+// (with the segment's entry state taken from the previous segment's CTA), the re-run, mix and clip.
 #include "common.cuh"
-
-#include <stdlib.h>
 
 namespace modfx {
 namespace {
@@ -41,80 +33,9 @@ struct PhaserArgs {
     int n_items;
     int n_ctl;       // control points per example = ceil(N / 4)
     int n_chunks;    // ceil(N / kChunk)
-    float* C;        // (n_items, n_ctl)   phase, then all-pass coefficient c
-    float* Mw;       // (n_items, n_chunks, 56)
-    float* S;        // (n_items, n_chunks, 8)
 };
 
 __device__ __forceinline__ int example_of(const PhaserArgs& a, int item) { return a.index ? a.index[item] : item; }
-
-// ---- K0: control-rate all-pass coefficient ----------------------------------------------------
-// juce::dsp::Oscillator semantics: inside a host block the phase advances by `inc` per control point
-// with a wrap at 2 pi (sequential float32 adds, reproduced exactly); between blocks it advances by
-// inc * (points in the block) in one step.  A CTA owns 32 (example, host block) pairs: warp 0 walks
-// the 32 phase sequences (lane = pair) 32 control points at a time into a shared tile, then all 256
-// threads map the 1024 phases to c = 2G-1 (sin, 10^x, tan: the expensive part) and store them with
-// 128-byte rows.
-constexpr int kK0Threads = 256;
-__global__ void __launch_bounds__(kK0Threads) phaser_ctl_kernel(const PhaserArgs a, int n_blocks) {
-    __shared__ float tile[32][33];
-    __shared__ int j0s[32], j1s[32], items[32];
-    __shared__ float vol[32], ctr[32];
-    const int tid = threadIdx.x;
-    const float two_pi = MODFX_TWO_PI_F;
-    const float f_lo = 20.0f;
-    const double f_hi_d = (0.49 * (double)a.sr < 20000.0) ? 0.49 * (double)a.sr : 20000.0;
-    const float log_min = log10f(f_lo), log_max = log10f((float)f_hi_d);
-    const float log_span = log_max - log_min;
-    const float w0 = MODFX_PI_F / a.sr;
-    float p = 0.0f, inc = 0.0f;
-    if (tid < 32) {
-        const int pair = blockIdx.x * 32 + tid;
-        const bool live = pair < a.n_items * n_blocks;
-        const int item = live ? pair / n_blocks : 0, blk = live ? pair - item * n_blocks : 0;
-        const int b = example_of(a, item);
-        const float sr_down = (float)((double)a.sr / (double)kUpd);
-        inc = a.rate[b] * (two_pi / sr_down);
-        for (int i = 0; i < blk; ++i) {
-            const int64_t s0 = (int64_t)i * a.block, s1 = min((int64_t)(i + 1) * a.block, (int64_t)a.N);
-            const int n_down = (int)((s1 + kUpd - 1) / kUpd - (s0 + kUpd - 1) / kUpd);
-            float next = p + inc * (float)n_down;
-            while (next >= two_pi) next -= two_pi;
-            p = next;
-        }
-        const int64_t s0 = (int64_t)blk * a.block, s1 = min((int64_t)(blk + 1) * a.block, (int64_t)a.N);
-        j0s[tid] = live ? (int)((s0 + kUpd - 1) / kUpd) : 0;
-        j1s[tid] = live ? (int)((s1 + kUpd - 1) / kUpd) : 0;
-        items[tid] = item;
-        vol[tid] = a.depth[b] * 0.5f;                                           // oscVolume target
-        ctr[tid] = (log10f(a.centre[b]) - log_min) / log_span;                   // mapFromLog10(centre)
-    }
-    const int rounds = (int)((((int64_t)a.block + kUpd - 1) / kUpd + 31) / 32) + 1;
-    for (int r = 0; r < rounds; ++r) {
-        __syncthreads();
-        if (tid < 32) {
-#pragma unroll 8
-            for (int q = 0; q < 32; ++q) {
-                tile[tid][q] = p;
-                float next = p + inc;
-                while (next >= two_pi) next -= two_pi;
-                p = next;
-            }
-        }
-        __syncthreads();
-        for (int e = tid; e < 32 * 32; e += kK0Threads) {
-            const int t = e >> 5, q = e & 31;
-            const int j = j0s[t] + 32 * r + q;
-            if (j < j1s[t]) {
-                float lfo = sinf(tile[t][q] - MODFX_PI_F) * vol[t] + ctr[t];
-                lfo = fminf(fmaxf(lfo, 0.0f), 1.0f);
-                const float fc = exp10f(lfo * log_span + log_min);               // mapToLog10
-                const float g = tanf(w0 * fc);                                   // TPT prewarp
-                a.C[(int64_t)items[t] * a.n_ctl + j] = 2.0f * (g / (1.0f + g)) - 1.0f;
-            }
-        }
-    }
-}
 
 // One sample of the cascade.  With c = 2G-1 the TPT all-pass (v = G(in-s); y = v+s; s' = y+v; out = 2y-in)
 // is out = c*in + (1-c)*s, s' = (1+c)*in - c*s.  Carrying w = (1-c)*s instead of s turns every stage into
@@ -139,7 +60,7 @@ __device__ __forceinline__ void cascade_retune(float (&w)[kStagesAP], float c_ol
 }
 
 // Two runs of the cascade at once, one per half of a float2 (same coefficient): Blackwell's packed FFMA2 does the
-// work of two FFMAs in one issue slot, and the map kernel is bound by instruction issue.
+// work of two FFMAs in one issue slot, and the map stage is bound by instruction issue.
 __device__ __forceinline__ float2 cascade_step2(float2 in, float2 (&w)[kStagesAP], float c) {
     const float2 c2 = make_float2(c, c), nc2 = make_float2(-c, -c);
     float2 v = in;
@@ -159,287 +80,17 @@ __device__ __forceinline__ void cascade_retune2(float2 (&w)[kStagesAP], float c_
     for (int k = 0; k < kStagesAP; ++k) w[k] = __fmul2_rn(w[k], r2);
 }
 
-// ---- K1: per-chunk affine map ----------------------------------------------------------------
-// block = 128 threads = 4 warps; warp p performs runs 2p and 2p+1 packed in a float2 (runs 0..6: unit state
-// e_r, no input; run 7: zero state, driven by x) for 32 consecutive chunks, lane = chunk.  The run pair is
-// warp-uniform, so the homogeneous warps never touch the audio.
-template <bool DRIVEN>
-__device__ __forceinline__ void map_run2(const float (*xs)[kChunk + 1], const float (*cs)[kCtl + 2], int ch, int len,
-                                         float fbk, float2 (&s)[kStagesAP], float2& out_prev, int j_begin, float c_cur) {
-    // j_begin is 0, or kUpd when the caller has already done the first control group by hand
-    // out_prev holds the previous cascade outputs; lastOutput = out_prev * feedback.
-    // cs[ch][0] is the coefficient of the sample before the chunk, cs[ch][1 + g] that of control group g.
-    const float2 nfb = make_float2(-fbk, -fbk);
-    if (len == kChunk) {                       // full chunk: no guards, one coefficient per 4 samples
-#pragma unroll 2
-        for (int g = j_begin / kUpd; g < kCtl; ++g) {
-            const float c = cs[ch][1 + g];
-            cascade_retune2(s, c_cur, c);
-            c_cur = c;
-#pragma unroll
-            for (int q = 0; q < kUpd; ++q) {
-                const float2 u = DRIVEN ? __ffma2_rn(nfb, out_prev, make_float2(0.0f, xs[ch][g * kUpd + q]))
-                                        : __fmul2_rn(nfb, out_prev);
-                out_prev = cascade_step2(u, s, c);
-            }
-        }
-    } else {
-        for (int j = j_begin; j < len; ++j) {
-            const float c = cs[ch][1 + (j >> 2)];
-            if (c != c_cur) {
-                cascade_retune2(s, c_cur, c);
-                c_cur = c;
-            }
-            const float2 u = DRIVEN ? __ffma2_rn(nfb, out_prev, make_float2(0.0f, xs[ch][j])) : __fmul2_rn(nfb, out_prev);
-            out_prev = cascade_step2(u, s, c);
-        }
-    }
-}
-
-constexpr int kMapThreads = 128;
-__global__ void __launch_bounds__(kMapThreads) phaser_map_kernel(const PhaserArgs a, int n_super) {
-    __shared__ float xs[32][kChunk + 1];
-    __shared__ float cs[32][kCtl + 2];
-    const int item = blockIdx.x / n_super, sc = blockIdx.x - item * n_super;
-    const int b = example_of(a, item);
-    const int tid = threadIdx.x;
-    const int n_base = sc * 32 * kChunk;
-    const float* xr = a.x + (int64_t)b * a.N;
-    for (int i = tid; i < 32 * kChunk; i += kMapThreads) {
-        const int n = n_base + i;
-        xs[i / kChunk][i % kChunk] = (n < a.N) ? xr[n] : 0.0f;
-    }
-    const float* cr = a.C + (int64_t)item * a.n_ctl;
-    for (int i = tid; i < 32 * (kCtl + 1); i += kMapThreads) {
-        const int row = i / (kCtl + 1), col = i % (kCtl + 1);          // col 0 = coefficient before the chunk
-        const int j = n_base / kUpd + row * kCtl + col - 1;
-        cs[row][col] = cr[max(0, min(j, a.n_ctl - 1))];
-    }
-    __syncthreads();
-    const int pair = tid >> 5, ch = tid & 31;
-    const int chunk = sc * 32 + ch;
-    if (chunk >= a.n_chunks) return;
-    const int len = min(kChunk, a.N - chunk * kChunk);
-    const float fbk = a.feedback[b];
-    float2 s[kStagesAP];
-#pragma unroll
-    for (int k = 0; k < kStagesAP; ++k) s[k] = make_float2((2 * pair == k) ? 1.0f : 0.0f, (2 * pair + 1 == k) ? 1.0f : 0.0f);
-    float2 out_prev = make_float2(0.0f, 0.0f);
-    const float c_prev = cs[ch][0];
-    if (pair == 3) {
-        // runs 6 and 7.  State 6 is lastOutput = out_prev * feedback: a unit lastOutput is out_prev = 1 / feedback; to
-        // stay finite for feedback = 0 the unit run is fed u = -1 by hand for the first sample.  Both runs start
-        // with zero all-pass states, so there is nothing to retune before the first control group.
-        const float c0 = cs[ch][1];
-        out_prev = cascade_step2(make_float2(-1.0f, xs[ch][0]), s, c0);
-        const int n0 = min(kUpd, len);
-        const float2 nfb = make_float2(-fbk, -fbk);
-        for (int q = 1; q < n0; ++q)
-            out_prev = cascade_step2(__ffma2_rn(nfb, out_prev, make_float2(0.0f, xs[ch][q])), s, c0);
-        map_run2<true>(xs, cs, ch, len, fbk, s, out_prev, kUpd, c0);
-    } else {
-        map_run2<false>(xs, cs, ch, len, fbk, s, out_prev, 0, c_prev);
-    }
-    float* m = a.Mw + ((int64_t)item * a.n_chunks + chunk) * kMapFloats + 2 * pair * kState;
-#pragma unroll
-    for (int k = 0; k < kStagesAP; ++k) {
-        m[k] = s[k].x;
-        m[kState + k] = s[k].y;
-    }
-    m[6] = out_prev.x * fbk;
-    m[kState + 6] = out_prev.y * fbk;
-}
-
-// ---- K2: chain the maps: state at the start of every chunk --------------------------------------
-// 8 lanes per example; lane i < 7 owns state component i.
-// The chain of n_chunks affine maps per example is resolved in three short passes instead of one long
-// one (689 dependent steps for 2 s, 20 672 for 60 s): (a) groups of 32 consecutive chunk maps are
-// composed into one map each, all groups in parallel; (b) the group maps are chained serially (22 steps
-// for 2 s); (c) every group re-chains its 32 chunk maps from its now known initial state.
-constexpr int kGroup = 32;
-constexpr int kSerialChainMax = 4096;     // up to this many maps per example a single serial chain is used (measured faster)
-
-// (a) compose the maps of one group: 8 lanes per group, lane r carries column r of [Phi | z]
-__global__ void __launch_bounds__(256) phaser_compose_kernel(const PhaserArgs a, int n_groups, float* __restrict__ GM) {
-    const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int64_t team = gid >> 3;
-    const int r = (int)(gid & 7);
-    if (team >= (int64_t)a.n_items * n_groups) return;
-    const int item = (int)(team / n_groups), g = (int)(team - (int64_t)item * n_groups);
-    const int c0 = g * kGroup, c1 = min(c0 + kGroup, a.n_chunks);
-    const float* m = a.Mw + ((int64_t)item * a.n_chunks + c0) * kMapFloats;
-    float col[kState];
-#pragma unroll
-    for (int i = 0; i < kState; ++i) col[i] = (i == r) ? 1.0f : 0.0f;      // r == 7: the z column starts at 0
-    for (int c = c0; c < c1; ++c, m += kMapFloats) {
-        float nxt[kState];
-#pragma unroll
-        for (int i = 0; i < kState; ++i) nxt[i] = (r == 7) ? __ldg(m + 7 * kState + i) : 0.0f;
-#pragma unroll
-        for (int k = 0; k < kState; ++k) {
-#pragma unroll
-            for (int i = 0; i < kState; ++i) nxt[i] = fmaf(__ldg(m + k * kState + i), col[k], nxt[i]);
-        }
-#pragma unroll
-        for (int i = 0; i < kState; ++i) col[i] = nxt[i];
-    }
-    float* o = GM + team * kMapFloats + r * kState;
-#pragma unroll
-    for (int i = 0; i < kState; ++i) o[i] = col[i];
-}
-
-// (b), (c) chain maps [seg * seg_len, (seg + 1) * seg_len) of every example from an initial state
-// (zero when init == nullptr), writing the state at the start of every map.  8 lanes per segment;
-// lane i < 7 owns state component i.
-__global__ void __launch_bounds__(256) phaser_chain_kernel(const float* __restrict__ maps, int n_maps, int seg_len,
-                                                           int n_items, const float* __restrict__ init,
-                                                           float* __restrict__ out) {
-    const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int i = (int)(gid & 7);
-    const int n_seg = (n_maps + seg_len - 1) / seg_len;
-    int64_t team = gid >> 3;
-    const bool live = team < (int64_t)n_items * n_seg;
-    if (!live) team = 0;
-    const int item = (int)(team / n_seg), seg = (int)(team - (int64_t)item * n_seg);
-    const int c0 = seg * seg_len, c1 = min(c0 + seg_len, n_maps);
-    const float* m = maps + ((int64_t)item * n_maps + c0) * kMapFloats;
-    float* S = out + ((int64_t)item * n_maps + c0) * kSFloats;
-    const int ii = (i < kState) ? i : 0;
-    const int n = c1 - c0;
-    constexpr int kAhead = 4;                  // maps in flight (their coefficients do not depend on the state)
-    float buf[kAhead][8];
-#pragma unroll
-    for (int d = 0; d < kAhead; ++d) {
-        const float* mc = m + (int64_t)min(d, n - 1) * kMapFloats;
-#pragma unroll
-        for (int r = 0; r < 8; ++r) buf[d][r] = mc[r * kState + ii];
-    }
-    float s = (init && i < kState) ? init[((int64_t)item * n_seg + seg) * kSFloats + i] : 0.0f;
-    // every team of the warp runs the same number of steps (the shuffles below need all 32 lanes);
-    // steps past the end of a short last segment are computed and discarded
-    for (int b0 = 0; b0 < seg_len; b0 += kAhead) {
-#pragma unroll
-        for (int d = 0; d < kAhead; ++d) {
-            const int cidx = b0 + d;
-            float cur[8];
-#pragma unroll
-            for (int r = 0; r < 8; ++r) cur[r] = buf[d][r];
-            {   // refill this slot with map cidx + kAhead
-                const float* mc = m + (int64_t)min(cidx + kAhead, n - 1) * kMapFloats;
-#pragma unroll
-                for (int r = 0; r < 8; ++r) buf[d][r] = mc[r * kState + ii];
-            }
-            float acc = cur[7];                                        // zero-state response
-#pragma unroll
-            for (int r = 0; r < kState; ++r) acc = fmaf(cur[r], __shfl_sync(kFull, s, r, 8), acc);
-            if (cidx < n) {
-                if (live) S[cidx * kSFloats + i] = s;
-                s = (i < kState) ? acc : 0.0f;
-            }
-        }
-    }
-}
-
-// ---- K3: re-run every chunk from its true state, mix and clip --------------------------------------
-// (Packing two chunks per thread like K1 was measured: 0.56 ms instead of 0.36 ms for 1365 x 2 s, because it
-// halves the warps that hide the tile loads; this kernel is latency-bound, not issue-bound.)
-// One thread per chunk; a warp owns 32 consecutive chunks (16 KB of audio).  The audio moves through a
-// per-warp 32 x 32 shared tile: row i is filled by one coalesced 128-byte request (all lanes read chunk
-// i), then lane i walks row i.  That keeps every global request at one cache line (a lane-per-chunk
-// access would touch 32 lines per request and saturate the L1 tag stage).
-constexpr int kRunWarps = 4;
-__global__ void __launch_bounds__(32 * kRunWarps) phaser_run_kernel(const PhaserArgs a) {
-    __shared__ float tile[kRunWarps][32][33];
-    __shared__ float ctile[kRunWarps][32][33];
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int64_t wid = (int64_t)blockIdx.x * kRunWarps + w;          // warp id = group of 32 chunks of one example
-    const int groups = (a.n_chunks + 31) / 32;
-    if (wid >= (int64_t)a.n_items * groups) return;
-    const int item = (int)(wid / groups), grp = (int)(wid - (int64_t)item * groups);
-    const int b = example_of(a, item);
-    const int chunk0 = grp * 32;
-    const int chunk = chunk0 + lane;
-    const bool live = chunk < a.n_chunks;
-    const int n_base = chunk0 * kChunk;                                // first sample of the warp's span
-    const float* xr = a.x + (int64_t)b * a.N;
-    float* yr = a.y + (int64_t)b * a.N;
-    const float* cr = a.C + (int64_t)item * a.n_ctl;
-    float(*t)[33] = tile[w];
-    float(*ct)[33] = ctile[w];
-    // coefficients of the 32 chunks: row i = chunk i's 32 control points
-#pragma unroll 4
-    for (int i = 0; i < 32; ++i) {
-        const int j = (n_base >> 2) + i * kCtl + lane;
-        ct[i][lane] = (j < a.n_ctl) ? __ldg(cr + j) : 0.0f;
-    }
-    const float fbk = a.feedback[b];
-    const float wet = a.mix[b], dry = 1.0f - a.mix[b];
-    float s[kStagesAP];
-    float last = 0.0f;
-    if (live) {
-        const float* S = a.S + ((int64_t)item * a.n_chunks + chunk) * kSFloats;
-#pragma unroll
-        for (int k = 0; k < kStagesAP; ++k) s[k] = S[k];
-        last = S[6];
-    } else {
-#pragma unroll
-        for (int k = 0; k < kStagesAP; ++k) s[k] = 0.0f;
-    }
-    const int len = live ? min(kChunk, a.N - chunk * kChunk) : 0;
-    float c_cur = cr[max(0, min(chunk * kCtl - 1, a.n_ctl - 1))];      // coefficient of the sample before the chunk
-    for (int q0 = 0; q0 < kChunk; q0 += 32) {                          // 4 sub-tiles of 32 samples
-        __syncwarp();
-#pragma unroll 4
-        for (int i = 0; i < 32; ++i) {
-            const int n = n_base + i * kChunk + q0 + lane;
-            t[i][lane] = (n < a.N) ? __ldg(xr + n) : 0.0f;
-        }
-        __syncwarp();
-        if (q0 + 32 <= len) {
-#pragma unroll 2
-            for (int g = 0; g < 8; ++g) {
-                const float c = ct[lane][(q0 >> 2) + g];
-                cascade_retune(s, c_cur, c);
-                c_cur = c;
-#pragma unroll
-                for (int q = 0; q < kUpd; ++q) {
-                    const float in = t[lane][g * kUpd + q];
-                    const float out = cascade_step(in - last, s, c);
-                    last = out * fbk;
-                    t[lane][g * kUpd + q] = fminf(fmaxf(fmaf(wet, out, dry * in), -1.0f), 1.0f);   // datasets.py:472
-                }
-            }
-        } else {
-            for (int q = 0; q0 + q < len && q < 32; ++q) {
-                const float c = ct[lane][(q0 + q) >> 2];
-                if (c != c_cur) {
-                    cascade_retune(s, c_cur, c);
-                    c_cur = c;
-                }
-                const float in = t[lane][q];
-                const float out = cascade_step(in - last, s, c);
-                last = out * fbk;
-                t[lane][q] = fminf(fmaxf(fmaf(wet, out, dry * in), -1.0f), 1.0f);
-            }
-        }
-        __syncwarp();
-#pragma unroll 4
-        for (int i = 0; i < 32; ++i) {
-            const int n = n_base + i * kChunk + q0 + lane;
-            if (n < a.N) yr[n] = t[i][lane];
-        }
-    }
-}
-
 // =====================================================================================================================
-// Single-pass fused phaser (the default path): one kernel reads the audio once and writes the result once.
+// Single-pass fused phaser: one kernel reads the audio once and writes the result once.
 //
-// The four-kernel pipeline above moves 2.3x the algorithmic bytes (the audio is read twice, the control-rate coefficients
-// and the per-chunk maps round-trip HBM).  Here a CTA owns one SEGMENT of 4096 samples of one example and does everything
-// for it out of shared memory:
+// A CTA owns one SEGMENT of 4096 samples of one example and does everything for it out of shared memory (a pipeline
+// of separate kernels, with the audio read twice and the coefficients and per-chunk maps round-tripping HBM, moved 2.3x
+// the algorithmic bytes):
 //   A  the segment's audio lands in shared memory (one coalesced pass); the float32 oscillator phases of its 1024
 //      control points are walked chunk by chunk from chunk-start phases (phaser_phase_kernel below: a few bytes per
-//      128 samples, the only thing that is precomputed) -- sequential adds with the wrap at 2 pi, like the restatement;
+//      128 samples, the only thing that is precomputed) -- sequential adds with the wrap at 2 pi, like the restatement.
+//      With a host block that is not a multiple of 128 samples a block boundary can fall inside a chunk, and the phase
+//      of every control point is precomputed and copied instead;
 //   B  the transcendental map phase -> all-pass coefficient c = 2G - 1, all threads;
 //   C  per 64-sample sub-chunk the 7 unit-state runs + the zero-state run (two runs per thread, packed FFMA2) give its
 //      affine map; lanes = sub-chunks, so a warp's 32 lanes walk 32 different sub-chunks (padded rows: no conflicts);
@@ -473,9 +124,14 @@ struct FusedArgs {
     int* flags;                 // (n_items, n_seg), zero at launch
     float* rec;                 // (n_items, n_seg, kRec)
     float2* ph;                 // (n_items, n_chunks): phase at the chunk's first control point, phase of the one before
+    float* phc;                 // (n_items, n_ctl): phase of every control point; used instead of ph (then nullptr) when
+                                // the host block is not a multiple of kChunk samples
 };
 
-// chunk-start phases: one thread per (example, host block), juce::dsp::Oscillator semantics (see phaser_ctl_kernel).
+// Oscillator phases: one thread per (example, host block), juce::dsp::Oscillator semantics.  Control points sit at
+// global multiples of 4 samples; inside a host block the phase advances by `inc` per control point with a wrap at 2 pi
+// (sequential float32 adds, reproduced exactly); a block starts from the previous block's start phase advanced by
+// inc * (control points in that block) in one step.
 // The float32 phase is a chain of sequential additions with the wrap at 2 pi, so a host block of 8192 samples is 2048
 // dependent steps whatever is done -- what can be kept short is the step: when the increment is below 2 pi (always, for
 // an LFO) the wrap is ONE conditional subtraction (p + inc < 4 pi), computed branch-free (add, subtract, select: 12 cycles
@@ -501,11 +157,23 @@ __global__ void __launch_bounds__(128) phaser_phase_kernel(const FusedArgs f, in
     const float inc = a.rate[b] * (two_pi / sr_down);
     float p = 0.0f;
     for (int i = 0; i < blk; ++i) {                  // whole blocks before this one: phase.advance(freq * n_down)
-        float next = p + inc * (float)(a.block / kUpd);
+        // a rounded product, like the reference: contracted into an FMA it drifts from it whenever inc * n_down is inexact
+        const int n_down = ((i + 1) * a.block + kUpd - 1) / kUpd - (i * a.block + kUpd - 1) / kUpd;
+        float next = __fadd_rn(p, __fmul_rn(inc, (float)n_down));
         while (next >= two_pi) next -= two_pi;
         p = next;
     }
     const int s0 = blk * a.block, s1 = min(s0 + a.block, a.N);
+    if (f.phc) {                                     // the phase of every control point of the block
+        float* out = f.phc + (int64_t)item * a.n_ctl;
+        for (int j = (s0 + kUpd - 1) / kUpd; j < (s1 + kUpd - 1) / kUpd; ++j) {
+            out[j] = p;
+            float next = p + inc;
+            while (next >= two_pi) next -= two_pi;
+            p = next;
+        }
+        return;
+    }
     const int c0 = s0 / kChunk, c1 = (s1 + kChunk - 1) / kChunk;
     float2* out = f.ph + (int64_t)item * a.n_chunks;
     // a clip's very first control point has no predecessor and the value is unused (all filter states are zero there)
@@ -581,7 +249,13 @@ __global__ void __launch_bounds__(kFusedThreads) phaser_fused_kernel(const Fused
         }
     }
     const float two_pi = MODFX_TWO_PI_F;
-    if (tid < kSegChunks) {
+    if (f.phc) {                                                          // precomputed: copy them
+        const float* pr = f.phc + (int64_t)item * a.n_ctl;
+        for (int i = tid; i <= kSegCtl; i += kFusedThreads) {
+            const int j = seg * kSegCtl - 1 + i;                          // i = 0: the control point before the segment
+            phs[i] = (j >= 0 && j < a.n_ctl) ? pr[j] : 0.0f;
+        }
+    } else if (tid < kSegChunks) {
         const int chunk = seg * kSegChunks + tid;
         const float sr_down = (float)((double)a.sr / (double)kUpd);
         const float inc = a.rate[b] * (two_pi / sr_down);
@@ -818,14 +492,10 @@ using namespace modfx;
 extern "C" int64_t modfx_phaser_workspace_bytes(int32_t B, int64_t N) {
     if (B <= 0 || N <= 0) return 0;
     const int64_t n_ctl = (N + kUpd - 1) / kUpd, n_chunks = (N + kChunk - 1) / kChunk;
-    const int64_t multi = align_up((int64_t)B * n_ctl * 4, 256) + align_up((int64_t)B * n_chunks * kMapFloats * 4, 256) +
-                          align_up((int64_t)B * n_chunks * kSFloats * 4, 256) +
-                          align_up((int64_t)B * ((n_chunks + 31) / 32) * kMapFloats * 4, 256) +
-                          align_up((int64_t)B * ((n_chunks + 31) / 32) * kSFloats * 4, 256);
     const int64_t n_seg = (N + kSeg - 1) / kSeg;
-    const int64_t fused = 256 + align_up((int64_t)B * n_seg * 4, 256) + align_up((int64_t)B * n_seg * kRec * 4, 256) +
-                          align_up((int64_t)B * n_chunks * 8, 256);
-    return (multi > fused ? multi : fused) + 256;
+    const int64_t phase_bytes = (n_ctl * 4 > n_chunks * 8) ? n_ctl * 4 : n_chunks * 8;     // phc or ph, per row
+    return 256 + align_up((int64_t)B * n_seg * 4, 256) + align_up((int64_t)B * n_seg * kRec * 4, 256) +
+           align_up((int64_t)B * phase_bytes, 256) + 256;
 }
 
 namespace {
@@ -853,67 +523,24 @@ int phaser_launch(const float* x, int x_compact, const int64_t* x_offset, float*
     char* w = static_cast<char*>(workspace);
     const int n_blocks = (int)((N + block - 1) / block);
 
-    const char* force = getenv("MODFX_PHASER_KERNEL");
-    const bool fused_ok = (block % kChunk == 0) && !(force && force[0] == 'm');
-    if (fused_ok) {
-        // ---- single-pass fused kernel
-        FusedArgs f{};
-        f.a = a;
-        f.start = start; f.n_out = (int)n_out; f.dry_out = dry_out; f.x_compact = x_compact; f.x_offset = x_offset;
-        f.n_seg = (int)((N + kSeg - 1) / kSeg);
-        f.ticket = reinterpret_cast<int*>(w);                                     w += 256;
-        f.flags = reinterpret_cast<int*>(w);
-        const int64_t flag_bytes = align_up((int64_t)a.n_items * f.n_seg * 4, 256);  w += flag_bytes;
-        f.rec = reinterpret_cast<float*>(w);                                      w += align_up((int64_t)a.n_items * f.n_seg * kRec * 4, 256);
-        f.ph = reinterpret_cast<float2*>(w);
-        MODFX_CUDA_OK(cudaMemsetAsync(workspace, 0, (size_t)(256 + flag_bytes), s));
-        const int pairs = a.n_items * n_blocks;
-        phaser_phase_kernel<<<(pairs + 127) / 128, 128, 0, s>>>(f, n_blocks);
-        const size_t smem = sizeof(float) * (size_t)(kSubs * (kSub + 1) + kSubs * (kSubCtl + 1) + kSubs * (kMapFloats + 1) + kSubs * kSFloats +
-                                                     8 * (kMapFloats + 1) + 8 * kSFloats);
-        const int64_t tiles = (int64_t)a.n_items * f.n_seg;
-        MODFX_REQUIRE(tiles < (1ll << 31), "too many segments in one call");
-        phaser_fused_kernel<<<(unsigned)tiles, kFusedThreads, smem, s>>>(f);
-        MODFX_CUDA_OK(cudaGetLastError());
-        return MODFX_OK;
-    }
-    // ---- four-kernel pipeline (host blocks that are not a multiple of 128 samples; MODFX_PHASER_KERNEL=multi)
-    if (start || dry_out || n_out != N || x_compact || x_offset)
-        return fail(MODFX_ERR_UNSUPPORTED, "cropped output needs a host block size that is a multiple of %d samples", kChunk);
-    a.C = reinterpret_cast<float*>(w);
-    w += align_up((int64_t)a.n_items * a.n_ctl * 4, 256);
-    a.Mw = reinterpret_cast<float*>(w);
-    w += align_up((int64_t)a.n_items * a.n_chunks * kMapFloats * 4, 256);
-    a.S = reinterpret_cast<float*>(w);
-    w += align_up((int64_t)a.n_items * a.n_chunks * kSFloats * 4, 256);
-    {
-        const int total = a.n_items * n_blocks;
-        phaser_ctl_kernel<<<(total + 31) / 32, kK0Threads, 0, s>>>(a, n_blocks);
-    }
-    {
-        const int n_super = (a.n_chunks + 31) / 32;
-        phaser_map_kernel<<<(unsigned)((int64_t)a.n_items * n_super), kMapThreads, 0, s>>>(a, n_super);
-    }
-    if (a.n_chunks <= kSerialChainMax) {
-        // short clips (689 maps for 2 s): one serial chain per example is the cheapest
-        phaser_chain_kernel<<<(unsigned)(((int64_t)a.n_items * 8 + 255) / 256), 256, 0, s>>>(a.Mw, a.n_chunks, a.n_chunks,
-                                                                                          a.n_items, nullptr, a.S);
-    } else {
-        // long clips (20 672 maps for 60 s): compose groups in parallel, chain the groups, re-chain inside groups
-        const int n_groups = (a.n_chunks + kGroup - 1) / kGroup;
-        float* GM = reinterpret_cast<float*>(w);
-        w += align_up((int64_t)a.n_items * n_groups * kMapFloats * 4, 256);
-        float* GS = reinterpret_cast<float*>(w);
-        const int64_t teams = (int64_t)a.n_items * n_groups;
-        phaser_compose_kernel<<<(unsigned)((teams * 8 + 255) / 256), 256, 0, s>>>(a, n_groups, GM);
-        phaser_chain_kernel<<<(unsigned)(((int64_t)a.n_items * 8 + 255) / 256), 256, 0, s>>>(GM, n_groups, n_groups, a.n_items,
-                                                                                          nullptr, GS);
-        phaser_chain_kernel<<<(unsigned)((teams * 8 + 255) / 256), 256, 0, s>>>(a.Mw, a.n_chunks, kGroup, a.n_items, GS, a.S);
-    }
-    {
-        const int64_t warps = (int64_t)a.n_items * ((a.n_chunks + 31) / 32);
-        phaser_run_kernel<<<(unsigned)((warps + kRunWarps - 1) / kRunWarps), 32 * kRunWarps, 0, s>>>(a);
-    }
+    FusedArgs f{};
+    f.a = a;
+    f.start = start; f.n_out = (int)n_out; f.dry_out = dry_out; f.x_compact = x_compact; f.x_offset = x_offset;
+    f.n_seg = (int)((N + kSeg - 1) / kSeg);
+    f.ticket = reinterpret_cast<int*>(w);                                     w += 256;
+    f.flags = reinterpret_cast<int*>(w);
+    const int64_t flag_bytes = align_up((int64_t)a.n_items * f.n_seg * 4, 256);  w += flag_bytes;
+    f.rec = reinterpret_cast<float*>(w);                                      w += align_up((int64_t)a.n_items * f.n_seg * kRec * 4, 256);
+    if (block % kChunk == 0) f.ph = reinterpret_cast<float2*>(w);
+    else f.phc = reinterpret_cast<float*>(w);
+    MODFX_CUDA_OK(cudaMemsetAsync(workspace, 0, (size_t)(256 + flag_bytes), s));
+    const int pairs = a.n_items * n_blocks;
+    phaser_phase_kernel<<<(pairs + 127) / 128, 128, 0, s>>>(f, n_blocks);
+    const size_t smem = sizeof(float) * (size_t)(kSubs * (kSub + 1) + kSubs * (kSubCtl + 1) + kSubs * (kMapFloats + 1) + kSubs * kSFloats +
+                                                 8 * (kMapFloats + 1) + 8 * kSFloats);
+    const int64_t tiles = (int64_t)a.n_items * f.n_seg;
+    MODFX_REQUIRE(tiles < (1ll << 31), "too many segments in one call");
+    phaser_fused_kernel<<<(unsigned)tiles, kFusedThreads, smem, s>>>(f);
     MODFX_CUDA_OK(cudaGetLastError());
     return MODFX_OK;
 }

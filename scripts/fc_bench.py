@@ -1,8 +1,10 @@
-"""Device-time probe of the flanger / chorus kernels on the BASELINE shapes, old one-warp schedule against the
-warp-specialised CTA-per-delay-line kernel (MODFX_FC_KERNEL=warp forces the former), and a bit-equality check of the two.
+"""Device-time probe of the flanger / chorus kernels on the BASELINE shapes and on the in-kernel LFO sources (one value
+per sample, n_lo = N; a synthesised control row too long to stage in shared memory), with a digest of every output so
+that two builds (MODFX_LIB=...) can be compared bit for bit.
 
-    python scripts/fc_bench.py [c4] [c4s] [c3] [c5] [c1]
+    python scripts/fc_bench.py [c4] [c4s] [c3] [c5] [c1] [lfo]
 """
+import hashlib
 import math
 import os
 import sys
@@ -11,12 +13,12 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import torch
 from mod_extraction_b200.fx import MonoFlangerChorusModule
-from mod_extraction_b200.modulations import make_combined_mod_sig_batch, make_mod_signal_batch
+from mod_extraction_b200.modulations import SHAPE_ID, make_combined_mod_sig_batch, make_mod_signal_batch
 
 dev = torch.device("cuda", 0)
 SR = 44100
 SHAPES6 = ["cos", "tri", "rect_cos", "inv_rect_cos", "saw", "rsaw"]
-which = sys.argv[1:] or ["c1", "c4", "c4s", "c3", "c5"]
+which = sys.argv[1:] or ["c1", "c4", "c4s", "c3", "c5", "lfo"]
 
 
 def timed(fn, reps):
@@ -36,25 +38,28 @@ def white(B, N, seed):
     return (torch.rand((B, 1, N), device=dev, generator=g) * 2 - 1) * 0.5
 
 
-def run(name, B, N, lo, mmd=1.0, mld=10.0, mdw_lo=0.0, reps=10, seed=0):
+def run(name, B, N, lo=None, mmd=1.0, mld=10.0, mdw_lo=0.0, reps=10, seed=0, lfo=None):
+    """lo: (B, n_lo) control-rate row, or lfo: (n_lo, sr_lo) to synthesise the LFO in-kernel (forward_lfo)."""
     rng = np.random.RandomState(seed)
     x = white(B, N, seed + 1)
     U = lambda a, b: torch.from_numpy(rng.uniform(a, b, B).astype(np.float32)).to(dev)
     p = [U(0, 0.7), U(mdw_lo, 1.0), U(0.25, 1), U(0.25, 1), U(0.25, 1)]
     m = MonoFlangerChorusModule(B, 1, N, SR, mmd, mld, check_ranges=False)
-    outs = {}
-    for kern in ("warp", "cta"):
-        os.environ["MODFX_FC_KERNEL"] = kern
-        out = torch.empty_like(x)
-        t = timed(lambda: m.forward_control_rate(x, lo, *p, out=out), reps)
-        outs[kern] = out
-        gbs = B * N * 8 / (t * 1e-3) / 1e9
-        print(f"{name:34s} {kern:5s} B={B:5d} N={N:8d} {t:8.3f} ms  {B * N / SR / (t * 1e-3) / 1e6:7.3f} M audio-s/s  "
-              f"{gbs:7.1f} GB/s ({gbs / 6547.8 * 100:5.1f} %)", flush=True)
-    same = torch.equal(outs["warp"], outs["cta"])
-    print(f"{'':34s} outputs bit-identical: {same}", flush=True)
-    assert same
-    os.environ.pop("MODFX_FC_KERNEL", None)
+    out = torch.empty_like(x)
+    if lfo is None:
+        fn = lambda: m.forward_control_rate(x, lo, *p, out=out)
+    else:
+        n_lo, sr_lo = lfo
+        rate = torch.from_numpy(np.exp(rng.uniform(math.log(0.5), math.log(3.0), B)))
+        phase = torch.from_numpy(rng.uniform(0, 2 * math.pi, B))
+        shape = torch.tensor([SHAPE_ID[SHAPES6[b % 6]] for b in range(B)])
+        fn = lambda: m.forward_lfo(x, rate, phase, shape, n_lo=n_lo, sr_lo=sr_lo, feedback=p[0], min_delay_width=p[1],
+                                   width=p[2], depth=p[3], mix=p[4], out=out)
+    t = timed(fn, reps)
+    gbs = B * N * 8 / (t * 1e-3) / 1e9
+    digest = hashlib.sha256(out.cpu().numpy().tobytes()).hexdigest()[:16]
+    print(f"{name:38s} B={B:5d} N={N:8d} {t:8.3f} ms  {B * N / SR / (t * 1e-3) / 1e6:7.3f} M audio-s/s  "
+          f"{gbs:7.1f} GB/s ({gbs / 6547.8 * 100:5.1f} %)  output sha256 {digest}", flush=True)
 
 
 def plain_lfo(B, n_lo, rate_lo, rate_hi, exp, seed):
@@ -84,3 +89,6 @@ if "c3" in which:
 if "c5" in which:
     run("config 5 flanger 60 s x 512", 512, 2646000, plain_lfo(512, 26460, 0.5, 3.0, 1.0, 46), reps=3)
     run("config 5 flanger 60 s x 64 (8 GPUs)", 64, 2646000, plain_lfo(64, 26460, 0.5, 3.0, 1.0, 47), reps=3)
+if "lfo" in which:
+    run("in-kernel LFO, n_lo = N (512)", 512, 88200, lfo=(88200, float(SR)))
+    run("in-kernel LFO 60 s, 26 460-point row (512)", 512, 2646000, lfo=(26460, 441.0), reps=3)

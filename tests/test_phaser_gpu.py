@@ -33,6 +33,20 @@ def test_phaser_vs_own_oracle(family, N):
     assert err <= 1e-4 and snr_db(ref, y) >= 80.0, (family, N, float(err), snr_db(ref, y))
 
 
+@pytest.mark.parametrize("block", [1000, 130, 100, 384])
+def test_phaser_host_block_sizes(block):
+    """Host blocks other than pedalboard's 8192: 1000 is not a multiple of the 4-sample update period, 130 puts one block
+    boundary inside a 128-sample chunk, 100 several, 384 is a multiple of 128 whose boundaries fall inside segments."""
+    from mod_extraction_b200.phaser import Phaser
+    B, N = 32, 88200
+    x = white((B, N), 6)
+    ps = _params(B, block)
+    ref = oracle.phaser(x, 44100.0, *ps, block=block)
+    y = Phaser(44100.0, buffer_size=block)(torch.from_numpy(x).to(DEV), *[torch.from_numpy(p) for p in ps]).cpu().numpy()
+    err = np.abs(y - ref).max()
+    assert err <= 1e-4 and snr_db(ref, y) >= 80.0, (block, float(err), snr_db(ref, y))
+
+
 def test_phaser_extreme_parameters():
     from mod_extraction_b200.phaser import Phaser
     N = 30000
@@ -89,13 +103,22 @@ def test_phaser_render_step_follows_getitem_example_by_example():
     one extra LFO period rendered, random crop of dry / wet, ground-truth LFO cropped and resampled to n // 100 points.
     The restatement below walks the examples with the reference's scalar draws; the DSP is this repo's own phaser
     restatement (PARITY UNPINNED)."""
+    _check_render_step(8192)
+
+
+def test_phaser_render_step_odd_host_block():
+    """The same cropped render with a host block that is not a multiple of the 4-sample update period."""
+    _check_render_step(1000)
+
+
+def _check_render_step(buffer_size):
     from scipy.stats import loguniform
     from mod_extraction_b200.phaser import PhaserRenderStep
     cfg = {"pedalboard_phaser": {"rate_hz": {"min": 0.5, "max": 3.0}, "depth": {"min": 0.2, "max": 1.0},
                                  "centre_frequency_hz": {"min": 70.0, "max": 18000.0},
                                  "feedback": {"min": 0.0, "max": 0.7}, "mix": {"min": 0.2, "max": 1.0}}}
     sr, n, B = 44100.0, 22050, 7
-    step = PhaserRenderStep(cfg, n, sr)
+    step = PhaserRenderStep(cfg, n, sr, buffer_size=buffer_size)
     L = step.max_proc_n_samples
     assert L == n + 88200
     audio = white((B, 1, L), 31)
@@ -115,7 +138,7 @@ def test_phaser_render_step_follows_getitem_example_by_example():
         centre = float(loguniform.rvs(c["centre_frequency_hz"]["min"], c["centre_frequency_hz"]["max"], size=1)[0])
         feedback = (torch.rand(1) * (c["feedback"]["max"] - c["feedback"]["min"]) + c["feedback"]["min"]).item()
         mix = (torch.rand(1) * (c["mix"]["max"] - c["mix"]["min"]) + c["mix"]["min"]).item()
-        proc = oracle.phaser(chunk, sr, rate, depth, centre, feedback, mix)
+        proc = oracle.phaser(chunk, sr, rate, depth, centre, feedback, mix, block=buffer_size)
         gt = oracle.make_mod_signal(proc_n, sr, rate, np.pi / 2, "cos")                              # datasets.py:442
         start = torch.randint(low=0, high=proc_n - n + 1, size=(1,)).item()                         # datasets.py:445
         assert fx["rate_hz"][b].item() == rate and fx["depth"][b].item() == depth
