@@ -534,7 +534,9 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
                             const int kmin = __reduce_min_sync(kFull, mine ? kp : 0x7fffffff);
                             const int kmax = __reduce_max_sync(kFull, mine ? kp : 0);
                             unsigned code;
-                            if (nb + kWarp <= N && kmax - kmin <= 1 && kmin <= kSerialK && c.M >= 2 * kWarp) {
+                            // (M >= a tile: a K = 1 run takes the stale sample M back of each of its samples before it
+                            // starts, so that sample must precede the run, and a run covers up to a whole tile)
+                            if (nb + kWarp <= N && kmax - kmin <= 1 && kmin <= kSerialK && c.M >= kTile) {
                                 code = (unsigned)kmin;
                                 const bool sel = kp == kmin;        // tap distance K (else K + 1)
                                 float4 o;

@@ -185,24 +185,33 @@ def test_flanger_example_index_and_out():
             assert (got[b] == 7.0).all()
 
 
+# (max_min_delay_ms, max_lfo_delay_ms, lowest min_delay_width) of the fused-LFO tests: the flanger, and the chorus with
+# min_delay_width in [0, 1] -- a synthesised LFO never takes fc_wide_kernel, so chorus-length lines go through
+# fc_cta_kernel in each of its in-kernel LFO modes
+_FUSED_LFO_LINES = [(1.0, 10.0, 0.0), (30.0, 10.0, 0.0)]
+
+
 def test_flanger_fused_lfo_synthesis():
     """LFO params in, audio out: the LFO itself is within 1e-6 of the reference arithmetic
     (cos is not bit-identical across libms), so the audio is compared per shape family:
     bit-exact for the cos-free shapes, SNR-bounded for the cos shapes (SURVEY F3)."""
-    _check_fused_lfo(882, 441.0)            # the control row of the reference pipeline, staged in shared memory
+    for line in _FUSED_LFO_LINES:
+        _check_fused_lfo(882, 441.0, *line)     # the control row of the reference pipeline, staged in shared memory
 
 
 def test_flanger_fused_lfo_long_row():
     """Same comparison for a synthesised control row longer than the kernel stages: evaluated at the taps."""
-    _check_fused_lfo(8820, 4410.0)
+    for line in _FUSED_LFO_LINES:
+        _check_fused_lfo(8820, 4410.0, *line)
 
 
 def test_flanger_fused_lfo_direct():
     """Same comparison with one LFO value per sample (n_lo = N): no upsample."""
-    _check_fused_lfo(88200, float(SR))
+    for line in _FUSED_LFO_LINES:
+        _check_fused_lfo(88200, float(SR), *line)
 
 
-def _check_fused_lfo(n_lo, sr_lo):
+def _check_fused_lfo(n_lo, sr_lo, mmd, mld, mdw_lo):
     from mod_extraction_b200.fx import MonoFlangerChorusModule
     from mod_extraction_b200.modulations import SHAPE_ID
     rng = np.random.RandomState(23)
@@ -212,19 +221,19 @@ def _check_fused_lfo(n_lo, sr_lo):
     rate = np.exp(rng.uniform(np.log(0.5), np.log(3.0), B))
     phase = rng.uniform(0, 2 * math.pi, B)
     lo = np.stack([oracle.make_mod_signal(n_lo, sr_lo, rate[b], phase[b], shapes[b], 2.0) for b in range(B)])
-    params = _rand_params(B, rng)
-    ref = oracle.flanger_chorus(x, oracle.linear_interpolate_last_dim(lo, N), *params, max_min_delay_ms=1.0,
-                                max_lfo_delay_ms=10.0)
-    m = MonoFlangerChorusModule(B, 1, N, SR, 1.0, 10.0)
+    params = _rand_params(B, rng, mdw_lo)
+    ref = oracle.flanger_chorus(x, oracle.linear_interpolate_last_dim(lo, N), *params, max_min_delay_ms=mmd,
+                                max_lfo_delay_ms=mld)
+    m = MonoFlangerChorusModule(B, 1, N, SR, mmd, mld)
     y = m.forward_lfo(torch.from_numpy(x).to(dev()), torch.from_numpy(rate), torch.from_numpy(phase),
                       torch.tensor([SHAPE_ID[s] for s in shapes]), exp=torch.full((B,), 2.0), n_lo=n_lo, sr_lo=sr_lo,
                       feedback=to_t(params[0]), min_delay_width=to_t(params[1]), width=to_t(params[2]),
                       depth=to_t(params[3]), mix=to_t(params[4])).cpu().numpy()
     for b in range(B):
         if shapes[b] in ("tri", "saw", "rsaw"):
-            assert np.array_equal(y[b], ref[b]), shapes[b]
+            assert np.array_equal(y[b], ref[b]), (mmd, shapes[b])
         else:
-            assert np.abs(y[b] - ref[b]).max() <= 1e-4 and snr_db(ref[b], y[b]) >= 80.0, shapes[b]
+            assert np.abs(y[b] - ref[b]).max() <= 1e-4 and snr_db(ref[b], y[b]) >= 80.0, (mmd, shapes[b])
 
 
 # --------------------------------------------------------------------------- E2, L1, L2, U1
