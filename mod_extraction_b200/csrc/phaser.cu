@@ -101,7 +101,9 @@ __device__ __forceinline__ void cascade_retune2(float2 (&w)[kStagesAP], float c_
 //   E  64 threads re-run their sub-chunk from its true entry state, mix, clip;
 //   F  coalesced store -- optionally only the window [start[b], start[b] + n_out) of the row, together with the same
 //      window of the dry input: the random crop of PedalboardPhaserDataset.__getitem__ (datasets.py:445-447).
-// Segments past the last needed sample are never touched.  HBM traffic: 4 B in + 4 B out per sample + 64 B per segment.
+// Segments past the last needed sample are never touched; a segment wholly before the window ends once its exit state
+// is published (no E, no stores).  HBM traffic: 4 B in + 4 B out per sample + 64 B per segment.
+// Shared memory is kept under 37.8 KB so that 6 CTAs fit an SM, which the 40 registers of a thread also allow.
 constexpr int kSegChunks = 32;                       // 128-sample chunks per segment
 constexpr int kSeg = kSegChunks * kChunk;            // 4096 samples
 constexpr int kSub = 64;                             // samples per scan sub-chunk
@@ -109,7 +111,11 @@ constexpr int kSubs = kSeg / kSub;                   // 64 sub-chunks per segmen
 constexpr int kSubCtl = kSub / kUpd;                 // 16 control points per sub-chunk
 constexpr int kSegCtl = kSeg / kUpd;                 // 1024
 constexpr int kFusedThreads = 256;
+constexpr int kFusedCtasPerSM = 6;
 constexpr int kRec = 8;                              // published state record: w1..w6, lastOutput, c the states are scaled for
+constexpr int kFusedSmemFloats = kSubs * (kSub + 1) + kSubs * (kSubCtl + 1) + kSubs * (kMapFloats + 1) + kSubs * kSFloats;
+// (+ 1 KB per CTA reserved by the runtime, + the few static bytes, within the 228 KB of an SM)
+static_assert(kFusedCtasPerSM * (kFusedSmemFloats * 4 + 128 + 1024) <= 228 * 1024, "phaser_fused_kernel: 6 CTAs per SM");
 
 struct FusedArgs {
     PhaserArgs a;
@@ -209,7 +215,24 @@ __device__ __forceinline__ float phaser_coef(float phase, float vol, float ctr, 
     return 2.0f * (g / (1.0f + g)) - 1.0f;
 }
 
-__global__ void __launch_bounds__(kFusedThreads) phaser_fused_kernel(const FusedArgs f) {
+// Stores samples [lo, hi) of a segment (sample n in xs at n - n_base) to row[n - start]: float4 stores where row + (n - start)
+// is 16-byte aligned, scalar stores for the at most 3 + 3 samples at the ends (with start % 4 != 0 a float4 there would
+// straddle the neighbouring segment, which another CTA stores).
+__device__ __forceinline__ void store_window(float* row, const float (*xs)[kSub + 1], int n_base, int start, int lo, int hi,
+                                             int tid) {
+    const auto at = [&](int n) { const unsigned i = n - n_base; return xs[i / kSub][i % kSub]; };
+    if ((reinterpret_cast<uintptr_t>(row) & 15) != 0) {
+        for (int n = lo + tid; n < hi; n += kFusedThreads) row[n - start] = at(n);
+        return;
+    }
+    const int v0 = min(lo + ((start - lo) & 3), hi), v1 = max(hi - ((hi - start) & 3), v0);
+    for (int n = v0 + 4 * tid; n < v1; n += 4 * kFusedThreads)
+        *reinterpret_cast<float4*>(row + (n - start)) = make_float4(at(n), at(n + 1), at(n + 2), at(n + 3));
+    if (tid < v0 - lo) row[lo + tid - start] = at(lo + tid);
+    if (tid < hi - v1) row[v1 + tid - start] = at(v1 + tid);
+}
+
+__global__ void __launch_bounds__(kFusedThreads, kFusedCtasPerSM) phaser_fused_kernel(const FusedArgs f) {
     extern __shared__ __align__(16) float sm[];
     float(*xs)[kSub + 1] = reinterpret_cast<float(*)[kSub + 1]>(sm);                        // [64][65] audio, then output
     float(*cs)[kSubCtl + 1] = reinterpret_cast<float(*)[kSubCtl + 1]>(sm + kSubs * (kSub + 1));   // [64][17] col 0: coefficient before
@@ -218,6 +241,7 @@ __global__ void __launch_bounds__(kFusedThreads) phaser_fused_kernel(const Fused
     float* phs = reinterpret_cast<float*>(Ms);                           // [1024 + 1] phases (dead before the maps are written)
     __shared__ int tile_s;
     __shared__ float entry[kRec];
+    __shared__ float coef_k[5];                                          // log_min, log_span, w0, vol, ctr of phaser_coef
     const PhaserArgs& a = f.a;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (tid == 0) tile_s = atomicAdd(f.ticket, 1);
@@ -247,6 +271,16 @@ __global__ void __launch_bounds__(kFusedThreads) phaser_fused_kernel(const Fused
             const int n = n_base + i;
             xs[i / kSub][i % kSub] = (n < row_len) ? __ldg(xr + n) : 0.0f;
         }
+    }
+    if (tid == kFusedThreads - 1) {                                       // the per-example constants of B, once per CTA
+        const float f_lo = 20.0f;
+        const double f_hi_d = (0.49 * (double)a.sr < 20000.0) ? 0.49 * (double)a.sr : 20000.0;
+        const float log_min = log10f(f_lo), log_span = log10f((float)f_hi_d) - log_min;
+        coef_k[0] = log_min;
+        coef_k[1] = log_span;
+        coef_k[2] = MODFX_PI_F / a.sr;
+        coef_k[3] = a.depth[b] * 0.5f;
+        coef_k[4] = (log10f(a.centre[b]) - log_min) / log_span;
     }
     const float two_pi = MODFX_TWO_PI_F;
     if (f.phc) {                                                          // precomputed: copy them
@@ -280,12 +314,7 @@ __global__ void __launch_bounds__(kFusedThreads) phaser_fused_kernel(const Fused
     __syncthreads();
     // ---- B: phase -> all-pass coefficient
     {
-        const float f_lo = 20.0f;
-        const double f_hi_d = (0.49 * (double)a.sr < 20000.0) ? 0.49 * (double)a.sr : 20000.0;
-        const float log_min = log10f(f_lo), log_span = log10f((float)f_hi_d) - log_min;
-        const float w0 = MODFX_PI_F / a.sr;
-        const float vol = a.depth[b] * 0.5f;
-        const float ctr = (log10f(a.centre[b]) - log_min) / log_span;
+        const float log_min = coef_k[0], log_span = coef_k[1], w0 = coef_k[2], vol = coef_k[3], ctr = coef_k[4];
         float cv[(kSegCtl + 1 + kFusedThreads - 1) / kFusedThreads];
 #pragma unroll
         for (int k = 0; k < (kSegCtl + 1 + kFusedThreads - 1) / kFusedThreads; ++k) {
@@ -351,18 +380,18 @@ __global__ void __launch_bounds__(kFusedThreads) phaser_fused_kernel(const Fused
     // Three short passes instead of one chain of 64 dependent steps: (1) every warp composes the 8 maps of its group
     // into one, all groups at once; (2) warp 0 takes the segment's entry state from the previous segment's CTA and
     // chains the 8 group maps; (3) every warp chains its 8 sub-chunks from its group's entry state.
-    float(*GM)[kMapFloats + 1] = reinterpret_cast<float(*)[kMapFloats + 1]>(Ss + kSubs);       // [8][57] group maps
-    float(*GS)[kSFloats] = reinterpret_cast<float(*)[kSFloats]>(reinterpret_cast<float*>(GM) + 8 * (kMapFloats + 1));   // [8][8]
+    // Pass 3 never reads the last map of a group (it would give the next group's entry), so pass 1 leaves the group map
+    // in that row, and pass 2 leaves a group's entry state in the state row of its first sub-chunk.
     {
-        // (1) lane = (row i = lane >> 3 and i + 4, column r = lane & 7) of the running product [Phi | z]
+        // (1) lane = (row i = lane >> 3 and i + 4, column r = lane & 7) of the running product [Phi | z], in registers;
+        // element (j, r) is in lane ((j & 3) << 3) | r
         const int r = lane & 7, i0 = lane >> 3, i1 = i0 + 4;
-        float* g = GM[warp];
+        float g0, g1;
         {
             const float* m = Ms[warp * 8];
-            g[r * kState + i0] = m[r * kState + i0];
-            if (i1 < kState) g[r * kState + i1] = m[r * kState + i1];
+            g0 = m[r * kState + i0];
+            g1 = (i1 < kState) ? m[r * kState + i1] : 0.0f;
         }
-        __syncwarp();
 #pragma unroll 1
         for (int k = 1; k < 8; ++k) {
             const float* m = Ms[warp * 8 + k];
@@ -370,15 +399,17 @@ __global__ void __launch_bounds__(kFusedThreads) phaser_fused_kernel(const Fused
             float a1 = (r == 7 && i1 < kState) ? m[7 * kState + i1] : 0.0f;
 #pragma unroll
             for (int j = 0; j < kState; ++j) {
-                const float cj = g[r * kState + j];
+                const float cj = __shfl_sync(0xffffffffu, (j < 4) ? g0 : g1, ((j & 3) << 3) | r);
                 a0 = fmaf(m[j * kState + i0], cj, a0);
                 if (i1 < kState) a1 = fmaf(m[j * kState + i1], cj, a1);
             }
-            __syncwarp();
-            g[r * kState + i0] = a0;
-            if (i1 < kState) g[r * kState + i1] = a1;
-            __syncwarp();
+            g0 = a0;
+            g1 = a1;
         }
+        __syncwarp();                                                     // every lane is done with the group's last map
+        float* g = Ms[warp * 8 + 7];
+        g[r * kState + i0] = g0;
+        if (i1 < kState) g[r * kState + i1] = g1;
     }
     __syncthreads();
     if (warp == 0) {
@@ -401,8 +432,8 @@ __global__ void __launch_bounds__(kFusedThreads) phaser_fused_kernel(const Fused
         if (lane < 8) {
 #pragma unroll 1
             for (int gq = 0; gq < 8; ++gq) {
-                GS[gq][i] = sv;
-                const float* m = GM[gq];
+                Ss[gq * 8][i] = sv;
+                const float* m = Ms[gq * 8 + 7];
                 float acc = m[7 * kState + ii];
 #pragma unroll
                 for (int r = 0; r < kState; ++r) acc = fmaf(m[r * kState + ii], __shfl_sync(0xffu, sv, r, 8), acc);
@@ -415,28 +446,26 @@ __global__ void __launch_bounds__(kFusedThreads) phaser_fused_kernel(const Fused
         __syncwarp();
         if (lane == 0) atomicExch(f.flags + (int64_t)item * f.n_seg + seg, 1);
     }
+    // a segment wholly before the window owed its successor the exit state, nothing else (CTA-uniform)
+    if (n_base + kSeg <= start) return;
+    // delivered samples of this segment: [lo, hi)
+    const int lo = max(n_base, start), hi = min(n_base + kSeg, need);
     // the window of the dry input goes out while warp 0 chains (xs still holds the audio)
-    if (f.dry_out) {
-        float* dr = f.dry_out + (int64_t)b * f.n_out;
-        for (int i = tid; i < kSeg; i += kFusedThreads) {
-            const int idx = n_base + i - start;
-            if (idx >= 0 && idx < f.n_out && n_base + i < row_len) dr[idx] = xs[i / kSub][i % kSub];
-        }
-    }
+    if (f.dry_out) store_window(f.dry_out + (int64_t)b * f.n_out, xs, n_base, start, lo, hi, tid);
     __syncthreads();
     // (3) entry state of every sub-chunk: each warp chains its group (8 lanes, lane i < 7 owns state component i)
     if (lane < 8) {
         const int i = lane, ii = (i < kState) ? i : 0;
-        float sv = (i < kState) ? GS[warp][i] : 0.0f;
+        float sv = (i < kState) ? Ss[warp * 8][i] : 0.0f;
 #pragma unroll 1
-        for (int k = 0; k < 8; ++k) {
+        for (int k = 0; k < 7; ++k) {
             const int sc = warp * 8 + k;
-            Ss[sc][i] = sv;
             const float* m = Ms[sc];
             float acc = m[7 * kState + ii];
 #pragma unroll
             for (int r = 0; r < kState; ++r) acc = fmaf(m[r * kState + ii], __shfl_sync(0xffu, sv, r, 8), acc);
             sv = (i < kState) ? acc : 0.0f;
+            Ss[sc + 1][i] = sv;
         }
     }
     __syncthreads();
@@ -466,7 +495,7 @@ __global__ void __launch_bounds__(kFusedThreads) phaser_fused_kernel(const Fused
     __syncthreads();
     // ---- F: coalesced store of the delivered window
     float* yr = a.y + (int64_t)b * f.n_out;
-    if (vec && start == 0 && n_base + kSeg <= f.n_out && ((reinterpret_cast<uintptr_t>(yr) & 15) == 0)) {
+    if (start == 0 && n_base + kSeg <= f.n_out && ((reinterpret_cast<uintptr_t>(yr) & 15) == 0)) {
 #pragma unroll
         for (int k = 0; k < kSeg / 4 / kFusedThreads; ++k) {
             const int i4 = tid + k * kFusedThreads;
@@ -474,11 +503,7 @@ __global__ void __launch_bounds__(kFusedThreads) phaser_fused_kernel(const Fused
             reinterpret_cast<float4*>(yr + n_base)[i4] = make_float4(d[0], d[1], d[2], d[3]);
         }
     } else {
-        for (int i = tid; i < kSeg; i += kFusedThreads) {
-            const int n = n_base + i;
-            const int idx = n - start;
-            if (idx >= 0 && idx < f.n_out && n < a.N) yr[idx] = xs[i / kSub][i % kSub];
-        }
+        store_window(yr, xs, n_base, start, lo, hi, tid);
     }
 }
 
@@ -536,11 +561,11 @@ int phaser_launch(const float* x, int x_compact, const int64_t* x_offset, float*
     MODFX_CUDA_OK(cudaMemsetAsync(workspace, 0, (size_t)(256 + flag_bytes), s));
     const int pairs = a.n_items * n_blocks;
     phaser_phase_kernel<<<(pairs + 127) / 128, 128, 0, s>>>(f, n_blocks);
-    const size_t smem = sizeof(float) * (size_t)(kSubs * (kSub + 1) + kSubs * (kSubCtl + 1) + kSubs * (kMapFloats + 1) + kSubs * kSFloats +
-                                                 8 * (kMapFloats + 1) + 8 * kSFloats);
     const int64_t tiles = (int64_t)a.n_items * f.n_seg;
     MODFX_REQUIRE(tiles < (1ll << 31), "too many segments in one call");
-    phaser_fused_kernel<<<(unsigned)tiles, kFusedThreads, smem, s>>>(f);
+    MODFX_CUDA_OK(cudaFuncSetAttribute(phaser_fused_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                       cudaSharedmemCarveoutMaxShared));
+    phaser_fused_kernel<<<(unsigned)tiles, kFusedThreads, sizeof(float) * kFusedSmemFloats, s>>>(f);
     MODFX_CUDA_OK(cudaGetLastError());
     return MODFX_OK;
 }
