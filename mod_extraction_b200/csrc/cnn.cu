@@ -335,12 +335,15 @@ extern "C" int modfx_cnn_layernorm_f32(const float* x, float* y, int32_t B, int3
 template <int kCin, int kCk>
 static int launch_conv_fp32(const float* x, float* y, int B, int H, int W, int dil, const float* weight,
                             const float* bias, const float* prelu, cudaStream_t st) {
-    const size_t smem = sizeof(ConvSmem<kCk>);
-    MODFX_CUDA_OK(cudaFuncSetAttribute(conv_fp32_kernel<kCin, kCk>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)smem));
-    conv_fp32_kernel<kCin, kCk><<<dim3((W + kTw - 1) / kTw, H / 2, B), kConvThreads, smem, st>>>(x, y, H, W, dil, weight,
-                                                                                                 bias, prelu);
-    MODFX_CUDA_OK(cudaGetLastError());
+    return launch(conv_fp32_kernel<kCin, kCk>, dim3((W + kTw - 1) / kTw, H / 2, B), kConvThreads, sizeof(ConvSmem<kCk>), st,
+                  x, y, H, W, dil, weight, bias, prelu);
+}
+
+// The limits every convolution entry point shares.  An empty batch passes them: the caller returns before launching.
+static int check_conv_shape(int B, int H, int dil_w) {
+    if ((H & 1) || dil_w < 1 || dil_w > kMaxDil)
+        return fail(MODFX_ERR_UNSUPPORTED, "H=%d must be even and the time dilation %d in [1, %d]", H, dil_w, kMaxDil);
+    if (B > 0) MODFX_REQUIRE(B <= 65535 && H / 2 <= 65535, "grid too large");
     return MODFX_OK;
 }
 
@@ -354,10 +357,7 @@ extern "C" int modfx_cnn_conv_pool_prelu_f32(const float* x, float* y, int32_t B
     if (KH != kKH || KW != kKW || Cout != kCo)
         return fail(MODFX_ERR_UNSUPPORTED, "only 5x13 kernels with 64 output channels are built (got %dx%d, %d)", KH, KW,
                     Cout);
-    if ((H & 1) || dil_w < 1 || dil_w > kMaxDil)
-        return fail(MODFX_ERR_UNSUPPORTED, "H=%d must be even and the time dilation %d in [1, %d]", H, dil_w, kMaxDil);
-    if (B == 0) return MODFX_OK;
-    MODFX_REQUIRE(B <= 65535 && H / 2 <= 65535, "grid too large");
+    if (const int st = check_conv_shape(B, H, dil_w); st != MODFX_OK || B == 0) return st;
     cudaStream_t st = as_stream(stream);
     if (precision == MODFX_CNN_TF32) {
         if (Cin == 2 && dil_w == 1) return cnn_conv1_tf32(x, y, B, H, W, weight, bias, prelu, st);
@@ -378,10 +378,7 @@ extern "C" int modfx_cnn_conv_pool_prelu_tf32x3_f32(const float* x_hi, const flo
     MODFX_REQUIRE(x_hi && x_lo && y && w_hi && w_lo && bias && prelu, "NULL pointer");
     MODFX_REQUIRE(B >= 0 && H >= 2 && W >= 1, "bad shape B=%d H=%d W=%d", B, H, W);
     MODFX_REQUIRE(x_hi != y && x_lo != y, "x and y must not alias");
-    if ((H & 1) || dil_w < 1 || dil_w > kMaxDil)
-        return fail(MODFX_ERR_UNSUPPORTED, "H=%d must be even and the time dilation %d in [1, %d]", H, dil_w, kMaxDil);
-    if (B == 0) return MODFX_OK;
-    MODFX_REQUIRE(B <= 65535 && H / 2 <= 65535, "grid too large");
+    if (const int st = check_conv_shape(B, H, dil_w); st != MODFX_OK || B == 0) return st;
     return cnn_conv_tf32(x_hi, x_lo, y, B, H, W, dil_w, w_hi, w_lo, bias, prelu, false, as_stream(stream));
 }
 
@@ -391,10 +388,7 @@ extern "C" int modfx_cnn_conv_pool_prelu_f16_f32(const void* x_f16, float* y, in
     MODFX_REQUIRE(x_f16 && y && w_f16 && bias && prelu, "NULL pointer");
     MODFX_REQUIRE(B >= 0 && H >= 2 && W >= 1, "bad shape B=%d H=%d W=%d", B, H, W);
     MODFX_REQUIRE(x_f16 != (const void*)y, "x and y must not alias");
-    if ((H & 1) || dil_w < 1 || dil_w > kMaxDil)
-        return fail(MODFX_ERR_UNSUPPORTED, "H=%d must be even and the time dilation %d in [1, %d]", H, dil_w, kMaxDil);
-    if (B == 0) return MODFX_OK;
-    MODFX_REQUIRE(B <= 65535 && H / 2 <= 65535, "grid too large");
+    if (const int st = check_conv_shape(B, H, dil_w); st != MODFX_OK || B == 0) return st;
     return cnn_conv_tf32(x_f16, nullptr, y, B, H, W, dil_w, w_f16, nullptr, bias, prelu, true, as_stream(stream));
 }
 
@@ -405,10 +399,6 @@ extern "C" int modfx_cnn_head_f32(const float* x, float* latent, float* out, int
     if (C > 1024) return fail(MODFX_ERR_UNSUPPORTED, "C=%d too large", C);
     if (B == 0) return MODFX_OK;
     MODFX_REQUIRE(B <= 65535, "B too large");
-    const size_t smem = (size_t)C * (kHeadW + 1) * sizeof(float);
-    MODFX_CUDA_OK(cudaFuncSetAttribute(head_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    head_kernel<<<dim3((W + kHeadW - 1) / kHeadW, B), 256, smem, as_stream(stream)>>>(x, latent, out, H, W, C, L, weight,
-                                                                                     bias);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    return launch(head_kernel, dim3((W + kHeadW - 1) / kHeadW, B), 256, (size_t)C * (kHeadW + 1) * sizeof(float),
+                  as_stream(stream), x, latent, out, H, W, C, L, weight, bias);
 }

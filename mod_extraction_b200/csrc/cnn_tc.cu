@@ -674,18 +674,10 @@ int cnn_conv_tf32(const void* x, const void* x_lo, float* y, int B, int H, int W
     st = make_maps(enc, &tm.x[1], &tm.w[1], split ? x_lo : x, split ? w_lo : weight, B, H, W, half);
     if (st != MODFX_OK) return st;
     const dim3 grid((W + kTileW - 1) / kTileW, (H + kRows - 1) / kRows, B);
-    if (half) {
-        MODFX_CUDA_OK(cudaFuncSetAttribute(conv_tf32_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           Fmt<true>::kSmemBytes));
-        conv_tf32_kernel<true><<<grid, kThreads, Fmt<true>::kSmemBytes, stream>>>(tm, 1, y, H, W, dil, bias, prelu);
-    } else {
-        MODFX_CUDA_OK(cudaFuncSetAttribute(conv_tf32_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           Fmt<false>::kSmemBytes));
-        conv_tf32_kernel<false><<<grid, kThreads, Fmt<false>::kSmemBytes, stream>>>(tm, split ? 3 : 1, y, H, W, dil, bias,
-                                                                                   prelu);
-    }
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    if (half)
+        return launch(conv_tf32_kernel<true>, grid, kThreads, Fmt<true>::kSmemBytes, stream, tm, 1, y, H, W, dil, bias, prelu);
+    return launch(conv_tf32_kernel<false>, grid, kThreads, Fmt<false>::kSmemBytes, stream, tm, split ? 3 : 1, y, H, W, dil,
+                  bias, prelu);
 }
 
 int cnn_conv1_tf32(const float* x, float* y, int B, int H, int W, const float* weight, const float* bias,
@@ -693,13 +685,10 @@ int cnn_conv1_tf32(const float* x, float* y, int B, int H, int W, const float* w
     MODFX_REQUIRE((reinterpret_cast<uintptr_t>(x) & 7) == 0 && (reinterpret_cast<uintptr_t>(weight) & 7) == 0 &&
                       (reinterpret_cast<uintptr_t>(y) & 15) == 0,
                   "x and weight must be 8-byte, y 16-byte aligned");
-    MODFX_CUDA_OK(cudaFuncSetAttribute(conv1_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes1));
     MODFX_CUDA_OK(cudaFuncSetAttribute(conv1_tf32_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                                        cudaSharedmemCarveoutMaxShared));
-    conv1_tf32_kernel<<<dim3((W + kTileW - 1) / kTileW, (H + kRows1 - 1) / kRows1, B), kThreads1, kSmemBytes1, stream>>>(
-        x, y, H, W, weight, bias, prelu);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    return launch(conv1_tf32_kernel, dim3((W + kTileW - 1) / kTileW, (H + kRows1 - 1) / kRows1, B), kThreads1, kSmemBytes1,
+                  stream, x, y, H, W, weight, bias, prelu);
 }
 
 }  // namespace modfx

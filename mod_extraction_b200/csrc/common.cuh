@@ -27,6 +27,19 @@ int fail(modfx_status st, const char* fmt, ...);
 
 inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
+// kernel<<<grid, block, smem, stream>>>(args...), opting in first when smem exceeds the default 48 KB.  That default
+// covers static and dynamic shared memory together, but only the dynamic size is tested here: the kernels launched
+// through this use no static shared memory except fc_wide_kernel's 32 B, and its dynamic size is a power of two, never
+// within 32 B of 48 KB.  A kernel that gains static shared memory must count it.
+template <typename... Params, typename... Args>
+int launch(void (*kernel)(Params...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
+    if (smem > 48 * 1024)
+        MODFX_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, block, smem, stream>>>(args...);
+    MODFX_CUDA_OK(cudaGetLastError());
+    return MODFX_OK;
+}
+
 constexpr int kWarp = 32;
 constexpr unsigned kFull = 0xffffffffu;
 

@@ -867,7 +867,9 @@ int next_pow2(int v) {
     return p;
 }
 
-int fill_mod(FcArgs& a, const modfx_mod_source* mod, int B, int64_t N, int& mode) {
+constexpr size_t kMaxSmem = 200 * 1024;    // dynamic shared memory an effect kernel may take; larger requests are refused
+
+int fill_mod(FcArgs& a, const modfx_mod_source* mod, int64_t N, int& mode) {
     MODFX_REQUIRE(mod != nullptr, "mod source is NULL");
     a.mod = mod->mod;
     a.mod_has_ch = mod->mod_has_ch;
@@ -911,7 +913,6 @@ int fill_mod(FcArgs& a, const modfx_mod_source* mod, int B, int64_t N, int& mode
         default:
             return fail(MODFX_ERR_INVALID, "unknown mod kind %d", mod->kind);
     }
-    (void)B;
     return MODFX_OK;
 }
 
@@ -921,6 +922,48 @@ int check_scalar(const modfx_param& p, const char* name, bool can_be_one) {
     MODFX_REQUIRE(p.value >= 0.0, "%s=%g must be >= 0", name, p.value);
     if (can_be_one) MODFX_REQUIRE(p.value <= 1.0, "%s=%g must be <= 1", name, p.value);
     else MODFX_REQUIRE(p.value < 1.0, "%s=%g must be < 1", name, p.value);
+    return MODFX_OK;
+}
+
+enum FcEffect { kLinearDelay, kAllpassDelay, kTremolo };
+
+struct FcParams { modfx_param feedback, min_delay_width, width, depth, mix; };    // tremolo takes mix alone
+
+// Validates the arguments of one entry point, in an order that gives every refusal its status and message, and fills
+// `a` and the modulation mode.  a.n_items == 0 on success: nothing to render.
+int fc_setup(FcArgs& a, int& mode, FcEffect fx, const float* x, float* y, int32_t B, int32_t C, int64_t N, int32_t Mmin,
+             int32_t Mlfo, const modfx_mod_source* mod, const FcParams& p, const int32_t* example_index, int32_t n_items) {
+    a = FcArgs{};
+    MODFX_REQUIRE(x && y, "x / y is NULL");
+    // the linear delay line names an over-long N on its own; the other two count it as a bad shape
+    MODFX_REQUIRE(B >= 0 && C >= 1 && N >= 1 && (fx == kLinearDelay || N < (1ll << 30)), "bad shape B=%d C=%d N=%lld", B,
+                  C, (long long)N);
+    MODFX_REQUIRE(N < (1ll << 30), "N=%lld too long (max 2^30-1 samples)", (long long)N);
+    int st;
+    if (fx != kTremolo) {
+        MODFX_REQUIRE(Mmin >= 0 && Mlfo >= 0 && Mmin + Mlfo >= 1, "bad delay line Mmin=%d Mlfo=%d", Mmin, Mlfo);
+        if ((st = check_scalar(p.feedback, "feedback", false)) != MODFX_OK) return st;          // fx.py:86
+        if ((st = check_scalar(p.min_delay_width, "min_delay_width", true)) != MODFX_OK) return st;
+        if ((st = check_scalar(p.width, "width", true)) != MODFX_OK) return st;
+        if ((st = check_scalar(p.depth, "depth", true)) != MODFX_OK) return st;
+    }
+    if ((st = check_scalar(p.mix, "mix", true)) != MODFX_OK) return st;                          // fx.py:21
+    a.x = x; a.y = y; a.B = B; a.C = C; a.N = (int)N;
+    a.Mmin = Mmin; a.Mlfo = Mlfo; a.M = Mmin + Mlfo;
+    if ((st = fill_mod(a, mod, N, mode)) != MODFX_OK) return st;
+    if (fx == kAllpassDelay) {
+        if (mode == kDirectLfo || a.lfo_freq)
+            return fail(MODFX_ERR_UNSUPPORTED, "all-pass interpolation takes the modulation signal from memory (audio or control rate)");
+        if (mode == kAudioRate) a.n_lo = 0;
+    }
+    a.fb_p = p.feedback.dev;         a.fb_s = (float)p.feedback.value;
+    a.mdw_p = p.min_delay_width.dev; a.min_delay_s = (float)(p.min_delay_width.value * (double)Mmin);
+    a.width_p = p.width.dev;         a.lfo_delay_s = (float)((double)Mlfo * p.width.value);
+    a.depth_p = p.depth.dev;         a.depth_s = (float)p.depth.value;
+    a.mix_p = p.mix.dev;             a.mix_s = (float)p.mix.value; a.omm_s = (float)(1.0 - p.mix.value);
+    a.index = example_index;
+    a.n_items = example_index ? n_items : B;
+    MODFX_REQUIRE(a.n_items >= 0, "n_items=%d", a.n_items);
     return MODFX_OK;
 }
 
@@ -934,33 +977,14 @@ extern "C" int modfx_flanger_chorus_f32(const float* x, float* y, int32_t B, int
                                         modfx_param feedback, modfx_param min_delay_width, modfx_param width,
                                         modfx_param depth, modfx_param mix, const int32_t* example_index,
                                         int32_t n_items, void* stream) {
-    MODFX_REQUIRE(x && y, "x / y is NULL");
-    MODFX_REQUIRE(B >= 0 && C >= 1 && N >= 1, "bad shape B=%d C=%d N=%lld", B, C, (long long)N);
-    MODFX_REQUIRE(N < (1ll << 30), "N=%lld too long (max 2^30-1 samples)", (long long)N);
-    MODFX_REQUIRE(Mmin >= 0 && Mlfo >= 0 && Mmin + Mlfo >= 1, "bad delay line Mmin=%d Mlfo=%d", Mmin, Mlfo);
-    int st;
-    if ((st = check_scalar(feedback, "feedback", false)) != MODFX_OK) return st;          // fx.py:86
-    if ((st = check_scalar(min_delay_width, "min_delay_width", true)) != MODFX_OK) return st;
-    if ((st = check_scalar(width, "width", true)) != MODFX_OK) return st;
-    if ((st = check_scalar(depth, "depth", true)) != MODFX_OK) return st;
-    if ((st = check_scalar(mix, "mix", true)) != MODFX_OK) return st;
-
-    FcArgs a{};
-    a.x = x; a.y = y; a.B = B; a.C = C; a.N = (int)N;
-    a.Mmin = Mmin; a.Mlfo = Mlfo; a.M = Mmin + Mlfo;
-    int mode = 0;
-    if ((st = fill_mod(a, mod, B, N, mode)) != MODFX_OK) return st;
+    FcArgs a;
+    int mode = 0, st;
+    if ((st = fc_setup(a, mode, kLinearDelay, x, y, B, C, N, Mmin, Mlfo, mod,
+                       {feedback, min_delay_width, width, depth, mix}, example_index, n_items)) != MODFX_OK ||
+        a.n_items == 0)
+        return st;
     const int ring = next_pow2(a.M + kTile);
     a.ring_mask = ring - 1;
-    a.fb_p = feedback.dev;         a.fb_s = (float)feedback.value;
-    a.mdw_p = min_delay_width.dev; a.min_delay_s = (float)(min_delay_width.value * (double)Mmin);
-    a.width_p = width.dev;         a.lfo_delay_s = (float)((double)Mlfo * width.value);
-    a.depth_p = depth.dev;         a.depth_s = (float)depth.value;
-    a.mix_p = mix.dev;             a.mix_s = (float)mix.value; a.omm_s = (float)(1.0 - mix.value);
-    a.index = example_index;
-    a.n_items = example_index ? n_items : B;
-    if (a.n_items == 0) return MODFX_OK;
-    MODFX_REQUIRE(a.n_items > 0, "n_items=%d", a.n_items);
 
     // The CTA-per-delay-line kernel renders every modulation source; a control row synthesised in-kernel is staged in
     // shared memory up to kLoSmemMax points and evaluated at the taps beyond that.
@@ -969,7 +993,7 @@ extern "C" int modfx_flanger_chorus_f32(const float* x, float* y, int32_t B, int
     const size_t csmem = sizeof(float) * (16 + (size_t)kNT * kSlotFloats +
                                           (size_t)kCtaProd * kXDepth * kTile * (mode == kAudioRate ? 2 : 1) +
                                           (size_t)lo_smem + (size_t)ring);
-    if (csmem > 200 * 1024)
+    if (csmem > kMaxSmem)
         return fail(MODFX_ERR_UNSUPPORTED, "delay line of %d samples needs %zu B of shared memory", a.M, csmem);
     const dim3 grid((unsigned)((int64_t)a.n_items * C));
     cudaStream_t s = as_stream(stream);
@@ -979,28 +1003,18 @@ extern "C" int modfx_flanger_chorus_f32(const float* x, float* y, int32_t B, int
     if (mode == kControlRate && !synth && Mmin >= kWideTile + kWideMargin) {
         const int wring = next_pow2(a.M + kWideTile);
         const size_t wsmem = sizeof(float) * (size_t)wring;
-        if (wsmem <= 200 * 1024) {
-            if (wsmem > 48 * 1024)
-                MODFX_CUDA_OK(cudaFuncSetAttribute(fc_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
+        if (wsmem <= kMaxSmem) {
             a.wide = 1;
-            fc_wide_kernel<<<grid, kWideThreads, wsmem, s>>>(a, wring - 1);
-            MODFX_CUDA_OK(cudaGetLastError());
+            if ((st = launch(fc_wide_kernel, grid, kWideThreads, wsmem, s, a, wring - 1)) != MODFX_OK) return st;
         }
     }
-#define LAUNCH_CTA(MODE, SYNTH)                                                                           \
-    do {                                                                                                  \
-        if (csmem > 48 * 1024)                                                                            \
-            MODFX_CUDA_OK(cudaFuncSetAttribute(fc_cta_kernel<MODE, SYNTH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)csmem)); \
-        fc_cta_kernel<MODE, SYNTH><<<grid, kCtaThreads, csmem, s>>>(a, lo_smem);                          \
-    } while (0)
-    if (mode == kAudioRate) LAUNCH_CTA(kAudioRate, kRead);
-    else if (mode == kDirectLfo) LAUNCH_CTA(kDirectLfo, kAtTap);
-    else if (!synth) LAUNCH_CTA(kControlRate, kRead);
-    else if (lo_smem > 0) LAUNCH_CTA(kControlRate, kStaged);
-    else LAUNCH_CTA(kControlRate, kAtTap);
-#undef LAUNCH_CTA
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    void (*cta)(FcArgs, int);
+    if (mode == kAudioRate) cta = fc_cta_kernel<kAudioRate, kRead>;
+    else if (mode == kDirectLfo) cta = fc_cta_kernel<kDirectLfo, kAtTap>;
+    else if (!synth) cta = fc_cta_kernel<kControlRate, kRead>;
+    else if (lo_smem > 0) cta = fc_cta_kernel<kControlRate, kStaged>;
+    else cta = fc_cta_kernel<kControlRate, kAtTap>;
+    return launch(cta, grid, kCtaThreads, csmem, s, a, lo_smem);
 }
 
 extern "C" int modfx_flanger_chorus_allpass_f32(const float* x, float* y, int32_t B, int32_t C, int64_t N,
@@ -1008,76 +1022,41 @@ extern "C" int modfx_flanger_chorus_allpass_f32(const float* x, float* y, int32_
                                                 modfx_param feedback, modfx_param min_delay_width, modfx_param width,
                                                 modfx_param depth, modfx_param mix, const int32_t* example_index,
                                                 int32_t n_items, void* stream) {
-    MODFX_REQUIRE(x && y, "x / y is NULL");
-    MODFX_REQUIRE(B >= 0 && C >= 1 && N >= 1 && N < (1ll << 30), "bad shape B=%d C=%d N=%lld", B, C, (long long)N);
-    MODFX_REQUIRE(Mmin >= 0 && Mlfo >= 0 && Mmin + Mlfo >= 1, "bad delay line Mmin=%d Mlfo=%d", Mmin, Mlfo);
-    int st;
-    if ((st = check_scalar(feedback, "feedback", false)) != MODFX_OK) return st;
-    if ((st = check_scalar(min_delay_width, "min_delay_width", true)) != MODFX_OK) return st;
-    if ((st = check_scalar(width, "width", true)) != MODFX_OK) return st;
-    if ((st = check_scalar(depth, "depth", true)) != MODFX_OK) return st;
-    if ((st = check_scalar(mix, "mix", true)) != MODFX_OK) return st;
-    FcArgs a{};
-    a.x = x; a.y = y; a.B = B; a.C = C; a.N = (int)N;
-    a.Mmin = Mmin; a.Mlfo = Mlfo; a.M = Mmin + Mlfo;
-    int mode = 0;
-    if ((st = fill_mod(a, mod, B, N, mode)) != MODFX_OK) return st;
-    if (mode == kDirectLfo || a.lfo_freq)
-        return fail(MODFX_ERR_UNSUPPORTED, "all-pass interpolation takes the modulation signal from memory (audio or control rate)");
-    if (mode == kAudioRate) a.n_lo = 0;
-    a.fb_p = feedback.dev;         a.fb_s = (float)feedback.value;
-    a.mdw_p = min_delay_width.dev; a.min_delay_s = (float)(min_delay_width.value * (double)Mmin);
-    a.width_p = width.dev;         a.lfo_delay_s = (float)((double)Mlfo * width.value);
-    a.depth_p = depth.dev;         a.depth_s = (float)depth.value;
-    a.mix_p = mix.dev;             a.mix_s = (float)mix.value; a.omm_s = (float)(1.0 - mix.value);
-    a.index = example_index;
-    a.n_items = example_index ? n_items : B;
-    if (a.n_items == 0) return MODFX_OK;
-    MODFX_REQUIRE(a.n_items > 0, "n_items=%d", a.n_items);
+    FcArgs a;
+    int mode = 0, st;
+    if ((st = fc_setup(a, mode, kAllpassDelay, x, y, B, C, N, Mmin, Mlfo, mod,
+                       {feedback, min_delay_width, width, depth, mix}, example_index, n_items)) != MODFX_OK ||
+        a.n_items == 0)
+        return st;
     const int ring = next_pow2(a.M + 1);
     a.ring_mask = ring - 1;
     int L = kWarp;
     while (L > 1 && (size_t)ring * L * sizeof(float) > 160 * 1024) L >>= 1;
     const size_t smem = sizeof(float) * ((size_t)ring * L + 2 * kWarp * (kWarp + 1));
-    if (smem > 200 * 1024) return fail(MODFX_ERR_UNSUPPORTED, "delay line of %d samples exceeds shared memory", a.M);
+    if (smem > kMaxSmem) return fail(MODFX_ERR_UNSUPPORTED, "delay line of %d samples exceeds shared memory", a.M);
     const int n_lines = a.n_items * C;
-    if (smem > 48 * 1024)
-        MODFX_CUDA_OK(cudaFuncSetAttribute(fc_allpass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fc_allpass_kernel<<<(unsigned)((n_lines + L - 1) / L), kWarp, smem, as_stream(stream)>>>(a, L, ring - 1, n_lines);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    return launch(fc_allpass_kernel, (unsigned)((n_lines + L - 1) / L), kWarp, smem, as_stream(stream), a, L, ring - 1,
+                  n_lines);
 }
 
 extern "C" int modfx_tremolo_f32(const float* x, float* y, int32_t B, int32_t C, int64_t N,
                                  const modfx_mod_source* mod, modfx_param mix, void* stream) {
-    MODFX_REQUIRE(x && y, "x / y is NULL");
-    MODFX_REQUIRE(B >= 0 && C >= 1 && N >= 1 && N < (1ll << 30), "bad shape B=%d C=%d N=%lld", B, C, (long long)N);
-    int st;
-    if ((st = check_scalar(mix, "mix", true)) != MODFX_OK) return st;                     // fx.py:21
-    FcArgs a{};
-    a.x = x; a.y = y; a.B = B; a.C = C; a.N = (int)N;
-    int mode = 0;
-    if ((st = fill_mod(a, mod, B, N, mode)) != MODFX_OK) return st;
-    a.mix_p = mix.dev; a.mix_s = (float)mix.value; a.omm_s = (float)(1.0 - mix.value);
-    if (B == 0) return MODFX_OK;
+    FcArgs a;
+    FcParams p{};
+    p.mix = mix;
+    int mode = 0, st;
+    if ((st = fc_setup(a, mode, kTremolo, x, y, B, C, N, 0, 0, mod, p, nullptr, 0)) != MODFX_OK || a.n_items == 0)
+        return st;
     const size_t smem = sizeof(float) * ((mode == kControlRate && a.lfo_freq) ? (size_t)a.n_lo : 0);
-    if (smem > 200 * 1024)
+    if (smem > kMaxSmem)
         return fail(MODFX_ERR_UNSUPPORTED, "tremolo with an in-kernel control-rate LFO of %d points exceeds shared memory", a.n_lo);
     int ny = (int)((N + 256 * 8 - 1) / (256 * 8));
     if (ny < 1) ny = 1;
     if (ny > 65535) ny = 65535;
     const dim3 grid((unsigned)(B * C), (unsigned)ny);
-    cudaStream_t s = as_stream(stream);
-#define LAUNCH_TR(MODE)                                                                                   \
-    do {                                                                                                  \
-        if (smem > 48 * 1024)                                                                             \
-            MODFX_CUDA_OK(cudaFuncSetAttribute(tremolo_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        tremolo_kernel<MODE><<<grid, 256, smem, s>>>(a);                                                  \
-    } while (0)
-    if (mode == kAudioRate) LAUNCH_TR(kAudioRate);
-    else if (mode == kControlRate) LAUNCH_TR(kControlRate);
-    else LAUNCH_TR(kDirectLfo);
-#undef LAUNCH_TR
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    void (*kernel)(FcArgs);
+    if (mode == kAudioRate) kernel = tremolo_kernel<kAudioRate>;
+    else if (mode == kControlRate) kernel = tremolo_kernel<kControlRate>;
+    else kernel = tremolo_kernel<kDirectLfo>;
+    return launch(kernel, grid, 256, smem, as_stream(stream), a);
 }

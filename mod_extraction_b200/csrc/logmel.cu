@@ -433,10 +433,7 @@ extern "C" int modfx_logmel_f32(const float* x, float* out, int64_t R, int64_t T
     const int span = (kFB - 1) * hop + kNfft;
     const size_t smem = sizeof(float) * (size_t)(4 + 2 * 512 + kWarps * kRegion + ((span + 3) & ~3) + fb_taps) +
                         sizeof(unsigned short) * (size_t)(2 * n_mels + 4) + 16;
-    MODFX_CUDA_OK(cudaFuncSetAttribute(logmel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     MODFX_CUDA_OK(cudaFuncSetAttribute(logmel_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                                        cudaSharedmemCarveoutMaxShared));
-    logmel_kernel<<<(unsigned)grid, kThreads, smem, as_stream(stream)>>>(a);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    return launch(logmel_kernel, (unsigned)grid, kThreads, smem, as_stream(stream), a);
 }

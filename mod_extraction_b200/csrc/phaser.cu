@@ -31,8 +31,21 @@ struct PhaserArgs {
     int block;
     const int32_t* index;
     int n_items;
-    int n_ctl;       // control points per example = ceil(N / 4)
-    int n_chunks;    // ceil(N / kChunk)
+    int n_ctl;                  // control points per example = ceil(N / 4)
+    int n_chunks;               // ceil(N / kChunk)
+    const int32_t* start;       // (B,) first delivered sample of each row, or nullptr (0)
+    int n_out;                  // delivered samples per row
+    float* dry_out;             // (B, n_out) window of the dry input, or nullptr
+    int x_compact;              // 1: row `item` of x (a compact (n_items, N) array), 0: row b like every other array
+    const int64_t* x_offset;    // (n_items,) or nullptr: x is a packed ragged array, row `item` starts at x + x_offset[item]
+                                // and holds start + n_out samples (the prefix that determines the delivered window)
+    int n_seg;
+    int* ticket;                // 1 int, zero at launch
+    int* flags;                 // (n_items, n_seg), zero at launch
+    float* rec;                 // (n_items, n_seg, kRec)
+    float2* ph;                 // (n_items, n_chunks): phase at the chunk's first control point, phase of the one before
+    float* phc;                 // (n_items, n_ctl): phase of every control point; used instead of ph (then nullptr) when
+                                // the host block is not a multiple of kChunk samples
 };
 
 __device__ __forceinline__ int example_of(const PhaserArgs& a, int item) { return a.index ? a.index[item] : item; }
@@ -117,23 +130,6 @@ constexpr int kFusedSmemFloats = kSubs * (kSub + 1) + kSubs * (kSubCtl + 1) + kS
 // (+ 1 KB per CTA reserved by the runtime, + the few static bytes, within the 228 KB of an SM)
 static_assert(kFusedCtasPerSM * (kFusedSmemFloats * 4 + 128 + 1024) <= 228 * 1024, "phaser_fused_kernel: 6 CTAs per SM");
 
-struct FusedArgs {
-    PhaserArgs a;
-    const int32_t* start;       // (B,) first delivered sample of each row, or nullptr (0)
-    int n_out;                  // delivered samples per row
-    float* dry_out;             // (B, n_out) window of the dry input, or nullptr
-    int x_compact;              // 1: row `item` of x (a compact (n_items, N) array), 0: row b like every other array
-    const int64_t* x_offset;    // (n_items,) or nullptr: x is a packed ragged array, row `item` starts at x + x_offset[item]
-                                // and holds start + n_out samples (the prefix that determines the delivered window)
-    int n_seg;
-    int* ticket;                // 1 int, zero at launch
-    int* flags;                 // (n_items, n_seg), zero at launch
-    float* rec;                 // (n_items, n_seg, kRec)
-    float2* ph;                 // (n_items, n_chunks): phase at the chunk's first control point, phase of the one before
-    float* phc;                 // (n_items, n_ctl): phase of every control point; used instead of ph (then nullptr) when
-                                // the host block is not a multiple of kChunk samples
-};
-
 // Oscillator phases: one thread per (example, host block), juce::dsp::Oscillator semantics.  Control points sit at
 // global multiples of 4 samples; inside a host block the phase advances by `inc` per control point with a wrap at 2 pi
 // (sequential float32 adds, reproduced exactly); a block starts from the previous block's start phase advanced by
@@ -149,13 +145,12 @@ __device__ __forceinline__ float phase_advance(float p, float inc, float two_pi)
     return (next >= two_pi) ? wrapped : next;
 }
 
-__global__ void __launch_bounds__(128) phaser_phase_kernel(const FusedArgs f, int n_blocks) {
-    const PhaserArgs& a = f.a;
+__global__ void __launch_bounds__(128) phaser_phase_kernel(const PhaserArgs a, int n_blocks) {
     const int pair = blockIdx.x * blockDim.x + threadIdx.x;
     if (pair >= a.n_items * n_blocks) return;
     const int item = pair / n_blocks, blk = pair - item * n_blocks;
     const int b = example_of(a, item);
-    const int need = f.start ? min(a.N, f.start[b] + f.n_out) : a.N;
+    const int need = a.start ? min(a.N, a.start[b] + a.n_out) : a.N;
     // (a block past the window still has to hand its last phase to nobody: nothing after `need` is rendered)
     if ((int64_t)blk * a.block >= need) return;
     const float two_pi = MODFX_TWO_PI_F;
@@ -170,8 +165,8 @@ __global__ void __launch_bounds__(128) phaser_phase_kernel(const FusedArgs f, in
         p = next;
     }
     const int s0 = blk * a.block, s1 = min(s0 + a.block, a.N);
-    if (f.phc) {                                     // the phase of every control point of the block
-        float* out = f.phc + (int64_t)item * a.n_ctl;
+    if (a.phc) {                                     // the phase of every control point of the block
+        float* out = a.phc + (int64_t)item * a.n_ctl;
         for (int j = (s0 + kUpd - 1) / kUpd; j < (s1 + kUpd - 1) / kUpd; ++j) {
             out[j] = p;
             float next = p + inc;
@@ -181,7 +176,7 @@ __global__ void __launch_bounds__(128) phaser_phase_kernel(const FusedArgs f, in
         return;
     }
     const int c0 = s0 / kChunk, c1 = (s1 + kChunk - 1) / kChunk;
-    float2* out = f.ph + (int64_t)item * a.n_chunks;
+    float2* out = a.ph + (int64_t)item * a.n_chunks;
     // a clip's very first control point has no predecessor and the value is unused (all filter states are zero there)
     float prev = 0.0f;
     const bool small = inc < two_pi;
@@ -232,7 +227,7 @@ __device__ __forceinline__ void store_window(float* row, const float (*xs)[kSub 
     if (tid < hi - v1) row[v1 + tid - start] = at(v1 + tid);
 }
 
-__global__ void __launch_bounds__(kFusedThreads, kFusedCtasPerSM) phaser_fused_kernel(const FusedArgs f) {
+__global__ void __launch_bounds__(kFusedThreads, kFusedCtasPerSM) phaser_fused_kernel(const PhaserArgs a) {
     extern __shared__ __align__(16) float sm[];
     float(*xs)[kSub + 1] = reinterpret_cast<float(*)[kSub + 1]>(sm);                        // [64][65] audio, then output
     float(*cs)[kSubCtl + 1] = reinterpret_cast<float(*)[kSubCtl + 1]>(sm + kSubs * (kSub + 1));   // [64][17] col 0: coefficient before
@@ -242,19 +237,18 @@ __global__ void __launch_bounds__(kFusedThreads, kFusedCtasPerSM) phaser_fused_k
     __shared__ int tile_s;
     __shared__ float entry[kRec];
     __shared__ float coef_k[5];                                          // log_min, log_span, w0, vol, ctr of phaser_coef
-    const PhaserArgs& a = f.a;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if (tid == 0) tile_s = atomicAdd(f.ticket, 1);
+    if (tid == 0) tile_s = atomicAdd(a.ticket, 1);
     __syncthreads();
     const int tile = tile_s;
     const int seg = tile / a.n_items, item = tile - seg * a.n_items;     // segment-major: predecessors hold earlier tickets
     const int b = example_of(a, item);
-    const int start = f.start ? f.start[b] : 0;
-    const int need = min(a.N, start + f.n_out);
+    const int start = a.start ? a.start[b] : 0;
+    const int need = min(a.N, start + a.n_out);
     const int n_base = seg * kSeg;
     if (n_base >= need) return;
-    const float* xr = f.x_offset ? a.x + f.x_offset[item] : a.x + (int64_t)(f.x_compact ? item : b) * a.N;
-    const int row_len = f.x_offset ? need : a.N;                          // samples that exist in this row
+    const float* xr = a.x_offset ? a.x + a.x_offset[item] : a.x + (int64_t)(a.x_compact ? item : b) * a.N;
+    const int row_len = a.x_offset ? need : a.N;                          // samples that exist in this row
 
     // ---- A: audio + oscillator phases
     const bool vec = ((reinterpret_cast<uintptr_t>(xr) & 15) == 0) && (n_base + kSeg <= row_len);
@@ -283,8 +277,8 @@ __global__ void __launch_bounds__(kFusedThreads, kFusedCtasPerSM) phaser_fused_k
         coef_k[4] = (log10f(a.centre[b]) - log_min) / log_span;
     }
     const float two_pi = MODFX_TWO_PI_F;
-    if (f.phc) {                                                          // precomputed: copy them
-        const float* pr = f.phc + (int64_t)item * a.n_ctl;
+    if (a.phc) {                                                          // precomputed: copy them
+        const float* pr = a.phc + (int64_t)item * a.n_ctl;
         for (int i = tid; i <= kSegCtl; i += kFusedThreads) {
             const int j = seg * kSegCtl - 1 + i;                          // i = 0: the control point before the segment
             phs[i] = (j >= 0 && j < a.n_ctl) ? pr[j] : 0.0f;
@@ -293,7 +287,7 @@ __global__ void __launch_bounds__(kFusedThreads, kFusedCtasPerSM) phaser_fused_k
         const int chunk = seg * kSegChunks + tid;
         const float sr_down = (float)((double)a.sr / (double)kUpd);
         const float inc = a.rate[b] * (two_pi / sr_down);
-        float2 pp = (chunk < a.n_chunks) ? f.ph[(int64_t)item * a.n_chunks + chunk] : make_float2(0.0f, 0.0f);
+        float2 pp = (chunk < a.n_chunks) ? a.ph[(int64_t)item * a.n_chunks + chunk] : make_float2(0.0f, 0.0f);
         if (tid == 0) phs[0] = pp.y;                                      // control point before the segment
         float p = pp.x;
         if (inc < two_pi) {
@@ -413,9 +407,9 @@ __global__ void __launch_bounds__(kFusedThreads, kFusedCtasPerSM) phaser_fused_k
     }
     __syncthreads();
     if (warp == 0) {
-        float* rec = f.rec + ((int64_t)item * f.n_seg + seg) * kRec;
+        float* rec = a.rec + ((int64_t)item * a.n_seg + seg) * kRec;
         if (seg > 0) {
-            const int* flag = f.flags + (int64_t)item * f.n_seg + seg - 1;
+            const int* flag = a.flags + (int64_t)item * a.n_seg + seg - 1;
             if (lane == 0) {
                 while (atomicAdd(const_cast<int*>(flag), 0) == 0) __nanosleep(64);
                 __threadfence();
@@ -444,14 +438,14 @@ __global__ void __launch_bounds__(kFusedThreads, kFusedCtasPerSM) phaser_fused_k
             __threadfence();
         }
         __syncwarp();
-        if (lane == 0) atomicExch(f.flags + (int64_t)item * f.n_seg + seg, 1);
+        if (lane == 0) atomicExch(a.flags + (int64_t)item * a.n_seg + seg, 1);
     }
     // a segment wholly before the window owed its successor the exit state, nothing else (CTA-uniform)
     if (n_base + kSeg <= start) return;
     // delivered samples of this segment: [lo, hi)
     const int lo = max(n_base, start), hi = min(n_base + kSeg, need);
     // the window of the dry input goes out while warp 0 chains (xs still holds the audio)
-    if (f.dry_out) store_window(f.dry_out + (int64_t)b * f.n_out, xs, n_base, start, lo, hi, tid);
+    if (a.dry_out) store_window(a.dry_out + (int64_t)b * a.n_out, xs, n_base, start, lo, hi, tid);
     __syncthreads();
     // (3) entry state of every sub-chunk: each warp chains its group (8 lanes, lane i < 7 owns state component i)
     if (lane < 8) {
@@ -494,8 +488,8 @@ __global__ void __launch_bounds__(kFusedThreads, kFusedCtasPerSM) phaser_fused_k
     }
     __syncthreads();
     // ---- F: coalesced store of the delivered window
-    float* yr = a.y + (int64_t)b * f.n_out;
-    if (start == 0 && n_base + kSeg <= f.n_out && ((reinterpret_cast<uintptr_t>(yr) & 15) == 0)) {
+    float* yr = a.y + (int64_t)b * a.n_out;
+    if (start == 0 && n_base + kSeg <= a.n_out && ((reinterpret_cast<uintptr_t>(yr) & 15) == 0)) {
 #pragma unroll
         for (int k = 0; k < kSeg / 4 / kFusedThreads; ++k) {
             const int i4 = tid + k * kFusedThreads;
@@ -525,47 +519,39 @@ extern "C" int64_t modfx_phaser_workspace_bytes(int32_t B, int64_t N) {
 
 namespace {
 
-int phaser_launch(const float* x, int x_compact, const int64_t* x_offset, float* y, float* dry_out, int32_t B, int64_t N, int64_t n_out, const int32_t* start,
-                  float sr, const float* rate_hz, const float* depth, const float* centre_hz, const float* feedback,
-                  const float* mix, int32_t block, const int32_t* example_index, int32_t n_items, void* workspace,
-                  void* stream) {
-    MODFX_REQUIRE(x && y && rate_hz && depth && centre_hz && feedback && mix, "NULL pointer");
+// The entry points fill in the pointers, sr, block, index, n_items and what a cropped call adds; the rest is set here.
+int phaser_launch(PhaserArgs a, int32_t B, int64_t N, int64_t n_out, void* workspace, void* stream) {
+    MODFX_REQUIRE(a.x && a.y && a.rate && a.depth && a.centre && a.feedback && a.mix, "NULL pointer");
     MODFX_REQUIRE(B >= 0 && N >= 1 && N < (1ll << 30), "bad shape B=%d N=%lld", B, (long long)N);
     MODFX_REQUIRE(n_out >= 1 && n_out <= N, "bad output window n_out=%lld (row length %lld)", (long long)n_out, (long long)N);
-    MODFX_REQUIRE(sr > 0.0f, "sample rate must be positive");
-    if (block <= 0) block = 8192;           // pedalboard's default buffer_size
-    PhaserArgs a{};
-    a.x = x; a.y = y; a.N = (int)N; a.sr = sr;
-    a.rate = rate_hz; a.depth = depth; a.centre = centre_hz; a.feedback = feedback; a.mix = mix;
-    a.block = block;
-    a.index = example_index;
-    a.n_items = example_index ? n_items : B;
+    MODFX_REQUIRE(a.sr > 0.0f, "sample rate must be positive");
+    if (a.block <= 0) a.block = 8192;       // pedalboard's default buffer_size
+    a.N = (int)N;
+    a.n_out = (int)n_out;
+    if (!a.index) a.n_items = B;
     if (a.n_items == 0) return MODFX_OK;
     MODFX_REQUIRE(a.n_items > 0 && workspace, "workspace is NULL or n_items=%d", a.n_items);
     a.n_ctl = (int)((N + kUpd - 1) / kUpd);
     a.n_chunks = (int)((N + kChunk - 1) / kChunk);
     cudaStream_t s = as_stream(stream);
     char* w = static_cast<char*>(workspace);
-    const int n_blocks = (int)((N + block - 1) / block);
+    const int n_blocks = (int)((N + a.block - 1) / a.block);
 
-    FusedArgs f{};
-    f.a = a;
-    f.start = start; f.n_out = (int)n_out; f.dry_out = dry_out; f.x_compact = x_compact; f.x_offset = x_offset;
-    f.n_seg = (int)((N + kSeg - 1) / kSeg);
-    f.ticket = reinterpret_cast<int*>(w);                                     w += 256;
-    f.flags = reinterpret_cast<int*>(w);
-    const int64_t flag_bytes = align_up((int64_t)a.n_items * f.n_seg * 4, 256);  w += flag_bytes;
-    f.rec = reinterpret_cast<float*>(w);                                      w += align_up((int64_t)a.n_items * f.n_seg * kRec * 4, 256);
-    if (block % kChunk == 0) f.ph = reinterpret_cast<float2*>(w);
-    else f.phc = reinterpret_cast<float*>(w);
+    a.n_seg = (int)((N + kSeg - 1) / kSeg);
+    a.ticket = reinterpret_cast<int*>(w);                                     w += 256;
+    a.flags = reinterpret_cast<int*>(w);
+    const int64_t flag_bytes = align_up((int64_t)a.n_items * a.n_seg * 4, 256);  w += flag_bytes;
+    a.rec = reinterpret_cast<float*>(w);                                      w += align_up((int64_t)a.n_items * a.n_seg * kRec * 4, 256);
+    if (a.block % kChunk == 0) a.ph = reinterpret_cast<float2*>(w);
+    else a.phc = reinterpret_cast<float*>(w);
     MODFX_CUDA_OK(cudaMemsetAsync(workspace, 0, (size_t)(256 + flag_bytes), s));
     const int pairs = a.n_items * n_blocks;
-    phaser_phase_kernel<<<(pairs + 127) / 128, 128, 0, s>>>(f, n_blocks);
-    const int64_t tiles = (int64_t)a.n_items * f.n_seg;
+    phaser_phase_kernel<<<(pairs + 127) / 128, 128, 0, s>>>(a, n_blocks);
+    const int64_t tiles = (int64_t)a.n_items * a.n_seg;
     MODFX_REQUIRE(tiles < (1ll << 31), "too many segments in one call");
     MODFX_CUDA_OK(cudaFuncSetAttribute(phaser_fused_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                                        cudaSharedmemCarveoutMaxShared));
-    phaser_fused_kernel<<<(unsigned)tiles, kFusedThreads, sizeof(float) * kFusedSmemFloats, s>>>(f);
+    phaser_fused_kernel<<<(unsigned)tiles, kFusedThreads, sizeof(float) * kFusedSmemFloats, s>>>(a);
     MODFX_CUDA_OK(cudaGetLastError());
     return MODFX_OK;
 }
@@ -576,8 +562,11 @@ extern "C" int modfx_phaser_f32(const float* x, float* y, int32_t B, int64_t N, 
                                 const float* depth, const float* centre_hz, const float* feedback,
                                 const float* mix, int32_t block, const int32_t* example_index, int32_t n_items,
                                 void* workspace, void* stream) {
-    return phaser_launch(x, 0, nullptr, y, nullptr, B, N, N, nullptr, sr, rate_hz, depth, centre_hz, feedback, mix, block, example_index,
-                         n_items, workspace, stream);
+    PhaserArgs a{};
+    a.x = x; a.y = y; a.sr = sr;
+    a.rate = rate_hz; a.depth = depth; a.centre = centre_hz; a.feedback = feedback; a.mix = mix;
+    a.block = block; a.index = example_index; a.n_items = n_items;
+    return phaser_launch(a, B, N, N, workspace, stream);
 }
 
 extern "C" int modfx_phaser_crop_f32(const float* x, int32_t x_compact, float* y, float* dry_out, int32_t B, int64_t N,
@@ -586,8 +575,12 @@ extern "C" int modfx_phaser_crop_f32(const float* x, int32_t x_compact, float* y
                                      const int32_t* example_index, int32_t n_items, void* workspace, void* stream) {
     MODFX_REQUIRE(start, "start is NULL");
     MODFX_REQUIRE(!x_compact || example_index, "x_compact needs an example_index list");
-    return phaser_launch(x, x_compact ? 1 : 0, nullptr, y, dry_out, B, N, n_out, start, sr, rate_hz, depth, centre_hz, feedback, mix, block, example_index,
-                         n_items, workspace, stream);
+    PhaserArgs a{};
+    a.x = x; a.y = y; a.sr = sr;
+    a.rate = rate_hz; a.depth = depth; a.centre = centre_hz; a.feedback = feedback; a.mix = mix;
+    a.block = block; a.index = example_index; a.n_items = n_items;
+    a.start = start; a.dry_out = dry_out; a.x_compact = x_compact ? 1 : 0;
+    return phaser_launch(a, B, N, n_out, workspace, stream);
 }
 
 extern "C" int modfx_phaser_crop_packed_f32(const float* x, const int64_t* x_offset, float* y, float* dry_out, int32_t B,
@@ -597,6 +590,10 @@ extern "C" int modfx_phaser_crop_packed_f32(const float* x, const int64_t* x_off
                                             void* stream) {
     MODFX_REQUIRE(start && x_offset, "start or x_offset is NULL");
     MODFX_REQUIRE(example_index, "a packed x needs an example_index list (row i belongs to example example_index[i])");
-    return phaser_launch(x, 1, x_offset, y, dry_out, B, N_max, n_out, start, sr, rate_hz, depth, centre_hz, feedback, mix, block,
-                         example_index, n_items, workspace, stream);
+    PhaserArgs a{};
+    a.x = x; a.y = y; a.sr = sr;
+    a.rate = rate_hz; a.depth = depth; a.centre = centre_hz; a.feedback = feedback; a.mix = mix;
+    a.block = block; a.index = example_index; a.n_items = n_items;
+    a.start = start; a.dry_out = dry_out; a.x_compact = 1; a.x_offset = x_offset;
+    return phaser_launch(a, B, N_max, n_out, workspace, stream);
 }

@@ -109,6 +109,53 @@ def test_cnn_entry_points_validate_before_touching_the_gpu():
     assert L.modfx_specaugment_fill_f32(p, 1, 4, 4, 0, 0, 0, 0, 1e-7, 1, nul) == 0                             # nothing to mask
 
 
+def test_effect_entry_points_validate_before_touching_the_gpu():
+    """Argument checks of the flanger / chorus, tremolo and phaser entry points run on the host: status codes without a
+    device, and a call with nothing to render returns MODFX_OK before any shared-memory refusal."""
+    import ctypes
+    L = _lib.lib()
+    buf = (ctypes.c_float * 64)()
+    p = ctypes.cast(buf, ctypes.c_void_p)
+    nul = ctypes.c_void_p(0)
+    P = _lib.ModfxParam
+    Mod = _lib.ModfxModSource
+    audio = Mod(kind=_lib.MOD_AUDIO_RATE, mod=p)
+    lfo = Mod(kind=_lib.MOD_LFO, n_lo=64, sr_lo=100.0, lfo_freq=p, lfo_phase=p, lfo_shape=p)
+
+    def fc(x=p, B=1, N=64, M=(10, 10), mod=audio, feedback=0.5, index=nul, n_items=0, allpass=False):
+        f = L.modfx_flanger_chorus_allpass_f32 if allpass else L.modfx_flanger_chorus_f32
+        half = P(None, 0.5)
+        return f(x, p, B, 1, N, M[0], M[1], ctypes.byref(mod), P(None, feedback), half, half, half, half, index,
+                 n_items, nul)
+
+    long_line = (20000, 20441)                                                  # 40 441 samples
+    assert fc(x=nul) == -1
+    assert fc(feedback=1.0) == -1                                               # fx.py:69 (feedback < 1 strictly)
+    assert fc(B=0, M=long_line) == 0
+    assert fc(index=p, n_items=0, M=long_line) == 0                             # empty example_index
+    assert fc(M=long_line) == -2 and b"shared memory" in L.modfx_last_error()
+    assert fc(M=long_line, allpass=True) == -2 and b"shared memory" in L.modfx_last_error()
+    assert fc(mod=lfo, allpass=True) == -2                                      # all-pass reads mod from memory
+    assert fc(mod=Mod(kind=_lib.MOD_CONTROL_RATE, mod=p, n_lo=65)) == -1       # n_lo > N
+    assert fc(mod=Mod(kind=7, mod=p)) == -1                                     # unknown modulation kind
+
+    def tremolo(B, mod=audio, N=64):
+        return L.modfx_tremolo_f32(p, p, B, 1, N, ctypes.byref(mod), P(None, 0.5), nul)
+
+    big_lfo = Mod(kind=_lib.MOD_LFO, n_lo=60000, sr_lo=100.0, lfo_freq=p, lfo_phase=p, lfo_shape=p)
+    assert tremolo(0) == 0
+    assert tremolo(0, big_lfo, N=100000) == 0
+    assert tremolo(1, big_lfo, N=100000) == -2 and b"shared memory" in L.modfx_last_error()
+
+    sr = ctypes.c_float(44100.0)
+    assert L.modfx_phaser_f32(nul, p, 1, 64, sr, p, p, p, p, p, 0, nul, 0, p, nul) == -1
+    assert L.modfx_phaser_f32(p, p, 1, 64, sr, p, p, p, p, p, 0, p, 0, nul, nul) == 0       # empty example_index
+    assert L.modfx_phaser_crop_f32(p, 0, p, nul, 1, 64, 64, nul, sr, p, p, p, p, p, 0, nul, 0, p, nul) == -1   # NULL start
+    assert L.modfx_phaser_crop_f32(p, 0, p, nul, 1, 64, 65, p, sr, p, p, p, p, p, 0, nul, 0, p, nul) == -1     # n_out > N
+    assert L.modfx_phaser_crop_f32(p, 1, p, nul, 1, 64, 64, p, sr, p, p, p, p, p, 0, nul, 0, p, nul) == -1     # x_compact
+    assert L.modfx_phaser_crop_packed_f32(p, p, p, nul, 1, 64, 64, p, sr, p, p, p, p, p, 0, nul, 0, p, nul) == -1
+
+
 def test_build_is_keyed_by_source_content():
     """_build.build() must not reuse a library built from other sources: the hash of csrc/ + include/ + flags is stored
     beside the library and compared, whatever the file times say."""
