@@ -314,22 +314,24 @@ extern "C" int modfx_cnn_layernorm_f32(const float* x, float* y, int32_t B, int3
     MODFX_REQUIRE(B <= 65535, "B=%d: at most 65535 examples per call", B);
     const int64_t P = (int64_t)H * W;
     double* part = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(workspace) + 15) & ~(uintptr_t)15);
-    cudaStream_t st = as_stream(stream);
+    cudaStream_t s = as_stream(stream);
     const size_t smem = 2 * (size_t)C * sizeof(float);
+    int st;
     if (x_is_nchw) {
         MODFX_REQUIRE((int64_t)B * C <= 65535, "B*C too large for one call");
         const int chunks = ln_chunks(P);
-        ln_stats_kernel<<<dim3(chunks, B * C), kLnThreads, 0, st>>>(x, part, P, 1, chunks);
-        ln_apply_kernel<true><<<dim3(ln_chunks(P * C), B), kLnThreads, smem, st>>>(x, y, part, P, C, chunks, eps,
-                                                                                   round_tf32, 0);
+        st = launch(ln_stats_kernel, dim3(chunks, B * C), kLnThreads, 0, s, x, part, P, 1, chunks);
+        if (st == MODFX_OK)
+            st = launch(ln_apply_kernel<true>, dim3(ln_chunks(P * C), B), kLnThreads, smem, s, x, y, part, P, C, chunks,
+                        eps, round_tf32, 0);
     } else {
         const int chunks = ln_chunks(P * C);
-        ln_stats_kernel<<<dim3(chunks, B), kLnThreads, 0, st>>>(x, part, P * C, C, chunks);
-        ln_apply_kernel<false><<<dim3(chunks, B), kLnThreads, smem, st>>>(x, y, part, P, C, chunks, eps, round_tf32,
-                                                                          (int64_t)B * P * C);
+        st = launch(ln_stats_kernel, dim3(chunks, B), kLnThreads, 0, s, x, part, P * C, C, chunks);
+        if (st == MODFX_OK)
+            st = launch(ln_apply_kernel<false>, dim3(chunks, B), kLnThreads, smem, s, x, y, part, P, C, chunks, eps,
+                        round_tf32, (int64_t)B * P * C);
     }
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    return st;
 }
 
 template <int kCin, int kCk>

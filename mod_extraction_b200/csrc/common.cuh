@@ -28,15 +28,25 @@ int fail(modfx_status st, const char* fmt, ...);
 inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
 // kernel<<<grid, block, smem, stream>>>(args...), opting in first when smem exceeds the default 48 KB.  That default
-// covers static and dynamic shared memory together, but only the dynamic size is tested here: the kernels launched
-// through this use no static shared memory except fc_wide_kernel's 32 B, and its dynamic size is a power of two, never
-// within 32 B of 48 KB.  A kernel that gains static shared memory must count it.
+// covers static and dynamic shared memory together, but only the dynamic size is tested here: of the kernels launched
+// with dynamic shared memory, only fc_wide_kernel (32 B, dynamic size a power of two, never within 32 B of 48 KB) and
+// phaser_fused_kernel (under 100 B, dynamic size under 40 KB) also have static shared memory.  A kernel that gains
+// static shared memory must count it.
 template <typename... Params, typename... Args>
 int launch(void (*kernel)(Params...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
     if (smem > 48 * 1024)
         MODFX_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kernel<<<grid, block, smem, stream>>>(args...);
     MODFX_CUDA_OK(cudaGetLastError());
+    return MODFX_OK;
+}
+
+// Grid of a kernel that strides over the elements of row blockIdx.y in blocks of 256 threads: one block per 256
+// elements of a row, at most `cap`.  More rows than grid.y holds are refused.
+inline int row_grid(dim3& grid, int64_t per_row, int64_t rows, int cap) {
+    MODFX_REQUIRE(rows <= 65535, "%lld rows exceed grid.y", (long long)rows);
+    const int64_t gx = (per_row + 255) / 256;
+    grid = dim3((unsigned)(gx < cap ? gx : cap), (unsigned)rows);
     return MODFX_OK;
 }
 
@@ -116,17 +126,39 @@ __device__ __forceinline__ float lfo_value(const LfoDesc& d, int64_t i) {
     return v;
 }
 
-// F.interpolate(mode="linear", align_corners=True) element i of an O-point output from an
-// I-point row `lo` (ATen upsample_linear1d; the torch CPU build contracts the blend to
-// fma(w0, x0, w1*x1) -- pinned bitwise by tests/golden/interp.npz).  scale = f32(I-1)/f32(O-1).
+// The two taps and weights of F.interpolate(mode="linear") at source position src of an I-point row (ATen
+// upsample_linear1d, util.py:15-29).  Int is the index type of the row.
+template <typename Int>
+struct LinearTaps {
+    Int i0, i1;
+    float l0, l1;
+};
+
+template <typename Int>
+__device__ __forceinline__ LinearTaps<Int> linear_taps(float src, Int I) {
+    LinearTaps<Int> t;
+    t.i0 = min((Int)src, I - 1);
+    t.i1 = t.i0 + ((t.i0 < I - 1) ? 1 : 0);
+    t.l1 = __fsub_rn(src, (float)t.i0);
+    t.l0 = __fsub_rn(1.0f, t.l1);
+    return t;
+}
+
+// align_corners=True: output element i reads source position scale * i, scale = f32(I-1)/f32(O-1).
+__device__ __forceinline__ LinearTaps<int> taps_ac(float scale, int i, int I) {
+    return linear_taps(__fmul_rn(scale, (float)i), I);
+}
+
+// The torch CPU build contracts the blend to fma(l0, x0, l1*x1) -- pinned bitwise by tests/golden/interp.npz.
+template <typename Int>
+__device__ __forceinline__ float blend(const LinearTaps<Int>& t, float v0, float v1) {
+    return __fmaf_rn(t.l0, v0, __fmul_rn(t.l1, v1));
+}
+
+// F.interpolate(mode="linear", align_corners=True) element i of an O-point output from an I-point row `lo`.
 __device__ __forceinline__ float upsample_ac(const float* __restrict__ lo, int I, float scale, int i) {
-    const float src = __fmul_rn(scale, (float)i);
-    int i0 = (int)src;
-    i0 = min(i0, I - 1);
-    const int i1 = i0 + ((i0 < I - 1) ? 1 : 0);
-    const float l1 = __fsub_rn(src, (float)i0);
-    const float l0 = __fsub_rn(1.0f, l1);
-    return __fmaf_rn(l0, lo[i0], __fmul_rn(l1, lo[i1]));
+    const LinearTaps<int> t = taps_ac(scale, i, I);
+    return blend(t, lo[t.i0], lo[t.i1]);
 }
 
 __device__ __forceinline__ float upsample_scale_ac_dev(int I, int O) {
@@ -135,6 +167,22 @@ __device__ __forceinline__ float upsample_scale_ac_dev(int I, int O) {
 
 inline float upsample_scale_ac(int64_t I, int64_t O) {
     return (O > 1) ? (float)(I - 1) / (float)(O - 1) : 0.0f;
+}
+
+// find_corners (modulations.py:219-238) at sample i of the n-point row m: bit 0 = top corner, bit 1 = bottom corner,
+// 0 outside 1..n-2.  A corner is a sign change of the first difference; the flags are
+// -floor(diff_l(+/-) * (diff_r + 1e-16)) compared against 1.
+template <typename Int>
+__device__ __forceinline__ unsigned corner_flags(const float* m, Int i, Int n) {
+    if (i < 1 || i > n - 2) return 0u;
+    const float dl = __fsub_rn(m[i], m[i - 1]);
+    const float dr = __fadd_rn(__fsub_rn(m[i + 1], m[i]), 1e-16f);
+    const float pos = (dl > 0.0f) ? dl : 0.0f;          // (diff_l > 0) * diff_l
+    const float neg = (dl < 0.0f) ? dl : 0.0f;
+    unsigned f = 0;
+    if (-floorf(__fmul_rn(pos, dr)) == 1.0f) f |= 1u;
+    if (-floorf(__fmul_rn(neg, dr)) == 1.0f) f |= 2u;
+    return f;
 }
 
 int num_sms();

@@ -189,7 +189,8 @@ __global__ void __launch_bounds__(kWideThreads) fc_wide_kernel(const FcArgs a, i
         for (int k = 0; k < kWideSub; ++k) {
             const int n = n0 + k * kWideThreads + tid;
             // x100 upsample (util.py:15-29) and index arithmetic (fx.py:95-102), branch-free: 0 <= mod <= 1 and the
-            // parameter bounds keep (w - d) + M inside [0, 2M)
+            // parameter bounds keep (w - d) + M inside [0, 2M).  The taps are linear_taps() of common.cuh written out:
+            // through the helper this kernel and fc_cta_kernel compile to other schedules and register counts.
             const float src = __fmul_rn(a.up_scale, (float)min(n, N - 1));
             const int i0 = min((int)src, last_lo);
             const float l1 = __fsub_rn(src, (float)i0);
@@ -477,6 +478,7 @@ __global__ void __launch_bounds__(kCtaThreads) fc_cta_kernel(const FcArgs a, int
                     } else if (MODE == kDirectLfo) {
                         m = lfo_value(lfo, min(n, N - 1));
                     } else {
+                        // linear_taps() written out, see fc_wide_kernel
                         const float src = __fmul_rn(a.up_scale, (float)min(n, N - 1));          // util.py:15-29
                         const int i0 = min((int)src, last_lo);
                         const int i1 = min(i0 + 1, last_lo);

@@ -5,10 +5,18 @@
 // (make_rand_mod_signal, the phaser ground-truth LFO of datasets.py:442-450, targets at 345 frames).
 #include "common.cuh"
 
-#include <algorithm>
-
 namespace modfx {
 namespace {
+
+// modulations.py:26-29: make_mod_signal halves frequency and phase for the rectified shapes (exact in float32)
+__device__ __forceinline__ bool is_rect(int shape) {
+    return shape == MODFX_SHAPE_RECT_COS || shape == MODFX_SHAPE_INV_RECT_COS;
+}
+
+// make_mod_signal(len, len, 1.0, 0.0, shape) of one section of make_combined_mod_sig, modulations.py:208
+__device__ __forceinline__ LfoDesc section_lfo(int shape, float len) {
+    return make_lfo_desc(is_rect(shape) ? 0.5f : 1.0f, 0.0f, shape, 1.0f, len);
+}
 
 __global__ void __launch_bounds__(256) lfo_kernel(float* __restrict__ out, int64_t n, float sr,
                                                   const float* __restrict__ freq, const float* __restrict__ phase,
@@ -20,8 +28,8 @@ __global__ void __launch_bounds__(256) lfo_kernel(float* __restrict__ out, int64
         o[i] = lfo_value(d, i);
 }
 
-// ATen upsample_linear1d: see upsample_ac in common.cuh for the align_corners=True arithmetic;
-// align_corners=False uses src = max(fma(scale, i + 0.5, -0.5), 0) with scale = I / O.
+// ATen upsample_linear1d: align_corners=True reads source position scale * i with scale = (I - 1) / (O - 1),
+// align_corners=False src = max(fma(scale, i + 0.5, -0.5), 0) with scale = I / O.
 __global__ void __launch_bounds__(256) interp_kernel(const float* __restrict__ in, float* __restrict__ out,
                                                      int64_t I, int64_t O, float scale, int align_corners) {
     const float* xi = in + (int64_t)blockIdx.y * I;
@@ -30,12 +38,8 @@ __global__ void __launch_bounds__(256) interp_kernel(const float* __restrict__ i
         float src;
         if (align_corners) src = __fmul_rn(scale, (float)i);
         else src = fmaxf(__fmaf_rn(scale, __fadd_rn((float)i, 0.5f), -0.5f), 0.0f);
-        int64_t i0 = (int64_t)src;
-        if (i0 > I - 1) i0 = I - 1;
-        const int64_t i1 = i0 + ((i0 < I - 1) ? 1 : 0);
-        const float l1 = __fsub_rn(src, (float)i0);
-        const float l0 = __fsub_rn(1.0f, l1);
-        yo[i] = __fmaf_rn(l0, xi[i0], __fmul_rn(l1, xi[i1]));
+        const LinearTaps<int64_t> t = linear_taps(src, I);
+        yo[i] = blend(t, xi[t.i0], xi[t.i1]);
     }
 }
 
@@ -49,12 +53,9 @@ extern "C" int modfx_lfo_f32(float* out, int32_t B, int64_t n, float sr, const f
     MODFX_REQUIRE(out && freq && phase && shape, "NULL pointer");
     MODFX_REQUIRE(B >= 0 && n >= 1 && sr > 0.0f, "bad arguments B=%d n=%lld sr=%g", B, (long long)n, sr);
     if (B == 0) return MODFX_OK;
-    MODFX_REQUIRE(B <= 65535, "B=%d exceeds grid.y", B);
-    int gx = (int)((n + 255) / 256);
-    if (gx > 1024) gx = 1024;
-    lfo_kernel<<<dim3(gx, B), 256, 0, as_stream(stream)>>>(out, n, sr, freq, phase, shape, exp_or_null);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    dim3 grid;
+    if (const int st = row_grid(grid, n, B, 1024)) return st;
+    return launch(lfo_kernel, grid, 256, 0, as_stream(stream), out, n, sr, freq, phase, shape, exp_or_null);
 }
 
 extern "C" int modfx_interp_linear_f32(const float* in, float* out, int64_t rows, int64_t I, int64_t O,
@@ -62,15 +63,12 @@ extern "C" int modfx_interp_linear_f32(const float* in, float* out, int64_t rows
     MODFX_REQUIRE(in && out, "NULL pointer");
     MODFX_REQUIRE(rows >= 0 && I >= 1 && O >= 1, "bad shape rows=%lld I=%lld O=%lld", (long long)rows, (long long)I, (long long)O);
     if (rows == 0) return MODFX_OK;
-    MODFX_REQUIRE(rows <= 65535, "rows=%lld exceeds grid.y", (long long)rows);
+    dim3 grid;
+    if (const int st = row_grid(grid, O, rows, 2048)) return st;
     float scale;
     if (align_corners) scale = upsample_scale_ac(I, O);
     else scale = (float)I / (float)O;
-    int gx = (int)((O + 255) / 256);
-    if (gx > 2048) gx = 2048;
-    interp_kernel<<<dim3(gx, (unsigned)rows), 256, 0, as_stream(stream)>>>(in, out, I, O, scale, align_corners);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    return launch(interp_kernel, grid, 256, 0, as_stream(stream), in, out, I, O, scale, align_corners);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -80,25 +78,16 @@ extern "C" int modfx_interp_linear_f32(const float* in, float* out, int64_t rows
 namespace modfx {
 namespace {
 
-// find_corners, reference modulations.py:219-238: a corner at i (1 <= i <= n-2) is a sign change of
-// the first difference; flags are -floor(diff_l(+/-) * (diff_r + 1e-16)) compared against 1.
+// find_corners, reference modulations.py:219-238, as two flag rows
 __global__ void __launch_bounds__(256) corners_kernel(const float* __restrict__ mod, uint8_t* __restrict__ top,
                                                       uint8_t* __restrict__ bottom, int64_t n) {
     const float* m = mod + (int64_t)blockIdx.y * n;
     uint8_t* t = top + (int64_t)blockIdx.y * n;
     uint8_t* bt = bottom + (int64_t)blockIdx.y * n;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        uint8_t ft = 0, fb = 0;
-        if (i >= 1 && i <= n - 2) {
-            const float dl = __fsub_rn(m[i], m[i - 1]);
-            const float dr = __fadd_rn(__fsub_rn(m[i + 1], m[i]), 1e-16f);
-            const float pos = (dl > 0.0f) ? dl : 0.0f;          // (diff_l > 0) * diff_l
-            const float neg = (dl < 0.0f) ? dl : 0.0f;
-            ft = (-floorf(__fmul_rn(pos, dr)) == 1.0f) ? 1 : 0;
-            fb = (-floorf(__fmul_rn(neg, dr)) == 1.0f) ? 1 : 0;
-        }
-        t[i] = ft;
-        bt[i] = fb;
+        const unsigned f = corner_flags(m, i, n);
+        t[i] = f & 1u;
+        bt[i] = f >> 1;
     }
 }
 
@@ -119,11 +108,7 @@ __global__ void __launch_bounds__(256) lfo_sections_kernel(float* __restrict__ o
         for (int s = s0; s < s1; ++s)
             if (sec_start[s] <= i && i < sec_start[s] + sec_len[s]) sec = s;
         if (sec < 0) continue;
-        const int shape = sec_shape[sec];
-        const float len = (float)sec_len[sec];
-        const bool rect = shape == MODFX_SHAPE_RECT_COS || shape == MODFX_SHAPE_INV_RECT_COS;
-        const LfoDesc d = make_lfo_desc(rect ? 0.5f : 1.0f, 0.0f, shape, 1.0f, len);
-        o[i] = lfo_value(d, i - sec_start[sec]);
+        o[i] = lfo_value(section_lfo(sec_shape[sec], (float)sec_len[sec]), i - sec_start[sec]);
     }
 }
 
@@ -163,39 +148,32 @@ extern "C" int modfx_find_corners_f32(const float* mod, uint8_t* top, uint8_t* b
     MODFX_REQUIRE(mod && top && bottom, "NULL pointer");
     MODFX_REQUIRE(rows >= 0 && n >= 1, "bad shape");
     if (rows == 0) return MODFX_OK;
-    MODFX_REQUIRE(rows <= 65535, "rows=%lld exceeds grid.y", (long long)rows);
-    int gx = (int)((n + 255) / 256);
-    if (gx > 256) gx = 256;
-    corners_kernel<<<dim3(gx, (unsigned)rows), 256, 0, as_stream(stream)>>>(mod, top, bottom, n);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    dim3 grid;
+    if (const int st = row_grid(grid, n, rows, 256)) return st;
+    return launch(corners_kernel, grid, 256, 0, as_stream(stream), mod, top, bottom, n);
 }
 
 extern "C" int modfx_lfo_sections_f32(float* out, int32_t B, int64_t n, const int32_t* sec_off,
                                       const int32_t* sec_start, const int32_t* sec_len, const int32_t* sec_shape,
                                       void* stream) {
     MODFX_REQUIRE(out && sec_off && sec_start && sec_len && sec_shape, "NULL pointer");
-    MODFX_REQUIRE(B >= 0 && B <= 65535 && n >= 1, "bad shape");
+    MODFX_REQUIRE(B >= 0 && n >= 1, "bad shape");
     if (B == 0) return MODFX_OK;
-    int gx = (int)((n + 255) / 256);
-    if (gx > 256) gx = 256;
-    lfo_sections_kernel<<<dim3(gx, B), 256, 0, as_stream(stream)>>>(out, n, sec_off, sec_start, sec_len, sec_shape);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    dim3 grid;
+    if (const int st = row_grid(grid, n, B, 256)) return st;
+    return launch(lfo_sections_kernel, grid, 256, 0, as_stream(stream), out, n, sec_off, sec_start, sec_len, sec_shape);
 }
 
 extern "C" int modfx_stretch_sections_f32(const float* in, float* out, int32_t B, int64_t n, const int32_t* sec_off,
                                           const int32_t* in_start, const int32_t* in_len, const int32_t* new_len,
                                           const int32_t* out_start, void* stream) {
     MODFX_REQUIRE(in && out && sec_off && in_start && in_len && new_len && out_start, "NULL pointer");
-    MODFX_REQUIRE(B >= 0 && B <= 65535 && n >= 1, "bad shape");
+    MODFX_REQUIRE(B >= 0 && n >= 1, "bad shape");
     if (B == 0) return MODFX_OK;
-    int gx = (int)((n + 255) / 256);
-    if (gx > 256) gx = 256;
-    stretch_sections_kernel<<<dim3(gx, B), 256, 0, as_stream(stream)>>>(in, out, n, sec_off, in_start, in_len,
-                                                                       new_len, out_start);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    dim3 grid;
+    if (const int st = row_grid(grid, n, B, 256)) return st;
+    return launch(stretch_sections_kernel, grid, 256, 0, as_stream(stream), in, out, n, sec_off, in_start, in_len,
+                  new_len, out_start);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -222,8 +200,7 @@ __global__ void __launch_bounds__(256) combined_cand_kernel(float* __restrict__ 
     const int row = blockIdx.y;                 // b * S + k
     const int b = row / S, k = row - b * S;
     const int shape = shapes[k];
-    const bool rect = shape == MODFX_SHAPE_RECT_COS || shape == MODFX_SHAPE_INV_RECT_COS;
-    // modulations.py:26-29: frequency and phase are halved for the rectified shapes (exact in float32)
+    const bool rect = is_rect(shape);
     const LfoDesc d = make_lfo_desc(rect ? freq[b] * 0.5f : freq[b], rect ? phase[b] * 0.5f : phase[b], shape, 1.0f, sr);
     float* o = cand + (int64_t)row * n;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) o[i] = lfo_value(d, i);
@@ -240,13 +217,7 @@ __global__ void __launch_bounds__(128) corner_list_kernel(const float* __restric
     int c = 0;
     for (int i0 = 0; i0 < n; i0 += kWarp) {
         const int i = i0 + lane;
-        bool fb = false;
-        if (i >= 1 && i <= n - 2) {
-            const float dl = __fsub_rn(m[i], m[i - 1]);
-            const float dr = __fadd_rn(__fsub_rn(m[i + 1], m[i]), 1e-16f);
-            const float neg = (dl < 0.0f) ? dl : 0.0f;
-            fb = (-floorf(__fmul_rn(neg, dr)) == 1.0f);
-        }
+        const bool fb = corner_flags(m, i, n) & 2u;
         const unsigned bal = __ballot_sync(kFull, fb);
         if (fb) {
             const int pos = c + __popc(bal & ((1u << lane) - 1u));
@@ -349,9 +320,7 @@ __global__ void __launch_bounds__(256) combined_fill_kernel(float* __restrict__ 
             const int start = cs[s];
             const float len = (float)(cs[s + 1] - start + 1);
             const int shape = shapes[words[w0 + s] % (uint32_t)S];      // util.choice(shapes), modulations.py:207
-            const bool rect = shape == MODFX_SHAPE_RECT_COS || shape == MODFX_SHAPE_INV_RECT_COS;
-            const LfoDesc d = make_lfo_desc(rect ? 0.5f : 1.0f, 0.0f, shape, 1.0f, len);       // modulations.py:208
-            v = lfo_value(d, i - start);
+            v = lfo_value(section_lfo(shape, len), i - start);
         }
         o[i] = v;
     }
@@ -376,21 +345,25 @@ extern "C" int modfx_combined_lfo_f32(float* out, int32_t B, int64_t n, float sr
     MODFX_REQUIRE(n_shapes >= 1 && n_shapes <= 64 && n_words >= 0, "bad shape list / word count");
     if (B == 0) return MODFX_OK;
     const int64_t rows = (int64_t)B * n_shapes;
-    MODFX_REQUIRE(rows <= 65535 * 64ll, "too many candidate rows");
+    dim3 cand_grid, fill_grid;
+    if (const int st = row_grid(cand_grid, n, rows, 64)) return st;
+    if (const int st = row_grid(fill_grid, n, B, 64)) return st;
     char* w = static_cast<char*>(workspace);
     float* cand = reinterpret_cast<float*>(w);          w += align256(rows * n * 4);
     int16_t* idx = reinterpret_cast<int16_t*>(w);       w += align256(rows * kMaxCorners * 2);
     int32_t* cnt = reinterpret_cast<int32_t*>(w);       w += align256(rows * 4);
     int32_t* woff = reinterpret_cast<int32_t*>(w);
     cudaStream_t s = as_stream(stream);
-    const int gx = (int)std::min<int64_t>((n + 255) / 256, 64);
-    MODFX_REQUIRE(rows <= 65535, "B * n_shapes = %lld exceeds grid.y", (long long)rows);
-    combined_cand_kernel<<<dim3(gx, (unsigned)rows), 256, 0, s>>>(cand, (int)n, sr, freq, phase, shapes, n_shapes);
-    corner_list_kernel<<<(unsigned)((rows + 3) / 4), 128, 0, s>>>(cand, (int)rows, (int)n, idx, cnt);
-    combined_scan_kernel<<<1, kScanThreads, 0, s>>>(words, n_words, cnt, B, n_shapes, base_out, woff, consumed_out);
-    combined_fill_kernel<<<dim3(gx, (unsigned)B), 256, 0, s>>>(out, (int)n, cand, idx, cnt, base_out, woff, words, shapes, n_shapes);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    int st = launch(combined_cand_kernel, cand_grid, 256, 0, s, cand, (int)n, sr, freq, phase, shapes, n_shapes);
+    if (st == MODFX_OK)
+        st = launch(corner_list_kernel, (unsigned)((rows + 3) / 4), 128, 0, s, cand, (int)rows, (int)n, idx, cnt);
+    if (st == MODFX_OK)
+        st = launch(combined_scan_kernel, 1, kScanThreads, 0, s, words, n_words, cnt, B, n_shapes, base_out, woff,
+                    consumed_out);
+    if (st == MODFX_OK)
+        st = launch(combined_fill_kernel, fill_grid, 256, 0, s, out, (int)n, cand, idx, cnt, base_out, woff, words, shapes,
+                    n_shapes);
+    return st;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -415,12 +388,8 @@ __global__ void __launch_bounds__(256) lfo_window_kernel(float* __restrict__ out
             o[i] = lfo_value(d, s0 + i);
             continue;
         }
-        const float src = __fmul_rn(scale, (float)i);
-        int i0 = min((int)src, n_window - 1);
-        const int i1 = i0 + ((i0 < n_window - 1) ? 1 : 0);
-        const float l1 = __fsub_rn(src, (float)i0);
-        const float l0 = __fsub_rn(1.0f, l1);
-        o[i] = __fmaf_rn(l0, lfo_value(d, s0 + i0), __fmul_rn(l1, lfo_value(d, s0 + i1)));
+        const LinearTaps<int> t = taps_ac(scale, i, n_window);
+        o[i] = blend(t, lfo_value(d, s0 + t.i0), lfo_value(d, s0 + t.i1));
     }
 }
 }  // namespace
@@ -433,10 +402,8 @@ extern "C" int modfx_lfo_window_f32(float* out, int32_t B, int64_t n_out, int64_
     MODFX_REQUIRE(B >= 0 && n_out >= 1 && n_window >= 1 && n_window < (1ll << 30) && n_out <= n_window && sr > 0.0f,
                   "bad arguments B=%d n_out=%lld n_window=%lld", B, (long long)n_out, (long long)n_window);
     if (B == 0) return MODFX_OK;
-    MODFX_REQUIRE(B <= 65535, "B=%d exceeds grid.y", B);
-    const int gx = (int)std::min<int64_t>((n_out + 255) / 256, 256);
-    lfo_window_kernel<<<dim3(gx, B), 256, 0, as_stream(stream)>>>(out, (int)n_out, (int)n_window, sr, freq, phase, shape,
-                                                                  exp_or_null, start_or_null);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    dim3 grid;
+    if (const int st = row_grid(grid, n_out, B, 256)) return st;
+    return launch(lfo_window_kernel, grid, 256, 0, as_stream(stream), out, (int)n_out, (int)n_window, sr, freq, phase,
+                  shape, exp_or_null, start_or_null);
 }

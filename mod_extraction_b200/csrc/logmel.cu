@@ -390,9 +390,8 @@ extern "C" int modfx_specaugment_fill_f32(float* out, int64_t R, int32_t n_mels,
     // same arithmetic as the kernel's own log of a clipped zero: lg2.approx(eps) * ln 2
     const float fill = is_log ? log2f(eps) * 0.69314718055994530942f : 0.0f;
     const int grid = (int)std::min<int64_t>((n + 255) / 256, (int64_t)num_sms() * 16);
-    specaugment_fill_kernel<<<grid, 256, 0, as_stream(stream)>>>(out, n, n_mels, n_frames, f0, f1, t0, t1, fill);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    return launch(specaugment_fill_kernel, grid, 256, 0, as_stream(stream), out, n, n_mels, n_frames, f0, f1, t0, t1,
+                  fill);
 }
 
 extern "C" int modfx_logmel_f32(const float* x, float* out, int64_t R, int64_t T, int32_t n_fft, int32_t hop,

@@ -538,6 +538,8 @@ int phaser_launch(PhaserArgs a, int32_t B, int64_t N, int64_t n_out, void* works
     const int n_blocks = (int)((N + a.block - 1) / a.block);
 
     a.n_seg = (int)((N + kSeg - 1) / kSeg);
+    const int64_t tiles = (int64_t)a.n_items * a.n_seg;
+    MODFX_REQUIRE(tiles < (1ll << 31), "too many segments in one call");
     a.ticket = reinterpret_cast<int*>(w);                                     w += 256;
     a.flags = reinterpret_cast<int*>(w);
     const int64_t flag_bytes = align_up((int64_t)a.n_items * a.n_seg * 4, 256);  w += flag_bytes;
@@ -546,14 +548,10 @@ int phaser_launch(PhaserArgs a, int32_t B, int64_t N, int64_t n_out, void* works
     else a.phc = reinterpret_cast<float*>(w);
     MODFX_CUDA_OK(cudaMemsetAsync(workspace, 0, (size_t)(256 + flag_bytes), s));
     const int pairs = a.n_items * n_blocks;
-    phaser_phase_kernel<<<(pairs + 127) / 128, 128, 0, s>>>(a, n_blocks);
-    const int64_t tiles = (int64_t)a.n_items * a.n_seg;
-    MODFX_REQUIRE(tiles < (1ll << 31), "too many segments in one call");
+    if (const int st = launch(phaser_phase_kernel, (pairs + 127) / 128, 128, 0, s, a, n_blocks)) return st;
     MODFX_CUDA_OK(cudaFuncSetAttribute(phaser_fused_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                                        cudaSharedmemCarveoutMaxShared));
-    phaser_fused_kernel<<<(unsigned)tiles, kFusedThreads, sizeof(float) * kFusedSmemFloats, s>>>(a);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    return launch(phaser_fused_kernel, (unsigned)tiles, kFusedThreads, sizeof(float) * kFusedSmemFloats, s, a);
 }
 
 }  // namespace

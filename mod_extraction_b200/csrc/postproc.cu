@@ -50,19 +50,6 @@ __global__ void __launch_bounds__(256) smoothen_kernel(const float* __restrict__
     }
 }
 
-// find_corners flags of sample i (see corners_kernel in lfo.cu): bit 0 = top, bit 1 = bottom
-__device__ __forceinline__ unsigned corner_flags(const float* m, int i, int n) {
-    if (i < 1 || i > n - 2) return 0u;
-    const float dl = __fsub_rn(m[i], m[i - 1]);
-    const float dr = __fadd_rn(__fsub_rn(m[i + 1], m[i]), 1e-16f);
-    const float pos = (dl > 0.0f) ? dl : 0.0f;
-    const float neg = (dl < 0.0f) ? dl : 0.0f;
-    unsigned f = 0;
-    if (-floorf(__fmul_rn(pos, dr)) == 1.0f) f |= 1u;
-    if (-floorf(__fmul_rn(neg, dr)) == 1.0f) f |= 2u;
-    return f;
-}
-
 constexpr int kMaxAnchors = 64;     // corners + the final sample; rows with more corners are left unchanged anyway
 constexpr int kRowsPerBlock = 4;    // warps per CTA, one row each
 
@@ -182,13 +169,10 @@ extern "C" int modfx_smoothen_f32(const float* in, float* out, int64_t rows, int
                   (long long)rows, (long long)n, window);
     if (rows == 0) return MODFX_OK;
     MODFX_REQUIRE(in && out, "NULL pointer");
-    MODFX_REQUIRE(rows <= 65535, "rows=%lld exceeds grid.y", (long long)rows);
     const int64_t n_out = n - window + 1;
-    int gx = (int)((n_out + 255) / 256);
-    if (gx > 1024) gx = 1024;
-    smoothen_kernel<<<dim3(gx, (unsigned)rows), 256, 0, as_stream(stream)>>>(in, out, n, n_out, window);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    dim3 grid;
+    if (const int st = row_grid(grid, n_out, rows, 1024)) return st;
+    return launch(smoothen_kernel, grid, 256, 0, as_stream(stream), in, out, n, n_out, window);
 }
 
 extern "C" int modfx_stretch_corners_f32(const float* in, float* out, int64_t rows, int64_t n, int32_t max_n_corners,
@@ -201,9 +185,8 @@ extern "C" int modfx_stretch_corners_f32(const float* in, float* out, int64_t ro
     MODFX_REQUIRE(in && out && in != out, "NULL or aliased pointer");
     MODFX_REQUIRE(rows < (1ll << 31), "too many rows");
     const unsigned grid = (unsigned)((rows + kRowsPerBlock - 1) / kRowsPerBlock);
-    stretch_corners_kernel<<<grid, 32 * kRowsPerBlock, 0, as_stream(stream)>>>(in, out, (int)rows, (int)n, max_n_corners);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    return launch(stretch_corners_kernel, grid, 32 * kRowsPerBlock, 0, as_stream(stream), in, out, (int)rows, (int)n,
+                  max_n_corners);
 }
 
 extern "C" int modfx_check_mod_sig_f32(const float* in, uint8_t* valid, int64_t rows, int64_t n, int32_t min_top,
@@ -214,8 +197,6 @@ extern "C" int modfx_check_mod_sig_f32(const float* in, uint8_t* valid, int64_t 
     MODFX_REQUIRE(in && valid, "NULL pointer");
     MODFX_REQUIRE(rows < (1ll << 31), "too many rows");
     const unsigned grid = (unsigned)((rows + kRowsPerBlock - 1) / kRowsPerBlock);
-    check_mod_sig_kernel<<<grid, 32 * kRowsPerBlock, 0, as_stream(stream)>>>(in, valid, (int)rows, (int)n, min_top, max_top,
-                                                                             min_bottom, max_bottom, min_frames);
-    MODFX_CUDA_OK(cudaGetLastError());
-    return MODFX_OK;
+    return launch(check_mod_sig_kernel, grid, 32 * kRowsPerBlock, 0, as_stream(stream), in, valid, (int)rows, (int)n,
+                  min_top, max_top, min_bottom, max_bottom, min_frames);
 }

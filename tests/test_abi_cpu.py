@@ -156,6 +156,70 @@ def test_effect_entry_points_validate_before_touching_the_gpu():
     assert L.modfx_phaser_crop_packed_f32(p, p, p, nul, 1, 64, 64, p, sr, p, p, p, p, p, 0, nul, 0, p, nul) == -1
 
 
+def test_lfo_and_postproc_entry_points_validate_before_touching_the_gpu():
+    """Argument checks of the LFO, resampling, post-processing, SpecAugment and layer-norm entry points run on the host:
+    per entry point a NULL pointer, a bad shape, an empty batch (MODFX_OK) and more rows than one launch grid holds."""
+    import ctypes
+    L = _lib.lib()
+    buf = (ctypes.c_float * 64)()
+    p = ctypes.cast(buf, ctypes.c_void_p)
+    q = ctypes.cast(ctypes.addressof(buf) + 64, ctypes.c_void_p)
+    nul = ctypes.c_void_p(0)
+    too_many = 65536                                                            # grid.y holds 65535 rows
+
+    def lfo(out=p, B=1, n=64):
+        return L.modfx_lfo_f32(out, B, n, 100.0, p, p, p, nul, nul)
+    assert (lfo(out=nul), lfo(n=0), lfo(B=0), lfo(B=too_many)) == (-1, -1, 0, -1)
+
+    def window(out=p, B=1, n_out=64, n_window=64):
+        return L.modfx_lfo_window_f32(out, B, n_out, n_window, 100.0, p, p, p, nul, nul, nul)
+    assert (window(out=nul), window(n_out=65), window(B=0), window(B=too_many)) == (-1, -1, 0, -1)
+
+    def interp(x=p, rows=1, I=8):
+        return L.modfx_interp_linear_f32(x, q, rows, I, 16, 1, nul)
+    assert (interp(x=nul), interp(I=0), interp(rows=0), interp(rows=too_many)) == (-1, -1, 0, -1)
+
+    def corners(mod=p, rows=1, n=64):
+        return L.modfx_find_corners_f32(mod, q, q, rows, n, nul)
+    assert (corners(mod=nul), corners(n=0), corners(rows=0), corners(rows=too_many)) == (-1, -1, 0, -1)
+
+    def sections(out=p, B=1, n=64):
+        return L.modfx_lfo_sections_f32(out, B, n, p, p, p, p, nul)
+    assert (sections(out=nul), sections(n=0), sections(B=0), sections(B=too_many)) == (-1, -1, 0, -1)
+
+    def stretch_sections(x=p, B=1, n=64):
+        return L.modfx_stretch_sections_f32(x, q, B, n, p, p, p, p, p, nul)
+    assert (stretch_sections(x=nul), stretch_sections(n=0), stretch_sections(B=0),
+            stretch_sections(B=too_many)) == (-1, -1, 0, -1)
+
+    def combined(out=p, B=1, n=64, n_shapes=4):
+        return L.modfx_combined_lfo_f32(out, B, n, 100.0, p, p, p, n_shapes, p, 64, p, p, p, nul)
+    assert (combined(out=nul), combined(n=2), combined(B=0), combined(B=too_many, n_shapes=1),
+            combined(B=too_many // 64, n_shapes=64), combined(B=65535 * 64 + 1, n_shapes=1)) == (-1, -1, 0, -1, -1, -1)
+
+    def smoothen(x=p, rows=1, window=4):
+        return L.modfx_smoothen_f32(x, q, rows, 64, window, nul)
+    assert (smoothen(x=nul), smoothen(window=65), smoothen(rows=0), smoothen(rows=too_many)) == (-1, -1, 0, -1)
+
+    def stretch_corners(x=p, rows=1, n=64):
+        return L.modfx_stretch_corners_f32(x, q, rows, n, 8, nul)
+    assert (stretch_corners(x=nul), stretch_corners(n=0), stretch_corners(rows=0),
+            stretch_corners(rows=1 << 31)) == (-1, -1, 0, -1)                  # one row per warp along grid.x
+
+    def check(x=p, rows=1, n=64):
+        return L.modfx_check_mod_sig_f32(x, q, rows, n, 1, 4, 1, 4, 2, nul)
+    assert (check(x=nul), check(n=0), check(rows=0), check(rows=1 << 31)) == (-1, -1, 0, -1)
+
+    def specaugment(out=p, R=1, n_mels=4):                                      # one grid-stride loop: no row limit
+        return L.modfx_specaugment_fill_f32(out, R, n_mels, 4, 0, 1, 0, 1, 1e-7, 1, nul)
+    assert (specaugment(out=nul), specaugment(n_mels=0), specaugment(R=0)) == (-1, -1, 0)
+
+    def layernorm(x=p, B=1, C=2, nchw=0):
+        return L.modfx_cnn_layernorm_f32(x, q, B, C, 4, 4, nchw, 1e-5, 0, p, nul)
+    assert (layernorm(x=nul), layernorm(C=0), layernorm(B=0), layernorm(B=too_many),
+            layernorm(B=too_many // 64, C=64, nchw=1)) == (-1, -1, 0, -1, -1)  # NCHW: one row per (example, channel)
+
+
 def test_build_is_keyed_by_source_content():
     """_build.build() must not reuse a library built from other sources: the hash of csrc/ + include/ + flags is stored
     beside the library and compared, whatever the file times say."""
