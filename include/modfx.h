@@ -323,6 +323,35 @@ int modfx_phaser_crop_packed_f32(const float* x, const int64_t* x_offset, float*
  *   modfx_cnn_head_f32        replaces tr.mean(x, dim=-2), Conv1d(C, L, 1) and tr.sigmoid,
  *                             models.py:210-214: x (B, H, W, C) -> latent (B, C, W), out (B, L, W).
  *                             weight (L, C), bias (L,).
+ *
+ * Training (parameter gradients only, TF32, the shipped 5x13 / 64-channel shape).  Gradient semantics are those of
+ * cuDNN TF32 training: operand rounding is a straight-through step, the max-pool routes to the upper row of a tied
+ * pair, the layer-norm backward uses the unrounded normalised value.  Every reduction is a fixed-order sum of per-CTA
+ * partials: results are bit-reproducible.  `workspace`: modfx_cnn_train_workspace_bytes(B, H, W, L) bytes, H = the
+ * largest conv-input height of the call (the network's n_mels covers every layer).
+ *   modfx_cnn_conv_pool_prelu_train_f32
+ *                             forward of Conv2d -> MaxPool2d((2, 1)) -> PReLU (models.py:187-190) that also keeps what
+ *                             its backward needs: y as modfx_cnn_conv_pool_prelu_f32 (MODFX_CNN_TF32, bit for bit),
+ *                             z (B, H/2, W, 64) = maxpool(conv) + bias and argmax (B, H/2, W, 64) bytes, 1 where the
+ *                             lower conv row of the pair won.  Cin = 64, or Cin = 2 with dil_w = 1.
+ *   modfx_cnn_conv_dgrad_tf32_f32
+ *                             input gradient of Conv2d(64, 64, (5, 13), dilation=(1, dil_w), padding="same"):
+ *                             dconv (B, H, W, 64) -> dx (B, H, W, 64), the same tensor-core convolution with
+ *                             weight_t[kh][kw][ci][co] = weight[4 - kh][12 - kw][co][ci] (TF32-rounded).
+ *   modfx_cnn_conv_wgrad_tf32_f32
+ *                             weight gradient of that Conv2d: x (B, H, W, Cin) (the TF32 conv input), dconv
+ *                             (B, H, W, 64) -> dweight (64, Cin, 5, 13), the parameter's own layout.  Cin = 64 on
+ *                             the tensor cores; Cin = 2 (dil_w = 1) on the CUDA cores.
+ *   modfx_cnn_pool_prelu_bwd_f32
+ *                             backward of MaxPool2d((2, 1)) -> PReLU: dy (B, H/2, W, 64), z, argmax, prelu ->
+ *                             dconv (B, H, W, 64) rounded to TF32, dbias (64,) and dprelu (64,).
+ *   modfx_cnn_layernorm_bwd_f32
+ *                             input gradient of nn.LayerNorm(elementwise_affine=False) (models.py:186): g and x
+ *                             (B, H, W, C) channels-last, stats = the workspace modfx_cnn_layernorm_f32 filled in the
+ *                             forward of x (left untouched since) -> dx = rstd (g - mean(g) - xhat mean(g xhat)).
+ *   modfx_cnn_head_bwd_f32    backward of tr.mean(x, dim=-2), Conv1d(C, L, 1) and tr.sigmoid (models.py:210-214):
+ *                             latent (B, C, W), out (B, L, W), dout, dlatent -> dx (B, H, W, C), dweight (L, C),
+ *                             dbias (L,).
  */
 typedef enum {
     MODFX_CNN_FP32 = 0,
@@ -343,6 +372,23 @@ int modfx_cnn_conv_pool_prelu_f16_f32(const void* x_f16, float* y, int32_t B, in
                                       const void* w_f16, const float* bias, const float* prelu, void* stream);
 int modfx_cnn_head_f32(const float* x, float* latent, float* out, int32_t B, int32_t H, int32_t W, int32_t C,
                        int32_t L, const float* weight, const float* bias, void* stream);
+
+int64_t modfx_cnn_train_workspace_bytes(int32_t B, int32_t H, int32_t W, int32_t L);
+int modfx_cnn_conv_pool_prelu_train_f32(const float* x, float* y, float* z, uint8_t* argmax, int32_t B, int32_t H,
+                                        int32_t W, int32_t Cin, int32_t dil_w, const float* weight, const float* bias,
+                                        const float* prelu, void* stream);
+int modfx_cnn_conv_dgrad_tf32_f32(const float* dconv, float* dx, int32_t B, int32_t H, int32_t W, int32_t dil_w,
+                                  const float* weight_t, void* stream);
+int modfx_cnn_conv_wgrad_tf32_f32(const float* x, const float* dconv, float* dweight, int32_t B, int32_t H, int32_t W,
+                                  int32_t Cin, int32_t dil_w, void* workspace, void* stream);
+int modfx_cnn_pool_prelu_bwd_f32(const float* dy, const float* z, const uint8_t* argmax, const float* prelu, float* dconv,
+                                 float* dbias, float* dprelu, int32_t B, int32_t H, int32_t W, void* workspace,
+                                 void* stream);
+int modfx_cnn_layernorm_bwd_f32(const float* g, const float* x, const void* stats, float* dx, int32_t B, int32_t C,
+                                int32_t H, int32_t W, float eps, void* workspace, void* stream);
+int modfx_cnn_head_bwd_f32(const float* latent, const float* out, const float* dout, const float* dlatent, float* dx,
+                           float* dweight, float* dbias, int32_t B, int32_t H, int32_t W, int32_t C, int32_t L,
+                           const float* weight, void* workspace, void* stream);
 
 #ifdef __cplusplus
 }

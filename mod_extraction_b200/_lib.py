@@ -85,6 +85,13 @@ _SIGNATURES = {
     "modfx_cnn_conv_pool_prelu_tf32x3_f32": ([_vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp], ctypes.c_int),
     "modfx_cnn_conv_pool_prelu_f16_f32": ([_vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp], ctypes.c_int),
     "modfx_cnn_head_f32": ([_vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp], ctypes.c_int),
+    "modfx_cnn_train_workspace_bytes": ([_i32, _i32, _i32, _i32], _i64),
+    "modfx_cnn_conv_pool_prelu_train_f32": ([_vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp], ctypes.c_int),
+    "modfx_cnn_conv_dgrad_tf32_f32": ([_vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp], ctypes.c_int),
+    "modfx_cnn_conv_wgrad_tf32_f32": ([_vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp], ctypes.c_int),
+    "modfx_cnn_pool_prelu_bwd_f32": ([_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp], ctypes.c_int),
+    "modfx_cnn_layernorm_bwd_f32": ([_vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, ctypes.c_float, _vp, _vp], ctypes.c_int),
+    "modfx_cnn_head_bwd_f32": ([_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp], ctypes.c_int),
     "modfx_phaser_workspace_bytes": ([_i32, _i64], _i64),
     "modfx_phaser_f32": ([_vp, _vp, _i32, _i64, ctypes.c_float, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _i32, _vp, _vp],
                          ctypes.c_int),

@@ -462,3 +462,106 @@ def cnn_head(x: Tensor, weight: Tensor, bias: Tensor):
         _lib.check(_lib.lib().modfx_cnn_head_f32(_ptr(x), _ptr(latent), _ptr(out), B, H, W, C, Ld, _ptr(weight), _ptr(bias),
                                                  _stream()))
     return out, latent
+
+
+# ---- training (TF32 parameter gradients of the body, models.Spectral2DCNN) ----------------------------------------
+
+def _train_ws(B: int, H: int, W: int, L: int, device) -> Tensor:
+    return torch.empty(int(_lib.lib().modfx_cnn_train_workspace_bytes(B, H, W, L)), dtype=torch.uint8, device=device)
+
+
+def cnn_conv_pool_prelu_train(x: Tensor, weight: Tensor, bias: Tensor, slope: Tensor, dil_w: int = 1):
+    """cnn_conv_pool_prelu (TF32) that also returns what its backward needs: (y, z = maxpool(conv) + bias, argmax uint8,
+    1 where the lower conv row of a pooled pair won)."""
+    for t, n in ((x, "x"), (weight, "weight"), (bias, "bias"), (slope, "slope")):
+        _require_cuda(t, n)
+    x, weight, bias, slope = x.contiguous(), weight.contiguous(), bias.contiguous(), slope.contiguous()
+    B, H, W, Cin = x.shape
+    y = torch.empty((B, H // 2, W, 64), device=x.device, dtype=torch.float32)
+    z = torch.empty_like(y)
+    am = torch.empty((B, H // 2, W, 64), device=x.device, dtype=torch.uint8)
+    with torch.cuda.device(x.device):
+        _lib.check(_lib.lib().modfx_cnn_conv_pool_prelu_train_f32(_ptr(x), _ptr(y), _ptr(z), _ptr(am), B, H, W, Cin, int(dil_w),
+                                                                  _ptr(weight), _ptr(bias), _ptr(slope), _stream()))
+    return y, z, am
+
+
+def cnn_conv_dgrad(dconv: Tensor, weight_t: Tensor, dil_w: int = 1) -> Tensor:
+    """Input gradient of the 64 -> 64 convolution: dconv (B, H, W, 64), weight_t[kh][kw][ci][co] = weight[4-kh][12-kw][co][ci]."""
+    _require_cuda(dconv, "dconv")
+    _require_cuda(weight_t, "weight_t")
+    dconv, weight_t = dconv.contiguous(), weight_t.contiguous()
+    B, H, W, _ = dconv.shape
+    dx = torch.empty_like(dconv)
+    with torch.cuda.device(dconv.device):
+        _lib.check(_lib.lib().modfx_cnn_conv_dgrad_tf32_f32(_ptr(dconv), _ptr(dx), B, H, W, int(dil_w), _ptr(weight_t), _stream()))
+    return dx
+
+
+def cnn_conv_wgrad(x: Tensor, dconv: Tensor, dil_w: int = 1) -> Tensor:
+    """Weight gradient (64, Cin, 5, 13) of the convolution: x (B, H, W, Cin) its TF32 input, dconv (B, H, W, 64)."""
+    _require_cuda(x, "x")
+    _require_cuda(dconv, "dconv")
+    x, dconv = x.contiguous(), dconv.contiguous()
+    B, H, W, Cin = x.shape
+    dw = torch.empty((64, Cin, 5, 13), device=x.device, dtype=torch.float32)
+    ws = _train_ws(B, H, W, 1, x.device)
+    with torch.cuda.device(x.device):
+        _lib.check(_lib.lib().modfx_cnn_conv_wgrad_tf32_f32(_ptr(x), _ptr(dconv), _ptr(dw), B, H, W, Cin, int(dil_w), _ptr(ws),
+                                                            _stream()))
+        ws.record_stream(torch.cuda.current_stream())
+    return dw
+
+
+def cnn_pool_prelu_bwd(dy: Tensor, z: Tensor, argmax: Tensor, slope: Tensor):
+    """Backward of MaxPool2d((2, 1)) -> PReLU: (dconv (B, H, W, 64) rounded to TF32, dbias (64,), dslope (64,))."""
+    for t, n in ((dy, "dy"), (z, "z"), (argmax, "argmax"), (slope, "slope")):
+        _require_cuda(t, n)
+    dy, z, argmax, slope = dy.contiguous(), z.contiguous(), argmax.contiguous(), slope.contiguous()
+    B, Hp, W, C = dy.shape
+    dconv = torch.empty((B, 2 * Hp, W, C), device=dy.device, dtype=torch.float32)
+    db = torch.empty(C, device=dy.device, dtype=torch.float32)
+    ds = torch.empty(C, device=dy.device, dtype=torch.float32)
+    ws = _train_ws(B, 2 * Hp, W, 1, dy.device)
+    with torch.cuda.device(dy.device):
+        _lib.check(_lib.lib().modfx_cnn_pool_prelu_bwd_f32(_ptr(dy), _ptr(z), _ptr(argmax), _ptr(slope), _ptr(dconv), _ptr(db),
+                                                           _ptr(ds), B, 2 * Hp, W, _ptr(ws), _stream()))
+        ws.record_stream(torch.cuda.current_stream())
+    return dconv, db, ds
+
+
+def cnn_layernorm_bwd(g: Tensor, x: Tensor, eps: float = 1e-5) -> Tensor:
+    """Input gradient of cnn_layernorm on a channels-last x (B, H, W, C), given the output gradient g."""
+    _require_cuda(g, "g")
+    _require_cuda(x, "x")
+    g, x = g.contiguous(), x.contiguous()
+    B, H, W, C = x.shape
+    L = _lib.lib()
+    stats = torch.empty(max(int(L.modfx_cnn_layernorm_workspace_bytes(B, C, H, W)), 16), dtype=torch.uint8, device=x.device)
+    ws = _train_ws(B, H, W, 1, x.device)
+    dx = torch.empty_like(x)
+    with torch.cuda.device(x.device):
+        _lib.check(L.modfx_cnn_layernorm_f32(_ptr(x), _ptr(dx), B, C, H, W, 0, float(eps), 0, _ptr(stats), _stream()))   # statistics
+        _lib.check(L.modfx_cnn_layernorm_bwd_f32(_ptr(g), _ptr(x), _ptr(stats), _ptr(dx), B, C, H, W, float(eps), _ptr(ws),
+                                                 _stream()))
+        ws.record_stream(torch.cuda.current_stream())
+        stats.record_stream(torch.cuda.current_stream())
+    return dx
+
+
+def cnn_head_bwd(latent: Tensor, out: Tensor, dout: Tensor, dlatent: Tensor, weight: Tensor, H: int):
+    """Backward of cnn_head: (dx (B, H, W, C), dweight (L, C), dbias (L,))."""
+    for t, n in ((latent, "latent"), (out, "out"), (dout, "dout"), (dlatent, "dlatent"), (weight, "weight")):
+        _require_cuda(t, n)
+    latent, out, dout, dlatent, weight = (t.contiguous() for t in (latent, out, dout, dlatent, weight))
+    B, C, W = latent.shape
+    Ld = out.size(1)
+    dx = torch.empty((B, H, W, C), device=latent.device, dtype=torch.float32)
+    dw = torch.empty((Ld, C), device=latent.device, dtype=torch.float32)
+    db = torch.empty(Ld, device=latent.device, dtype=torch.float32)
+    ws = _train_ws(B, 2, W, Ld, latent.device)
+    with torch.cuda.device(latent.device):
+        _lib.check(_lib.lib().modfx_cnn_head_bwd_f32(_ptr(latent), _ptr(out), _ptr(dout), _ptr(dlatent), _ptr(dx), _ptr(dw),
+                                                     _ptr(db), B, int(H), W, C, Ld, _ptr(weight), _ptr(ws), _stream()))
+        ws.record_stream(torch.cuda.current_stream())
+    return dx, dw, db

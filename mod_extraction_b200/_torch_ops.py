@@ -22,6 +22,12 @@ libmodfx.so of ``_ops.py``; registering them costs nothing when the ops are not 
     torch.ops.modfx.cnn_layernorm(x, x_is_nchw, eps, round_tf32)               # -> channels-last (B, H, W, C)
     torch.ops.modfx.cnn_conv_pool_prelu(x, weight, bias, slope, dil_w, tf32)    # tcgen05 when tf32
     torch.ops.modfx.cnn_head(x, weight, bias)                                   # -> (output, latent)
+    torch.ops.modfx.cnn_conv_pool_prelu_train(x, weight, bias, slope, dil_w)    # -> (y, z, argmax), TF32
+    torch.ops.modfx.cnn_conv_dgrad(dconv, weight_t, dil_w)                      # TF32 training backward ...
+    torch.ops.modfx.cnn_conv_wgrad(x, dconv, dil_w)
+    torch.ops.modfx.cnn_pool_prelu_bwd(dy, z, argmax, slope)                    # -> (dconv, dbias, dslope)
+    torch.ops.modfx.cnn_layernorm_bwd(g, x, eps)
+    torch.ops.modfx.cnn_head_bwd(latent, out, dout, dlatent, weight, H)         # -> (dx, dweight, dbias)
 """
 from __future__ import annotations
 
@@ -53,6 +59,12 @@ _lib.define("check_mod_sig(Tensor x, int min_top, int max_top, int min_bottom, i
 _lib.define("cnn_layernorm(Tensor x, bool x_is_nchw, float eps, bool round_tf32) -> Tensor")
 _lib.define("cnn_conv_pool_prelu(Tensor x, Tensor weight, Tensor bias, Tensor slope, int dil_w, bool tf32) -> Tensor")
 _lib.define("cnn_head(Tensor x, Tensor weight, Tensor bias) -> (Tensor, Tensor)")
+_lib.define("cnn_conv_pool_prelu_train(Tensor x, Tensor weight, Tensor bias, Tensor slope, int dil_w) -> (Tensor, Tensor, Tensor)")
+_lib.define("cnn_conv_dgrad(Tensor dconv, Tensor weight_t, int dil_w) -> Tensor")
+_lib.define("cnn_conv_wgrad(Tensor x, Tensor dconv, int dil_w) -> Tensor")
+_lib.define("cnn_pool_prelu_bwd(Tensor dy, Tensor z, Tensor argmax, Tensor slope) -> (Tensor, Tensor, Tensor)")
+_lib.define("cnn_layernorm_bwd(Tensor g, Tensor x, float eps) -> Tensor")
+_lib.define("cnn_head_bwd(Tensor latent, Tensor out, Tensor dout, Tensor dlatent, Tensor weight, int H) -> (Tensor, Tensor, Tensor)")
 
 
 def _flanger_chorus(x: Tensor, mod: Tensor, feedback: Tensor, min_delay_width: Tensor, width: Tensor, depth: Tensor,
@@ -109,3 +121,9 @@ _impl.impl("cnn_layernorm", lambda x, x_is_nchw, eps, round_tf32: _ops.cnn_layer
 _impl.impl("cnn_conv_pool_prelu", lambda x, weight, bias, slope, dil_w, tf32: _ops.cnn_conv_pool_prelu(x, weight, bias, slope,
                                                                                                       dil_w, tf32))
 _impl.impl("cnn_head", lambda x, weight, bias: _ops.cnn_head(x, weight, bias))
+_impl.impl("cnn_conv_pool_prelu_train", lambda x, w, b, s, d: _ops.cnn_conv_pool_prelu_train(x, w, b, s, d))
+_impl.impl("cnn_conv_dgrad", lambda dconv, weight_t, dil_w: _ops.cnn_conv_dgrad(dconv, weight_t, dil_w))
+_impl.impl("cnn_conv_wgrad", lambda x, dconv, dil_w: _ops.cnn_conv_wgrad(x, dconv, dil_w))
+_impl.impl("cnn_pool_prelu_bwd", lambda dy, z, am, slope: _ops.cnn_pool_prelu_bwd(dy, z, am, slope))
+_impl.impl("cnn_layernorm_bwd", lambda g, x, eps: _ops.cnn_layernorm_bwd(g, x, eps))
+_impl.impl("cnn_head_bwd", lambda latent, out, dout, dlatent, weight, H: _ops.cnn_head_bwd(latent, out, dout, dlatent, weight, H))

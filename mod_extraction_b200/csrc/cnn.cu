@@ -20,6 +20,13 @@ int cnn_conv_tf32(const void* x, const void* x_lo, float* y, int B, int H, int W
                   const void* w_lo, const float* bias, const float* prelu, bool half, cudaStream_t stream);   // cnn_tc.cu
 int cnn_conv1_tf32(const float* x, float* y, int B, int H, int W, const float* weight, const float* bias,
                    const float* prelu, cudaStream_t stream);     // cnn_tc.cu (2 input channels, dilation 1)
+int cnn_conv_tf32_grad(const float* x, float* y, float* z, uint8_t* am, int B, int H, int W, int dil, const float* weight,
+                       const float* bias, const float* prelu, cudaStream_t stream);            // cnn_tc.cu
+int cnn_conv1_tf32_train(const float* x, float* y, float* z, uint8_t* am, int B, int H, int W, const float* weight,
+                         const float* bias, const float* prelu, cudaStream_t stream);          // cnn_tc.cu
+int cnn_conv_wgrad_tf32(const float* x, const float* dconv, float* part, int B, int H, int W, int dil,
+                        cudaStream_t stream);                                                  // cnn_tc.cu
+int cnn_wgrad_splits();
 
 namespace {
 
@@ -284,6 +291,249 @@ __global__ void __launch_bounds__(256) head_kernel(const float* __restrict__ x, 
 
 int ln_chunks(int64_t row_len) { return (int)((row_len + kLnChunkElems - 1) / kLnChunkElems); }
 
+// ==== backward pass of the body (training, TF32 semantics: operand rounding is a straight-through step) ==========
+// Every reduction writes one partial per CTA; sum_parts_kernel adds them in a fixed order, so gradients are
+// bit-reproducible run to run.
+
+// out[i] = sum_k part[k * n + i] (k ascending); i < n0 goes to out0, the rest to out1
+__global__ void __launch_bounds__(256) sum_parts_kernel(const float* __restrict__ part, int n_parts, int64_t n, int64_t n0,
+                                                        float* __restrict__ out0, float* __restrict__ out1) {
+    const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    float s = 0.0f;
+    for (int k = 0; k < n_parts; ++k) s += part[(int64_t)k * n + i];
+    if (i < n0) out0[i] = s;
+    else out1[i - n0] = s;
+}
+
+// ---- max-pool (2x1) + PReLU backward: dA (B, H/2, W, 64) -> dConv (B, H, W, 64) rounded to TF32 (the operand of both
+// gradient GEMMs); the pool routes dz = dA * PReLU'(z) to the conv row its argmax names.  Partials per CTA:
+// [0, 64) dbias = sum dz, [64, 128) dslope = sum dA * z * [z <= 0].
+constexpr int kBwdChunk = 64 * 1024;          // pooled elements per CTA
+__global__ void __launch_bounds__(256) pool_prelu_bwd_kernel(const float* __restrict__ dA, const float* __restrict__ z,
+                                                             const uint8_t* __restrict__ am,
+                                                             const float* __restrict__ slope, float* __restrict__ dconv,
+                                                             float* __restrict__ part, int64_t n, int W) {
+    __shared__ float s_b[256], s_s[256];
+    const int tid = threadIdx.x, c = tid & 63;
+    const float a = slope[c];
+    const int64_t e0 = (int64_t)blockIdx.x * kBwdChunk, e1 = min(e0 + kBwdChunk, n);
+    float sb = 0.0f, ss = 0.0f;
+    for (int64_t e = e0 + tid; e < e1; e += 256) {
+        const int64_t pix = e >> 6, bp = pix / W, w = pix - bp * W;
+        const float g = dA[e], zv = z[e];
+        const float dz = zv > 0.0f ? g : a * g;
+        sb += dz;
+        if (zv <= 0.0f) ss += g * zv;
+        const int64_t up = ((2 * bp * W + w) << 6) + c, lo = up + ((int64_t)W << 6);
+        const float r = round_tf32(dz);
+        dconv[up] = am[e] ? 0.0f : r;
+        dconv[lo] = am[e] ? r : 0.0f;
+    }
+    s_b[tid] = sb;
+    s_s[tid] = ss;
+    __syncthreads();
+    if (tid < 64) {
+        float tb = 0.0f, ts = 0.0f;
+        for (int t = tid; t < 256; t += 64) {
+            tb += s_b[t];
+            ts += s_s[t];
+        }
+        part[(int64_t)blockIdx.x * 128 + tid] = tb;
+        part[(int64_t)blockIdx.x * 128 + 64 + tid] = ts;
+    }
+}
+
+// mean / rstd of (b, c) from the partial sums of the forward's ln_stats_kernel, exactly as ln_apply_kernel<false> forms them
+__device__ __forceinline__ float2 ln_stat(const double* __restrict__ part, int64_t b, int c, int C, int chunks, int64_t P,
+                                          float eps) {
+    double ts = 0.0, tq = 0.0;
+    const double* p = part + (b * chunks * C + c) * 2;
+    for (int k = 0; k < chunks; ++k) { ts += p[(int64_t)k * C * 2]; tq += p[(int64_t)k * C * 2 + 1]; }
+    const double mean = ts / (double)P;
+    const double var = fmax(tq / (double)P - mean * mean, 0.0);
+    return make_float2((float)mean, (float)(1.0 / sqrt(var + (double)eps)));
+}
+
+// ---- layer norm backward, pass 1: per-chunk sums of g and g * xhat per (b, c), xhat = (x - mean) * rstd unrounded
+__global__ void __launch_bounds__(kLnThreads) ln_bwd_stats_kernel(const float* __restrict__ g, const float* __restrict__ x,
+                                                                  const double* __restrict__ fwd, double* __restrict__ part,
+                                                                  int64_t P, int C, int chunks, float eps) {
+    __shared__ double s_sum[kLnThreads], s_gx[kLnThreads];
+    __shared__ float s_stat[2 * kLnThreads];
+    const int tid = threadIdx.x;
+    const int64_t b = blockIdx.y, n = P * C;
+    for (int c = tid; c < C; c += kLnThreads) {
+        const float2 mr = ln_stat(fwd, b, c, C, chunks, P, eps);
+        s_stat[c] = mr.x;
+        s_stat[C + c] = mr.y;
+    }
+    __syncthreads();
+    const int64_t e0 = (int64_t)blockIdx.x * kLnChunkElems, e1 = min(e0 + kLnChunkElems, n);
+    const int c = tid % C;
+    const float m = s_stat[c], r = s_stat[C + c];
+    double s = 0.0, q = 0.0;
+    for (int64_t e = e0 + tid; e < e1; e += kLnThreads) {
+        const float gv = g[b * n + e];
+        const float xh = (x[b * n + e] - m) * r;
+        s += (double)gv;
+        q += (double)gv * (double)xh;
+    }
+    s_sum[tid] = s;
+    s_gx[tid] = q;
+    __syncthreads();
+    if (tid < C) {
+        double ts = 0.0, tq = 0.0;
+        for (int t = tid; t < kLnThreads; t += C) {
+            ts += s_sum[t];
+            tq += s_gx[t];
+        }
+        double* p = part + ((b * chunks + blockIdx.x) * C + tid) * 2;
+        p[0] = ts;
+        p[1] = tq;
+    }
+}
+
+// ---- layer norm backward, pass 2: dx = rstd * (g - mean(g) - xhat * mean(g * xhat))
+__global__ void __launch_bounds__(kLnThreads) ln_bwd_apply_kernel(const float* __restrict__ g, const float* __restrict__ x,
+                                                                  const double* __restrict__ fwd,
+                                                                  const double* __restrict__ part, float* __restrict__ dx,
+                                                                  int64_t P, int C, int chunks, float eps) {
+    __shared__ float s_stat[4 * kLnThreads];    // mean, rstd, mean(g), mean(g * xhat)
+    const int tid = threadIdx.x;
+    const int64_t b = blockIdx.y, n = P * C;
+    for (int c = tid; c < C; c += kLnThreads) {
+        const float2 mr = ln_stat(fwd, b, c, C, chunks, P, eps);
+        s_stat[c] = mr.x;
+        s_stat[C + c] = mr.y;
+    }
+    for (int c = tid; c < C; c += kLnThreads) {
+        double ts = 0.0, tq = 0.0;
+        const double* p = part + (b * chunks * C + c) * 2;
+        for (int k = 0; k < chunks; ++k) { ts += p[(int64_t)k * C * 2]; tq += p[(int64_t)k * C * 2 + 1]; }
+        const double inv = 1.0 / (double)P;
+        s_stat[2 * C + c] = (float)(ts * inv);
+        s_stat[3 * C + c] = (float)(tq * inv);
+    }
+    __syncthreads();
+    const int64_t e0 = (int64_t)blockIdx.x * kLnChunkElems, e1 = min(e0 + kLnChunkElems, n);
+    const int c = tid % C;
+    const float m = s_stat[c], r = s_stat[C + c], mg = s_stat[2 * C + c], mgx = s_stat[3 * C + c];
+    for (int64_t e = e0 + tid; e < e1; e += kLnThreads) {
+        const float xh = (x[b * n + e] - m) * r;
+        dx[b * n + e] = r * (g[b * n + e] - mg - xh * mgx);
+    }
+}
+
+// ---- weight gradient of the 2-channel first layer on the CUDA cores (3 % of the backward's flops).  A CTA walks a fixed
+// range of (example, conv row, 64-frame) tiles; thread (co, g) keeps the 17 taps t = g + 4 j of output channel co for
+// both input channels.  Partial per CTA in the parameter's layout (64, 2, 5, 13).
+constexpr int kW1Tw = 64, kW1Parts = 296;
+__global__ void __launch_bounds__(256) wgrad1_kernel(const float* __restrict__ x, const float* __restrict__ dconv,
+                                                     float* __restrict__ part, int B, int H, int W) {
+    __shared__ float s_d[kW1Tw][kCo];
+    __shared__ float2 s_x[kKH][kW1Tw + kKW - 1];
+    const int tid = threadIdx.x, co = tid & 63, g = __shfl_sync(kFull, tid >> 6, 0);
+    const int ntw = (W + kW1Tw - 1) / kW1Tw;
+    const int64_t tiles = (int64_t)B * H * ntw;
+    const int64_t k0 = tiles * blockIdx.x / gridDim.x, k1 = tiles * (blockIdx.x + 1) / gridDim.x;
+    constexpr int kJ = (kKH * kKW + 3) / 4;     // 17
+    float acc[kJ][2];
+    int off[kJ];
+#pragma unroll
+    for (int j = 0; j < kJ; ++j) {
+        const int t = min(g + 4 * j, kKH * kKW - 1);
+        off[j] = (t / kKW) * (kW1Tw + kKW - 1) + t % kKW;
+        acc[j][0] = acc[j][1] = 0.0f;
+    }
+    for (int64_t k = k0; k < k1; ++k) {
+        const int tw = (int)(k % ntw);
+        const int64_t bh = k / ntw;
+        const int h = (int)(bh % H);
+        const int64_t b = bh / H;
+        const int w0 = tw * kW1Tw;
+        __syncthreads();
+        for (int i = tid; i < kW1Tw * kCo; i += 256) {
+            const int w = w0 + (i >> 6);
+            s_d[i >> 6][i & 63] = w < W ? dconv[((b * H + h) * W + w) * kCo + (i & 63)] : 0.0f;
+        }
+        for (int i = tid; i < kKH * (kW1Tw + kKW - 1); i += 256) {
+            const int r = i / (kW1Tw + kKW - 1), j = i - r * (kW1Tw + kKW - 1);
+            const int hr = h + r - kKH / 2, w = w0 + j - kKW / 2;
+            s_x[r][j] = (hr >= 0 && hr < H && w >= 0 && w < W)
+                            ? *reinterpret_cast<const float2*>(x + ((b * H + hr) * W + w) * 2)
+                            : make_float2(0.0f, 0.0f);
+        }
+        __syncthreads();
+        const float2* xs = &s_x[0][0];
+#pragma unroll 4
+        for (int w = 0; w < kW1Tw; ++w) {
+            const float d = s_d[w][co];
+#pragma unroll
+            for (int j = 0; j < kJ; ++j) {
+                const float2 v = xs[off[j] + w];
+                acc[j][0] = fmaf(d, v.x, acc[j][0]);
+                acc[j][1] = fmaf(d, v.y, acc[j][1]);
+            }
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < kJ; ++j) {
+        const int t = g + 4 * j;
+        if (t < kKH * kKW) {
+            part[(int64_t)blockIdx.x * kCo * 2 * kKH * kKW + (co * 2 + 0) * kKH * kKW + t] = acc[j][0];
+            part[(int64_t)blockIdx.x * kCo * 2 * kKH * kKW + (co * 2 + 1) * kKH * kKW + t] = acc[j][1];
+        }
+    }
+}
+
+// ---- head backward: out = sigmoid(W latent + b), latent = mean_H(x).  dx (B, H, W, C) = (W^T dlogit + dlatent) / H
+// on every row; partials per CTA: [0, L C) dW_out, [L C, L C + L) db_out.
+__global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__ latent, const float* __restrict__ out,
+                                                       const float* __restrict__ dout, const float* __restrict__ dlatent,
+                                                       float* __restrict__ dx, float* __restrict__ part, int H, int W,
+                                                       int C, int L, const float* __restrict__ weight) {
+    extern __shared__ float s_h[];              // [L][kHeadW + 1] dlogit, [C][kHeadW + 1] d(latent) / H
+    float* s_dl = s_h;
+    float* s_dt = s_h + L * (kHeadW + 1);
+    const int tid = threadIdx.x;
+    const int w0 = blockIdx.x * kHeadW;
+    const int64_t b = blockIdx.y;
+    const int nw = min(kHeadW, W - w0);
+    const float inv = 1.0f / (float)H;
+    for (int i = tid; i < L * nw; i += blockDim.x) {
+        const int l = i / nw, j = i - l * nw;
+        const int64_t o = (b * L + l) * (int64_t)W + w0 + j;
+        s_dl[l * (kHeadW + 1) + j] = dout[o] * out[o] * (1.0f - out[o]);
+    }
+    __syncthreads();
+    for (int i = tid; i < C * nw; i += blockDim.x) {
+        const int c = i / nw, j = i - c * nw;
+        float s = dlatent[(b * C + c) * (int64_t)W + w0 + j];
+        for (int l = 0; l < L; ++l) s = fmaf(weight[l * C + c], s_dl[l * (kHeadW + 1) + j], s);
+        s_dt[c * (kHeadW + 1) + j] = s * inv;
+    }
+    __syncthreads();
+    for (int64_t i = tid; i < (int64_t)H * nw * C; i += blockDim.x) {
+        const int c = (int)(i % C);
+        const int64_t hj = i / C;
+        const int j = (int)(hj % nw), h = (int)(hj / nw);
+        dx[((b * H + h) * (int64_t)W + w0 + j) * C + c] = s_dt[c * (kHeadW + 1) + j];
+    }
+    float* pp = part + (b * gridDim.x + blockIdx.x) * (int64_t)(L * C + L);
+    for (int i = tid; i < L * C + L; i += blockDim.x) {
+        const int l = i < L * C ? i / C : i - L * C, c = i < L * C ? i - l * C : -1;
+        float s = 0.0f;
+        for (int j = 0; j < nw; ++j)
+            s = fmaf(s_dl[l * (kHeadW + 1) + j], c >= 0 ? latent[(b * C + c) * (int64_t)W + w0 + j] : 1.0f, s);
+        pp[i] = s;
+    }
+}
+
+int sum_parts(const float* part, int n_parts, int64_t n, int64_t n0, float* out0, float* out1, cudaStream_t s) {
+    return launch(sum_parts_kernel, dim3((unsigned)((n + 255) / 256)), 256, 0, s, part, n_parts, n, n0, out0, out1);
+}
+
 }  // namespace
 }  // namespace modfx
 
@@ -403,4 +653,119 @@ extern "C" int modfx_cnn_head_f32(const float* x, float* latent, float* out, int
     MODFX_REQUIRE(B <= 65535, "B too large");
     return launch(head_kernel, dim3((W + kHeadW - 1) / kHeadW, B), 256, (size_t)C * (kHeadW + 1) * sizeof(float),
                   as_stream(stream), x, latent, out, H, W, C, L, weight, bias);
+}
+
+// ==== training: forward with saves, and the backward pass (TF32, the shipped 5x13 / 64-channel shape) ================
+
+extern "C" int64_t modfx_cnn_train_workspace_bytes(int32_t B, int32_t H, int32_t W, int32_t L) {
+    if (B < 0 || H < 2 || W < 1 || L < 1) return -1;
+    const int64_t wg = (int64_t)cnn_wgrad_splits() * kCo * kCo * kKH * kKW;
+    const int64_t wg1 = (int64_t)kW1Parts * kCo * 2 * kKH * kKW;
+    const int64_t pool = ((int64_t)B * (H / 2) * W * kCo + kBwdChunk - 1) / kBwdChunk * 128;
+    const int64_t ln = (int64_t)B * ln_chunks((int64_t)H * W * kCo) * kCo * 2 * 2;     // doubles, as floats
+    const int64_t head = (int64_t)B * ((W + kHeadW - 1) / kHeadW) * ((int64_t)L * kCo + L);
+    return std::max(std::max(std::max(wg, wg1), std::max(pool, ln)), head) * (int64_t)sizeof(float) + 16;
+}
+
+static float* ws_align(void* workspace) {
+    return reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(workspace) + 15) & ~(uintptr_t)15);
+}
+
+extern "C" int modfx_cnn_conv_pool_prelu_train_f32(const float* x, float* y, float* z, uint8_t* argmax, int32_t B,
+                                                   int32_t H, int32_t W, int32_t Cin, int32_t dil_w, const float* weight,
+                                                   const float* bias, const float* prelu, void* stream) {
+    MODFX_REQUIRE(x && y && z && argmax && weight && bias && prelu, "NULL pointer");
+    MODFX_REQUIRE(B >= 0 && H >= 2 && W >= 1, "bad shape B=%d H=%d W=%d", B, H, W);
+    MODFX_REQUIRE(x != y && x != z && y != z, "x, y and z must not alias");
+    if (const int st = check_conv_shape(B, H, dil_w); st != MODFX_OK || B == 0) return st;
+    cudaStream_t st = as_stream(stream);
+    if (Cin == 2 && dil_w == 1) return cnn_conv1_tf32_train(x, y, z, argmax, B, H, W, weight, bias, prelu, st);
+    if (Cin != 64)
+        return fail(MODFX_ERR_UNSUPPORTED, "the training forward is built for Cin=64, and Cin=2 with dilation 1 (got %d, %d)",
+                    Cin, dil_w);
+    return cnn_conv_tf32_grad(x, y, z, argmax, B, H, W, dil_w, weight, bias, prelu, st);
+}
+
+extern "C" int modfx_cnn_conv_dgrad_tf32_f32(const float* dconv, float* dx, int32_t B, int32_t H, int32_t W, int32_t dil_w,
+                                             const float* weight_t, void* stream) {
+    MODFX_REQUIRE(dconv && dx && weight_t, "NULL pointer");
+    MODFX_REQUIRE(B >= 0 && H >= 2 && W >= 1, "bad shape B=%d H=%d W=%d", B, H, W);
+    MODFX_REQUIRE(dconv != dx, "dconv and dx must not alias");
+    if (const int st = check_conv_shape(B, H, dil_w); st != MODFX_OK || B == 0) return st;
+    return cnn_conv_tf32_grad(dconv, dx, nullptr, nullptr, B, H, W, dil_w, weight_t, nullptr, nullptr, as_stream(stream));
+}
+
+extern "C" int modfx_cnn_conv_wgrad_tf32_f32(const float* x, const float* dconv, float* dweight, int32_t B, int32_t H,
+                                             int32_t W, int32_t Cin, int32_t dil_w, void* workspace, void* stream) {
+    MODFX_REQUIRE(x && dconv && dweight && workspace, "NULL pointer");
+    MODFX_REQUIRE(B >= 1 && H >= 2 && W >= 1, "bad shape B=%d H=%d W=%d (an empty batch has no gradient)", B, H, W);
+    if (const int st = check_conv_shape(B, H, dil_w); st != MODFX_OK) return st;
+    if (!(Cin == 64 || (Cin == 2 && dil_w == 1)))
+        return fail(MODFX_ERR_UNSUPPORTED, "the weight gradient is built for Cin=64, and Cin=2 with dilation 1 (got %d, %d)",
+                    Cin, dil_w);
+    float* part = ws_align(workspace);
+    cudaStream_t s = as_stream(stream);
+    const int64_t n = (int64_t)kCo * Cin * kKH * kKW;
+    int st;
+    int n_parts;
+    if (Cin == 2) {
+        const int64_t tiles = (int64_t)B * H * ((W + kW1Tw - 1) / kW1Tw);
+        n_parts = (int)std::min<int64_t>(tiles, kW1Parts);
+        st = launch(wgrad1_kernel, dim3(n_parts), 256, 0, s, x, dconv, part, B, H, W);
+    } else {
+        n_parts = cnn_wgrad_splits();
+        st = cnn_conv_wgrad_tf32(x, dconv, part, B, H, W, dil_w, s);
+    }
+    if (st != MODFX_OK) return st;
+    return sum_parts(part, n_parts, n, n, dweight, nullptr, s);
+}
+
+extern "C" int modfx_cnn_pool_prelu_bwd_f32(const float* dy, const float* z, const uint8_t* argmax, const float* prelu,
+                                            float* dconv, float* dbias, float* dprelu, int32_t B, int32_t H, int32_t W,
+                                            void* workspace, void* stream) {
+    MODFX_REQUIRE(dy && z && argmax && prelu && dconv && dbias && dprelu && workspace, "NULL pointer");
+    MODFX_REQUIRE(B >= 1 && H >= 2 && W >= 1 && !(H & 1), "bad shape B=%d H=%d W=%d (H even, an empty batch has no gradient)",
+                  B, H, W);
+    const int64_t n = (int64_t)B * (H / 2) * W * kCo;
+    const int64_t ctas = (n + kBwdChunk - 1) / kBwdChunk;
+    MODFX_REQUIRE(ctas <= 0x7fffffff, "too many elements");
+    float* part = ws_align(workspace);
+    cudaStream_t s = as_stream(stream);
+    const int st = launch(pool_prelu_bwd_kernel, dim3((unsigned)ctas), 256, 0, s, dy, z, argmax, prelu, dconv, part, n, W);
+    if (st != MODFX_OK) return st;
+    return sum_parts(part, (int)ctas, 2 * kCo, kCo, dbias, dprelu, s);
+}
+
+extern "C" int modfx_cnn_layernorm_bwd_f32(const float* g, const float* x, const void* stats, float* dx, int32_t B,
+                                           int32_t C, int32_t H, int32_t W, float eps, void* workspace, void* stream) {
+    MODFX_REQUIRE(g && x && stats && dx && workspace, "NULL pointer");
+    MODFX_REQUIRE(B >= 0 && C >= 1 && H >= 1 && W >= 1, "bad shape B=%d C=%d H=%d W=%d", B, C, H, W);
+    if (kLnThreads % C != 0) return fail(MODFX_ERR_UNSUPPORTED, "C=%d: the channel count must divide %d", C, kLnThreads);
+    if (B == 0) return MODFX_OK;
+    MODFX_REQUIRE(B <= 65535, "B=%d: at most 65535 examples per call", B);
+    const int64_t P = (int64_t)H * W;
+    const int chunks = ln_chunks(P * C);
+    const double* fwd = reinterpret_cast<const double*>((reinterpret_cast<uintptr_t>(stats) + 15) & ~(uintptr_t)15);
+    double* part = reinterpret_cast<double*>(ws_align(workspace));
+    cudaStream_t s = as_stream(stream);
+    const int st = launch(ln_bwd_stats_kernel, dim3(chunks, B), kLnThreads, 0, s, g, x, fwd, part, P, C, chunks, eps);
+    if (st != MODFX_OK) return st;
+    return launch(ln_bwd_apply_kernel, dim3(chunks, B), kLnThreads, 0, s, g, x, fwd, (const double*)part, dx, P, C, chunks,
+                  eps);
+}
+
+extern "C" int modfx_cnn_head_bwd_f32(const float* latent, const float* out, const float* dout, const float* dlatent,
+                                      float* dx, float* dweight, float* dbias, int32_t B, int32_t H, int32_t W, int32_t C,
+                                      int32_t L, const float* weight, void* workspace, void* stream) {
+    MODFX_REQUIRE(latent && out && dout && dlatent && dx && dweight && dbias && weight && workspace, "NULL pointer");
+    MODFX_REQUIRE(B >= 1 && H >= 1 && W >= 1 && C >= 1 && L >= 1, "bad shape (an empty batch has no gradient)");
+    if (C > 1024 || L > 1024) return fail(MODFX_ERR_UNSUPPORTED, "C=%d / L=%d too large", C, L);
+    MODFX_REQUIRE(B <= 65535, "B too large");
+    const int ntw = (W + kHeadW - 1) / kHeadW;
+    float* part = ws_align(workspace);
+    cudaStream_t s = as_stream(stream);
+    const int st = launch(head_bwd_kernel, dim3(ntw, B), 256, (size_t)(C + L) * (kHeadW + 1) * sizeof(float), s, latent, out,
+                          dout, dlatent, dx, part, H, W, C, L, weight);
+    if (st != MODFX_OK) return st;
+    return sum_parts(part, B * ntw, (int64_t)L * C + L, (int64_t)L * C, dweight, dbias, s);
 }

@@ -180,11 +180,16 @@ struct ConvMaps {
     CUtensorMap w[2];       // weights: hi, lo
 };
 
-template <bool kHalf>
-__global__ void __launch_bounds__(kThreads, 1) conv_tf32_kernel(const __grid_constant__ ConvMaps tm, int n_pass,
-                                                                float* __restrict__ y, int H, int W, int dil,
-                                                                const float* __restrict__ bias,
-                                                                const float* __restrict__ prelu) {
+// Epilogue of the convolution mainloop.  kInfer: y = PReLU(maxpool(conv) + bias).  kTrain: the same y, plus the pooled
+// pre-activation z = maxpool(conv) + bias and a byte per pooled element saying which conv row won (1 = the lower one;
+// a tie goes to the upper row, as torch's max_pool2d routes its gradient).  kRaw: all conv rows as they are, no pool,
+// bias or PReLU -- the data gradient, which is this same convolution run on dConv with flipped, transposed weights.
+enum ConvEpi { kInfer = 0, kTrain = 1, kRaw = 2 };
+
+template <bool kHalf, int kEpi>
+__device__ __forceinline__ void conv_tf32_body(const ConvMaps& tm, int n_pass, float* __restrict__ y, int H, int W, int dil,
+                                               const float* __restrict__ bias, const float* __restrict__ prelu,
+                                               float* __restrict__ z, uint8_t* __restrict__ am) {
     using F = Fmt<kHalf>;
     constexpr int kAStages = F::kAStages, kStageA = F::kStageA, kBytesB = F::kBytesB, kNumBars = F::kNumBars;
     extern __shared__ unsigned char smem_raw[];
@@ -379,8 +384,27 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tf32_kernel(const __grid_con
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         const int q = warp & 3;                                     // the TMEM lane quadrant this warp may read
         const int w = w0 + 32 * q + lane;
+        if constexpr (kEpi == kRaw) {
+            for (int a = 0; a < plan.nrows; ++a) {
+                float* yp = y + (((int64_t)b * H + plan.h0 + a) * W + w) * kC;
+#pragma unroll 1
+                for (int half = 0; half < 2; ++half) {
+                    uint32_t v[32];
+                    tmem_ld32(tmem + ((uint32_t)(32 * q) << 16) + a * kC + 32 * half, v);
+                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                    if (w < W) {
+#pragma unroll
+                        for (int j = 0; j < 32; j += 4)
+                            *reinterpret_cast<float4*>(yp + 32 * half + j) =
+                                make_float4(__uint_as_float(v[j]), __uint_as_float(v[j + 1]), __uint_as_float(v[j + 2]),
+                                            __uint_as_float(v[j + 3]));
+                    }
+                }
+            }
+        } else {
         for (int pr = 0; pr < plan.nrows / 2; ++pr) {
-            float* yp = y + (((int64_t)b * (H / 2) + plan.h0 / 2 + pr) * W + w) * kC;
+            const int64_t pix = ((int64_t)b * (H / 2) + plan.h0 / 2 + pr) * W + w;
+            float* yp = y + pix * kC;
 #pragma unroll 1
             for (int half = 0; half < 2; ++half) {
                 uint32_t up[32], lo[32];
@@ -391,18 +415,27 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tf32_kernel(const __grid_con
                 if (w < W) {
 #pragma unroll
                     for (int j = 0; j < 32; j += 4) {
-                        float o[4];
+                        float o[4], zz[4];
+                        uint32_t sel = 0;
 #pragma unroll
                         for (int i = 0; i < 4; ++i) {
                             const int c = 32 * half + j + i;
                             const float v =
                                 fmaxf(__uint_as_float(up[j + i]), __uint_as_float(lo[j + i])) + __ldg(bias + c);
                             o[i] = v > 0.0f ? v : __ldg(prelu + c) * v;
+                            zz[i] = v;
+                            if constexpr (kEpi == kTrain)
+                                sel |= (__uint_as_float(lo[j + i]) > __uint_as_float(up[j + i]) ? 1u : 0u) << (8 * i);
                         }
                         *reinterpret_cast<float4*>(yp + 32 * half + j) = make_float4(o[0], o[1], o[2], o[3]);
+                        if constexpr (kEpi == kTrain) {
+                            *reinterpret_cast<float4*>(z + pix * kC + 32 * half + j) = make_float4(zz[0], zz[1], zz[2], zz[3]);
+                            *reinterpret_cast<uint32_t*>(am + pix * kC + 32 * half + j) = sel;
+                        }
                     }
                 }
             }
+        }
         }
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     }
@@ -411,6 +444,24 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tf32_kernel(const __grid_con
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(kTmemCols) : "memory");
     }
+}
+
+template <bool kHalf>
+__global__ void __launch_bounds__(kThreads, 1) conv_tf32_kernel(const __grid_constant__ ConvMaps tm, int n_pass,
+                                                                float* __restrict__ y, int H, int W, int dil,
+                                                                const float* __restrict__ bias,
+                                                                const float* __restrict__ prelu) {
+    conv_tf32_body<kHalf, kInfer>(tm, n_pass, y, H, W, dil, bias, prelu, nullptr, nullptr);
+}
+
+// training forward (kTrain) and data gradient (kRaw, bias / prelu unused): TF32, one pass
+template <int kEpi>
+__global__ void __launch_bounds__(kThreads, 1) conv_tf32_grad_kernel(const __grid_constant__ ConvMaps tm,
+                                                                     float* __restrict__ y, int H, int W, int dil,
+                                                                     const float* __restrict__ bias,
+                                                                     const float* __restrict__ prelu,
+                                                                     float* __restrict__ z, uint8_t* __restrict__ am) {
+    conv_tf32_body<false, kEpi>(tm, 1, y, H, W, dil, bias, prelu, z, am);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -433,13 +484,17 @@ constexpr int kThreads1 = 5 * 32;
 constexpr int kTmemCols1 = kRows1 * kC;   // 256
 constexpr int kSmemBytes1 = kStages1 * kTileA1 + kKH * kTileB1 + 1024 + 8 * (2 * kStages1 + 2) + 16;
 
-__global__ void __launch_bounds__(kThreads1, 2) conv1_tf32_kernel(const float* __restrict__ x, float* __restrict__ y,
-                                                                  int H, int W, const float* __restrict__ weight,
-                                                                  const float* __restrict__ bias,
-                                                                  const float* __restrict__ prelu) {
+template <bool kTrainEpi>
+__device__ __forceinline__ void conv1_tf32_body(const float* __restrict__ x, float* __restrict__ y, int H, int W,
+                                                const float* __restrict__ weight, const float* __restrict__ bias,
+                                                const float* __restrict__ prelu, float* __restrict__ z,
+                                                uint8_t* __restrict__ am) {
     extern __shared__ unsigned char smem_raw[];
     const uint32_t raw = smem_u32(smem_raw);
     const uint32_t base = (raw + 1023u) & ~1023u;
+    // the thread range __launch_bounds__ gives the kernel, restated for the inlined body (the compiler's bit analysis
+    // of the swizzled tile addresses depends on it)
+    __builtin_assume(threadIdx.x < kThreads1);
     const uint32_t a_base = base, b_base = base + kStages1 * kTileA1;
     const uint32_t bar_full = b_base + kKH * kTileB1, bar_empty = bar_full + 8 * kStages1;
     const uint32_t bar_b = bar_empty + 8 * kStages1, bar_acc = bar_b + 8;
@@ -537,6 +592,7 @@ __global__ void __launch_bounds__(kThreads1, 2) conv1_tf32_kernel(const float* _
         const int w = w0 + tid;                                     // warp q reads TMEM lanes 32 q .. 32 q + 31
         for (int pr = 0; pr < nrows / 2; ++pr) {
             float* yp = y + (((int64_t)b * (H / 2) + h0 / 2 + pr) * W + w) * kC;
+            const int64_t pix = (yp - y) / kC;
 #pragma unroll 1
             for (int half = 0; half < 2; ++half) {
                 uint32_t up[32], lo[32];
@@ -547,15 +603,23 @@ __global__ void __launch_bounds__(kThreads1, 2) conv1_tf32_kernel(const float* _
                 if (w < W) {
 #pragma unroll
                     for (int j = 0; j < 32; j += 4) {
-                        float o[4];
+                        float o[4], zz[4];
+                        uint32_t sel = 0;
 #pragma unroll
                         for (int i = 0; i < 4; ++i) {
                             const int c = 32 * half + j + i;
                             const float v2 =
                                 fmaxf(__uint_as_float(up[j + i]), __uint_as_float(lo[j + i])) + __ldg(bias + c);
                             o[i] = v2 > 0.0f ? v2 : __ldg(prelu + c) * v2;
+                            zz[i] = v2;
+                            if constexpr (kTrainEpi)
+                                sel |= (__uint_as_float(lo[j + i]) > __uint_as_float(up[j + i]) ? 1u : 0u) << (8 * i);
                         }
                         *reinterpret_cast<float4*>(yp + 32 * half + j) = make_float4(o[0], o[1], o[2], o[3]);
+                        if constexpr (kTrainEpi) {
+                            *reinterpret_cast<float4*>(z + pix * kC + 32 * half + j) = make_float4(zz[0], zz[1], zz[2], zz[3]);
+                            *reinterpret_cast<uint32_t*>(am + pix * kC + 32 * half + j) = sel;
+                        }
                     }
                 }
             }
@@ -606,6 +670,161 @@ __global__ void __launch_bounds__(kThreads1, 2) conv1_tf32_kernel(const float* _
     }
 }
 
+__global__ void __launch_bounds__(kThreads1, 2) conv1_tf32_kernel(const float* __restrict__ x, float* __restrict__ y,
+                                                                  int H, int W, const float* __restrict__ weight,
+                                                                  const float* __restrict__ bias,
+                                                                  const float* __restrict__ prelu) {
+    conv1_tf32_body<false>(x, y, H, W, weight, bias, prelu, nullptr, nullptr);
+}
+
+// training forward of the first layer: y as above, plus z and the pool's argmax (kTrain of the 64-channel kernel)
+__global__ void __launch_bounds__(kThreads1, 2) conv1_tf32_train_kernel(const float* __restrict__ x, float* __restrict__ y,
+                                                                        int H, int W, const float* __restrict__ weight,
+                                                                        const float* __restrict__ bias,
+                                                                        const float* __restrict__ prelu,
+                                                                        float* __restrict__ z, uint8_t* __restrict__ am) {
+    conv1_tf32_body<true>(x, y, H, W, weight, bias, prelu, z, am);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Weight gradient of the 64 -> 64 convolution on tcgen05 (TF32 operands, float32 accumulation in tensor memory):
+//   dW[kh][kw][co][ci] = sum over (b, h, w) of dConv[b, h, w, co] * x[b, h + kh - 2, w + (kw - 6) d, ci].
+// The GEMM runs with K = pixels: one K step is 128 frames of one conv row.  A CTA owns a pair of taps t0 = 2 p,
+// t1 = 2 p + 1 (M = 128 = 2 taps x 64 input channels, from two shifted TMA boxes of x) and N = 64 output channels
+// (the dConv box of the same frames), over one slice of the K steps.  Both boxes are channel-contiguous, i.e. MN-major
+// operands (instruction descriptor bits 15 / 16, valid for kind::tf32).  MN-major TF32 operands take one shared-memory
+// layout only, SWIZZLE_128B_BASE32B (32-byte granules of a 128-byte row swizzled over 4 rows; the TMA unit writes it
+// with CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B): a 128-byte row is 32 channels of one frame, 4 frames are one 512-byte
+// K group (SBO), 8 frames (K = 8, one MMA) are 1024 bytes, and the 32-channel panels of a box lie LBO = 16 KB apart.  Rows and frames outside the image come back zero from the TMA unit (padding="same").
+// Each CTA writes its partial sum to a workspace slice; wgrad_reduce_kernel adds the slices in a fixed order, so the
+// result does not depend on scheduling (no float atomics).
+constexpr int kTaps = kKH * kKW;                      // 65
+constexpr int kWgPairs = (kTaps + 1) / 2;             // 33
+constexpr int kWgPanel = kTileW * 128;                // 16 KB: 128 frames x 32 channels
+constexpr int kWgStage = 6 * kWgPanel;                // x of t0, x of t1 (M), dConv (N): 96 KB
+constexpr int kWgStages = 2;
+constexpr int kWgThreads = 6 * 32;
+constexpr int kWgSmemBytes = kWgStages * kWgStage + 1024 + 8 * (2 * kWgStages + 1) + 16;
+constexpr int kWgSplits = 17;                         // K slices: 33 x 17 = 561 CTAs, 3.8 waves of 148 SMs
+constexpr uint32_t kWgLbo = (uint32_t)(kWgPanel >> 4) << 16;
+constexpr uint32_t kWgDescHi = (512u >> 4) | (1u << 14) | (1u << 29);     // SBO 512, version 1, SWIZZLE_128B_BASE32B
+// D = F32, A = B = TF32, A and B MN-major, N = 64, M = 128
+constexpr uint32_t kWgIdesc = (1u << 4) | (2u << 7) | (2u << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(kC >> 3) << 17) |
+                              ((uint32_t)(kTileW >> 4) << 24);
+
+__global__ void __launch_bounds__(kWgThreads, 1) conv_wgrad_tf32_kernel(const __grid_constant__ CUtensorMap tm_x,
+                                                                        const __grid_constant__ CUtensorMap tm_d,
+                                                                        float* __restrict__ part, int B, int H, int W,
+                                                                        int dil) {
+    extern __shared__ unsigned char smem_raw[];
+    const uint32_t raw = smem_u32(smem_raw);
+    const uint32_t base = (raw + 1023u) & ~1023u;
+    const uint32_t bar_full = base + kWgStages * kWgStage, bar_empty = bar_full + 8 * kWgStages;
+    const uint32_t bar_acc = bar_empty + 8 * kWgStages;
+    volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem_raw + (bar_acc + 8 - raw));
+
+    const int tid = threadIdx.x, lane = tid & 31;
+    const int warp = __shfl_sync(kFull, tid >> 5, 0);
+    const int pair = blockIdx.x, split = blockIdx.y;
+    const int t0 = 2 * pair, t1 = min(2 * pair + 1, kTaps - 1);  // the 66th "tap" repeats the 65th and is not stored
+    const int ntw = (W + kTileW - 1) / kTileW;
+    const int64_t steps = (int64_t)B * H * ntw;
+    const int64_t s0 = steps * split / gridDim.y, s1 = steps * (split + 1) / gridDim.y;
+
+    if (tid == 0) {
+        for (int i = 0; i < kWgStages; ++i) {
+            mbar_init(bar_full + 8 * i, 1);
+            mbar_init(bar_empty + 8 * i, 1);
+        }
+        mbar_init(bar_acc, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == 2) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(bar_acc + 8), "n"(kC)
+                     : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    const uint32_t tmem = __shfl_sync(kFull, *tmem_slot, 0);
+
+    if (warp == 0) {
+        // ===== producer: per K step the two shifted x boxes and the dConv box, two 32-channel panels each =====
+        for (int64_t st = s0; st < s1; ++st) {
+            const int i = (int)(st - s0);
+            const int s = i & (kWgStages - 1);
+            const int tw = (int)(st % ntw);
+            const int64_t bh = st / ntw;
+            const int h = (int)(bh % H), b = (int)(bh / H);
+            const int w0 = tw * kTileW;
+            mbar_wait(bar_empty + 8 * s, (((uint32_t)i / kWgStages) & 1u) ^ 1u);
+            if (elect_one()) {
+                const uint32_t full = bar_full + 8 * s, st_base = base + s * kWgStage;
+                mbar_expect_tx(full, kWgStage);
+#pragma unroll
+                for (int p = 0; p < 2; ++p) {
+                    const int kh0 = t0 / kKW, kw0 = t0 - kh0 * kKW, kh1 = t1 / kKW, kw1 = t1 - kh1 * kKW;
+                    tma_load_4d(st_base + p * kWgPanel, &tm_x, full, 32 * p, w0 + (kw0 - kKW / 2) * dil, h + kh0 - kKH / 2, b);
+                    tma_load_4d(st_base + (2 + p) * kWgPanel, &tm_x, full, 32 * p, w0 + (kw1 - kKW / 2) * dil,
+                                h + kh1 - kKH / 2, b);
+                    tma_load_4d(st_base + (4 + p) * kWgPanel, &tm_d, full, 32 * p, w0, h, b);
+                }
+            }
+            __syncwarp();
+        }
+    } else if (warp == 1) {
+        // ===== MMA issuer: 16 MMAs of K = 8 frames per step, D (128 x 64) in tensor memory =====
+        for (int64_t st = s0; st < s1; ++st) {
+            const int i = (int)(st - s0);
+            const int s = i & (kWgStages - 1);
+            mbar_wait(bar_full + 8 * s, ((uint32_t)i / kWgStages) & 1u);
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            const uint32_t a_lo = (umma_desc_lo(base + s * kWgStage) & 0xFFFFu) | kWgLbo;
+            const uint32_t b_lo = (umma_desc_lo(base + s * kWgStage + 4 * kWgPanel) & 0xFFFFu) | kWgLbo;
+            if (elect_one()) {
+#pragma unroll
+                for (int k = 0; k < kTileW / 8; ++k)
+                    umma_tf32(tmem, ((uint64_t)kWgDescHi << 32) | (a_lo + k * (1024 >> 4)),
+                              ((uint64_t)kWgDescHi << 32) | (b_lo + k * (1024 >> 4)), kWgIdesc,
+                              (i > 0 || k > 0) ? 1u : 0u);
+                umma_commit(bar_empty + 8 * s);
+            }
+            __syncwarp();
+        }
+        if (elect_one()) umma_commit(bar_acc);
+        __syncwarp();
+    } else {
+        // ===== epilogue: lane = row m of D (tap t0 + m / 64, input channel m % 64), 64 output channels; the slice is
+        // stored in the parameter's own layout (Cout, Cin, KH, KW) =====
+        const int q = warp & 3;
+        const int m = 32 * q + lane;
+        const int t = (m < kC) ? t0 : 2 * pair + 1, ci = m & (kC - 1);
+        float* dst = part + (int64_t)split * kC * kC * kTaps + (int64_t)ci * kTaps + t;
+        if (s1 > s0) {
+            mbar_wait(bar_acc, 0);
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        }
+#pragma unroll 1
+        for (int half = 0; half < 2; ++half) {
+            uint32_t v[32];
+            tmem_ld32(tmem + ((uint32_t)(32 * q) << 16) + 32 * half, v);
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            if (t < kTaps) {
+#pragma unroll
+                for (int j = 0; j < 32; ++j)
+                    dst[(int64_t)(32 * half + j) * kC * kTaps] = (s1 > s0) ? __uint_as_float(v[j]) : 0.0f;
+            }
+        }
+        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    }
+    __syncthreads();
+    if (warp == 2) {
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(kC) : "memory");
+    }
+}
+
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
@@ -626,7 +845,7 @@ EncodeTiledFn encode_tiled() {
 }  // namespace
 
 static int make_maps(EncodeTiledFn enc, CUtensorMap* tm_x, CUtensorMap* tm_w, const void* x, const void* weight, int B,
-                     int H, int W, bool half) {
+                     int H, int W, bool half, CUtensorMapSwizzle x_swizzle = CU_TENSOR_MAP_SWIZZLE_128B) {
     const cuuint64_t eb = half ? 2 : 4;                          // bytes per element
     const cuuint32_t row = (cuuint32_t)(128 / eb);               // channels in one 128-byte swizzle row
     const CUtensorMapDataType dt = half ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
@@ -637,7 +856,7 @@ static int make_maps(EncodeTiledFn enc, CUtensorMap* tm_x, CUtensorMap* tm_w, co
         const cuuint32_t box[4] = {row, (cuuint32_t)kTileW, 1, 1};
         const cuuint32_t es[4] = {1, 1, 1, 1};
         const CUresult r = enc(tm_x, dt, 4, const_cast<void*>(x), dims, strides, box, es,
-                               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                               CU_TENSOR_MAP_INTERLEAVE_NONE, x_swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) return fail(MODFX_ERR_CUDA, "cuTensorMapEncodeTiled(activations) failed: %d", (int)r);
     }
@@ -678,6 +897,57 @@ int cnn_conv_tf32(const void* x, const void* x_lo, float* y, int B, int H, int W
         return launch(conv_tf32_kernel<true>, grid, kThreads, Fmt<true>::kSmemBytes, stream, tm, 1, y, H, W, dil, bias, prelu);
     return launch(conv_tf32_kernel<false>, grid, kThreads, Fmt<false>::kSmemBytes, stream, tm, split ? 3 : 1, y, H, W, dil,
                   bias, prelu);
+}
+
+// training forward (z / am != nullptr: kTrain) or data gradient (z == nullptr: kRaw, y is (B, H, W, 64)) of the
+// 64-channel layer, TF32
+int cnn_conv_tf32_grad(const float* x, float* y, float* z, uint8_t* am, int B, int H, int W, int dil, const float* weight,
+                       const float* bias, const float* prelu, cudaStream_t stream) {
+    EncodeTiledFn enc = encode_tiled();
+    if (!enc) return fail(MODFX_ERR_CUDA, "cuTensorMapEncodeTiled is not available from this driver");
+    MODFX_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(weight) & 15) == 0 &&
+                      (reinterpret_cast<uintptr_t>(y) & 15) == 0 && (reinterpret_cast<uintptr_t>(z) & 15) == 0 &&
+                      (reinterpret_cast<uintptr_t>(am) & 3) == 0,
+                  "x, y, z and weight must be 16-byte aligned, argmax 4-byte aligned");
+    ConvMaps tm;
+    int st = make_maps(enc, &tm.x[0], &tm.w[0], x, weight, B, H, W, false);
+    if (st != MODFX_OK) return st;
+    tm.x[1] = tm.x[0];
+    tm.w[1] = tm.w[0];
+    const dim3 grid((W + kTileW - 1) / kTileW, (H + kRows - 1) / kRows, B);
+    if (z) return launch(conv_tf32_grad_kernel<kTrain>, grid, kThreads, Fmt<false>::kSmemBytes, stream, tm, y, H, W, dil, bias,
+                         prelu, z, am);
+    return launch(conv_tf32_grad_kernel<kRaw>, grid, kThreads, Fmt<false>::kSmemBytes, stream, tm, y, H, W, dil, bias, prelu,
+                  z, am);
+}
+
+int cnn_wgrad_splits() { return kWgSplits; }
+
+// part: kWgSplits x (64, 64, 5, 13) floats
+int cnn_conv_wgrad_tf32(const float* x, const float* dconv, float* part, int B, int H, int W, int dil, cudaStream_t stream) {
+    EncodeTiledFn enc = encode_tiled();
+    if (!enc) return fail(MODFX_ERR_CUDA, "cuTensorMapEncodeTiled is not available from this driver");
+    MODFX_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(dconv) & 15) == 0,
+                  "x and dconv must be 16-byte aligned");
+    CUtensorMap tm_x, tm_d, tm_w;
+    int st = make_maps(enc, &tm_x, &tm_w, x, x, B, H, W, false, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
+    if (st != MODFX_OK) return st;
+    st = make_maps(enc, &tm_d, &tm_w, dconv, x, B, H, W, false, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
+    if (st != MODFX_OK) return st;
+    return launch(conv_wgrad_tf32_kernel, dim3(kWgPairs, kWgSplits), kWgThreads, kWgSmemBytes, stream, tm_x, tm_d, part, B, H,
+                  W, dil);
+}
+
+int cnn_conv1_tf32_train(const float* x, float* y, float* z, uint8_t* am, int B, int H, int W, const float* weight,
+                         const float* bias, const float* prelu, cudaStream_t stream) {
+    MODFX_REQUIRE((reinterpret_cast<uintptr_t>(x) & 7) == 0 && (reinterpret_cast<uintptr_t>(weight) & 7) == 0 &&
+                      (reinterpret_cast<uintptr_t>(y) & 15) == 0 && (reinterpret_cast<uintptr_t>(z) & 15) == 0 &&
+                      (reinterpret_cast<uintptr_t>(am) & 3) == 0,
+                  "x and weight must be 8-byte, y and z 16-byte, argmax 4-byte aligned");
+    MODFX_CUDA_OK(cudaFuncSetAttribute(conv1_tf32_train_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                       cudaSharedmemCarveoutMaxShared));
+    return launch(conv1_tf32_train_kernel, dim3((W + kTileW - 1) / kTileW, (H + kRows1 - 1) / kRows1, B), kThreads1,
+                  kSmemBytes1, stream, x, y, H, W, weight, bias, prelu, z, am);
 }
 
 int cnn_conv1_tf32(const float* x, float* y, int B, int H, int W, const float* weight, const float* bias,

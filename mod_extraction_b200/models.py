@@ -13,7 +13,8 @@ and log into the same kernel for inference, where no masking sits in between.
 (sigmoid output, latent)`` and state-dict keys (models.py:127-215): log-mel kernel -> [SpecAugment fill when
 training] -> 6 x {layer norm, 5x13 dilated conv + 2x1 max-pool + PReLU} -> mean over mel -> 1x1 conv -> sigmoid,
 activations channels-last, the 64->64 convolutions on tcgen05 tensor cores (TF32, like cuDNN's default for the
-reference on a GPU) or, with ``precision="fp32"``, on the CUDA cores.  Inference only (no autograd).
+reference on a GPU) or, with ``precision="fp32"``, on the CUDA cores.  With ``precision="tf32"`` the body and head are
+trainable: parameter gradients (cuDNN TF32 training semantics) come from libmodfx's backward kernels.
 """
 from __future__ import annotations
 
@@ -185,7 +186,7 @@ def specaugment_bounds(size: int, mask_param: int) -> Tuple[int, int]:
 
 
 class Spectral2DCNN(nn.Module):
-    """GPU drop-in for ``mod_extraction.models.Spectral2DCNN`` (models.py:127-215), inference only.
+    """GPU drop-in for ``mod_extraction.models.Spectral2DCNN`` (models.py:127-215).
 
     Same constructor arguments, same ``forward(x) -> (x, latent)`` with x (B, in_ch, n_samples) ->
     (B, latent_dim, n_frames) and latent (B, out_channels[-1], n_frames), and the same parameter names, so
@@ -195,6 +196,11 @@ class Spectral2DCNN(nn.Module):
     error-compensated operands: meets the float32 parity bars of the network at a third of the TF32 rate, 6x faster than
     the CUDA-core path) or "fp32" (CUDA cores, exact float32 FMAs).
     Built: kernel_size (5, 13), pool_size (2, 1), 64 channels per layer, bin dilation 1, use_ln=True.
+
+    Training: in train mode, with grad enabled and a parameter that requires grad, ``forward`` / ``forward_features``
+    return outputs attached to the autograd graph (bitwise the no-grad numbers) and ``backward`` fills ``.grad`` of
+    every parameter -- ``precision="tf32"`` only: the other precisions run their forward-only path, whose outputs carry
+    no graph.  No gradient flows to the log-mel or the audio (an input that requires grad raises NotImplementedError).
     """
 
     def __init__(self, in_ch: int = 1, n_samples: int = 88200, sr: float = 44100, n_fft: int = 1024,
@@ -280,14 +286,43 @@ class Spectral2DCNN(nn.Module):
                     w = torch.stack([hi, round_to_tf32(w - hi)])
                 packed.append((w, conv.bias.detach().to(device=device, dtype=torch.float32).contiguous(),
                                act.weight.detach().to(device=device, dtype=torch.float32).contiguous(), mode))
+            # data-gradient weights of the tensor-core layers: w_t[kh][kw][ci][co] = w[4 - kh][12 - kw][co][ci]
+            self._packed_t = [w.flip(0, 1).transpose(2, 3).contiguous() if mode == _lib.CNN_TF32 and w.size(3) == 64 else None
+                              for (w, _, _, mode) in packed]
             w_out = self.output.weight.detach().to(device=device, dtype=torch.float32).reshape(self.latent_dim, -1).contiguous()
             b_out = self.output.bias.detach().to(device=device, dtype=torch.float32).contiguous()
             self._packed, self._packed_key = (packed, w_out, b_out), key
         return self._packed
 
-    @torch.no_grad()
+    def _builds_graph(self, x: Tensor) -> bool:
+        # the backward pass is TF32; other precisions keep their forward-only path, whose outputs carry no graph
+        if not (torch.is_grad_enabled() and self.training and self.precision == "tf32"
+                and any(p.requires_grad for p in self.parameters())):
+            return False
+        if x.requires_grad:
+            raise NotImplementedError("modfx: Spectral2DCNN has no gradient to its input (log-mel / audio)")
+        return True
+
     def forward_features(self, logmel: Tensor) -> Tuple[Tensor, Tensor]:
         """(B, in_ch, n_mels, n_frames) log-mel (clip + log already applied) -> (output, latent)."""
+        if self._builds_graph(logmel):
+            if not logmel.is_cuda:
+                raise RuntimeError("modfx: Spectral2DCNN needs CUDA tensors (no CPU kernel)")
+            outs = [_BodyFunction.apply(self, logmel[i:i + self.max_chunk], *self._grad_params())
+                    for i in range(0, logmel.size(0), self.max_chunk)]
+            if len(outs) == 1:
+                return outs[0]
+            return torch.cat([o[0] for o in outs], 0), torch.cat([o[1] for o in outs], 0)
+        return self._forward_features(logmel)
+
+    def _grad_params(self) -> List[Tensor]:
+        ps = []
+        for i in range(len(self.out_channels)):
+            ps += [self.cnn[4 * i + 1].weight, self.cnn[4 * i + 1].bias, self.cnn[4 * i + 3].weight]
+        return ps + [self.output.weight, self.output.bias]
+
+    @torch.no_grad()
+    def _forward_features(self, logmel: Tensor) -> Tuple[Tensor, Tensor]:
         if not logmel.is_cuda:
             raise RuntimeError("modfx: Spectral2DCNN needs CUDA tensors (no CPU kernel)")
         L = _lib.lib()
@@ -299,7 +334,7 @@ class Spectral2DCNN(nn.Module):
             return (torch.empty((0, self.latent_dim, W), dtype=torch.float32, device=dev),
                     torch.empty((0, self.out_channels[-1], W), dtype=torch.float32, device=dev))
         if B > self.max_chunk:                    # examples are independent: bound the activation memory
-            outs = [self.forward_features(logmel[i:i + self.max_chunk]) for i in range(0, B, self.max_chunk)]
+            outs = [self._forward_features(logmel[i:i + self.max_chunk]) for i in range(0, B, self.max_chunk)]
             return torch.cat([o[0] for o in outs], 0), torch.cat([o[1] for o in outs], 0)
         packed, w_out, b_out = self._pack(dev)
         with torch.cuda.device(dev):
@@ -338,8 +373,89 @@ class Spectral2DCNN(nn.Module):
         return out, latent
 
     @torch.no_grad()
+    def _train_forward(self, logmel: Tensor):
+        """The TF32 forward of one chunk that keeps what the backward needs: per layer the layer-norm input and its
+        statistics, the conv input, z = maxpool(conv) + bias and the pool's argmax."""
+        L = _lib.lib()
+        dev = logmel.device
+        logmel = logmel.detach().float().contiguous()
+        B, C, H, W = logmel.shape
+        assert C == self.in_ch and H == self.n_mels
+        packed, w_out, b_out = self._pack(dev)
+        saves = []
+        with torch.cuda.device(dev):
+            ws = torch.empty(L.modfx_cnn_layernorm_workspace_bytes(B, C, H, W), dtype=torch.uint8, device=dev)
+            x = torch.empty((B, H, W, C), dtype=torch.float32, device=dev)
+            _lib.check(L.modfx_cnn_layernorm_f32(_vp(logmel), _vp(x), B, C, H, W, 1, self.ln_eps, 1, _vp(ws), _stream()))
+            ln_in = stats = None
+            for i, (w, bias, slope, prec) in enumerate(packed):
+                y = torch.empty((B, H // 2, W, 64), dtype=torch.float32, device=dev)
+                z = torch.empty_like(y)
+                am = torch.empty((B, H // 2, W, 64), dtype=torch.uint8, device=dev)
+                _lib.check(L.modfx_cnn_conv_pool_prelu_train_f32(_vp(x), _vp(y), _vp(z), _vp(am), B, H, W, C,
+                                                                 self.temp_dilations[i], _vp(w), _vp(bias), _vp(slope),
+                                                                 _stream()))
+                saves.append((ln_in, stats, x, z, am))
+                H, C = H // 2, 64
+                if i + 1 < len(packed):
+                    ln_in = y
+                    stats = torch.empty(L.modfx_cnn_layernorm_workspace_bytes(B, C, H, W), dtype=torch.uint8, device=dev)
+                    x = torch.empty_like(y)
+                    _lib.check(L.modfx_cnn_layernorm_f32(_vp(y), _vp(x), B, C, H, W, 0, self.ln_eps, 1, _vp(stats),
+                                                        _stream()))
+            latent = torch.empty((B, C, W), dtype=torch.float32, device=dev)
+            out = torch.empty((B, self.latent_dim, W), dtype=torch.float32, device=dev)
+            _lib.check(L.modfx_cnn_head_f32(_vp(y), _vp(latent), _vp(out), B, H, W, C, self.latent_dim, _vp(w_out), _vp(b_out),
+                                           _stream()))
+        return out, latent, saves
+
+    @torch.no_grad()
+    def _backward(self, saves, out: Tensor, latent: Tensor, dout: Tensor, dlatent: Tensor) -> List[Tensor]:
+        """Parameter gradients of one chunk, in the order of ``_grad_params``."""
+        L = _lib.lib()
+        dev = out.device
+        packed, w_out, _ = self._pack(dev)
+        B, C, W = latent.shape
+        n = len(packed)
+        H = self.n_mels >> n
+        grads: List[Optional[Tensor]] = [None] * (3 * n + 2)
+        with torch.cuda.device(dev):
+            ws = torch.empty(L.modfx_cnn_train_workspace_bytes(B, self.n_mels, W, self.latent_dim), dtype=torch.uint8,
+                             device=dev)
+            dy = torch.empty((B, H, W, C), dtype=torch.float32, device=dev)
+            dw_out = torch.empty((self.latent_dim, C), dtype=torch.float32, device=dev)
+            db_out = torch.empty((self.latent_dim,), dtype=torch.float32, device=dev)
+            _lib.check(L.modfx_cnn_head_bwd_f32(_vp(latent), _vp(out), _vp(dout), _vp(dlatent), _vp(dy), _vp(dw_out),
+                                               _vp(db_out), B, H, W, C, self.latent_dim, _vp(w_out), _vp(ws), _stream()))
+            grads[3 * n] = dw_out.view_as(self.output.weight)
+            grads[3 * n + 1] = db_out
+            for i in range(n - 1, -1, -1):
+                ln_in, stats, x, z, am = saves[i]
+                slope = packed[i][2]
+                H *= 2
+                cin = x.size(3)
+                dconv = torch.empty((B, H, W, 64), dtype=torch.float32, device=dev)
+                dbias = torch.empty(64, dtype=torch.float32, device=dev)
+                dslope = torch.empty(64, dtype=torch.float32, device=dev)
+                _lib.check(L.modfx_cnn_pool_prelu_bwd_f32(_vp(dy), _vp(z), _vp(am), _vp(slope), _vp(dconv), _vp(dbias),
+                                                         _vp(dslope), B, H, W, _vp(ws), _stream()))
+                dw = torch.empty((64, cin, 5, 13), dtype=torch.float32, device=dev)
+                _lib.check(L.modfx_cnn_conv_wgrad_tf32_f32(_vp(x), _vp(dconv), _vp(dw), B, H, W, cin, self.temp_dilations[i],
+                                                          _vp(ws), _stream()))
+                grads[3 * i:3 * i + 3] = [dw, dbias, dslope]
+                if i > 0:
+                    g = torch.empty((B, H, W, 64), dtype=torch.float32, device=dev)
+                    _lib.check(L.modfx_cnn_conv_dgrad_tf32_f32(_vp(dconv), _vp(g), B, H, W, self.temp_dilations[i],
+                                                              _vp(self._packed_t[i]), _stream()))
+                    dy = torch.empty_like(ln_in)
+                    _lib.check(L.modfx_cnn_layernorm_bwd_f32(_vp(g), _vp(ln_in), _vp(stats), _vp(dy), B, 64, H, W,
+                                                            self.ln_eps, _vp(ws), _stream()))
+        return grads
+
     def forward(self, x: Tensor) -> Tuple[Tensor, Tensor]:
         assert x.ndim == 3
+        if x.requires_grad and self._builds_graph(x):
+            raise NotImplementedError("modfx: Spectral2DCNN has no gradient to its input (log-mel / audio)")
         logmel = self.spectrogram(x)                               # models.py:199,207-208 fused
         if self.training:                                          # models.py:201-205
             f0 = f1 = t0 = t1 = 0
@@ -352,6 +468,25 @@ class Spectral2DCNN(nn.Module):
                     _vp(logmel), logmel.size(0) * logmel.size(1), logmel.size(-2), logmel.size(-1), f0, f1, t0, t1,
                     float(self.eps), 1, _stream()))
         return self.forward_features(logmel)
+
+
+class _BodyFunction(torch.autograd.Function):
+    """Body + head of Spectral2DCNN for one chunk of examples: the forward keeps its saves, the backward returns the
+    parameter gradients (none to the log-mel, which is data)."""
+
+    @staticmethod
+    def forward(ctx, net: "Spectral2DCNN", logmel: Tensor, *params: Tensor):
+        out, latent, saves = net._train_forward(logmel)
+        ctx.net, ctx.saves = net, saves
+        ctx.save_for_backward(out, latent)
+        return out, latent
+
+    @staticmethod
+    def backward(ctx, dout: Tensor, dlatent: Tensor):
+        out, latent = ctx.saved_tensors
+        grads = ctx.net._backward(ctx.saves, out, latent, dout.float().contiguous(), dlatent.float().contiguous())
+        ctx.saves = None
+        return (None, None) + tuple(grads)
 
 
 class RandomLFO(nn.Module):
