@@ -1,7 +1,8 @@
 """GPU tests of the Spectral2DCNN backward pass (TF32, parameter gradients): the gradient kernels against float64
 references, and the trainable module against torch float64 autograd and cuDNN TF32 training of its own containers.
 
-Bounds (relative L2 error per tensor) were set from a B200 run with about 2x head-room; see each test's docstring."""
+Bounds (relative L2 error per tensor) were set from a B200 run with about 2x head-room, see each test's docstring; the
+elementwise bounds of check_conv_grads with about 4x."""
 import copy
 import ctypes
 
@@ -33,8 +34,45 @@ def rel(a, b):
     return float((a - b).norm() / b.norm().clamp_min(1e-300))
 
 
-def make_net(seed=3, max_chunk=256):
-    net = Spectral2DCNN(in_ch=2, n_samples=N_SAMPLES, n_mels=N_MELS, out_channels=[64] * 6, temp_dilations=CNN_DILATIONS,
+def bounded(name, lib, ref, mag, c):
+    """Asserts |lib - ref| <= c * mag elementwise (ref, mag float64; an unwritten NaN fails) and prints the worst
+    |lib - ref| / mag."""
+    err = (lib.double() - ref).abs()
+    assert bool(torch.isfinite(err).all()), (name, "non-finite output")
+    worst = float((err / mag.clamp_min(1e-300)).max())
+    print(f"{name}: max |lib - ref| / M = {worst:.2e} (bound {c:.1e})")
+    assert bool((err <= c * mag).all()), (name, worst, c)
+
+
+# Elementwise bounds of the tensor-core convolution gradients, in units of the float64 magnitude (the same operation
+# on |operands|), about 4x the worst |lib - ref| / M measured on a B200 over test_cnn_backward_gpu.py and
+# test_cnn_backward_stages_gpu.py (2^-24 = 6.0e-8).
+C_DGRAD = 1e-5      # measured max 2.3e-6 (38 x 2^-24: K = 4160 products, tensor-core accumulation)
+C_WGRAD = 1.6e-6    # measured max 4.1e-7
+C_WGRAD1 = 5e-7     # layer 0 (CUDA cores); measured max 1.1e-7
+
+
+def check_conv_grads(x, dconv, w, dil, dx, dw):
+    """dgrad `dx` (None: not checked) and wgrad `dw` (co, ci, kh, kw) of the 'same' convolution of channels-last x
+    (B, H, W, Cin) with w (co, ci, kh, kw) against float64 autograd of the same TF32 operands, elementwise.  Without
+    dx, only the weight gradient is formed, and w (which it does not depend on) may be None."""
+    if w is None:
+        w = torch.zeros(64, x.size(3), 5, 13, device=x.device)
+
+    def grads(xx, dd, ww):
+        x64 = xx.permute(0, 3, 1, 2).double().requires_grad_(dx is not None)
+        w64 = ww.double().requires_grad_(True)
+        (F.conv2d(x64, w64, dilation=(1, dil), padding="same") * dd.permute(0, 3, 1, 2).double()).sum().backward()
+        return x64.grad, w64.grad
+    rx, rw = grads(x, dconv, w)
+    mx, mw = grads(x.abs(), dconv.abs(), w.abs())
+    if dx is not None:
+        bounded(f"dgrad dil {dil}", dx, rx.permute(0, 2, 3, 1), mx.permute(0, 2, 3, 1), C_DGRAD)
+    bounded(f"wgrad Cin {x.size(3)} dil {dil}", dw, rw, mw, C_WGRAD if x.size(3) == 64 else C_WGRAD1)
+
+
+def make_net(seed=3, max_chunk=256, n_mels=N_MELS, n_samples=N_SAMPLES):
+    net = Spectral2DCNN(in_ch=2, n_samples=n_samples, n_mels=n_mels, out_channels=[64] * 6, temp_dilations=CNN_DILATIONS,
                         pool_size=(2, 1), precision="tf32", max_chunk=max_chunk)
     net.load_state_dict({k: torch.from_numpy(v) for k, v in cnn_weights(seed).items()}, strict=False)
     return net.cuda().train()
@@ -169,21 +207,25 @@ def test_it_trains():
 
 
 @pytest.mark.parametrize("dil", [1, 2, 4, 8, 16])
-@pytest.mark.parametrize("B,H,W", [(1, 2, 200), (2, 8, 130), (3, 16, 345)])
+@pytest.mark.parametrize("B,H,W", [(1, 2, 200), (2, 8, 130), (3, 16, 345), (1, 6, 1), (1, 12, 127), (1, 20, 128),
+                                   (17, 6, 1), (3, 12, 129), (2, 20, 257)])
 def test_dgrad_and_wgrad_kernels_against_float64(dil, B, H, W):
     """dgrad (tensor-core conv with flipped weights) and wgrad (tcgen05, MN-major operands) against float64
-    transposed convolution / correlation of the same TF32 operands.  Bound: relative L2 <= 1e-5 (the operands are
-    exact in TF32, only the float32 accumulation differs)."""
+    transposed convolution / correlation of the same TF32 operands.  Bounds: relative L2 <= 1e-5 (the operands are
+    exact in TF32, only the float32 accumulation differs), and elementwise check_conv_grads.
+    Heights 6, 12 and 20 end in a partial 8-row tile of 6 or 4 rows.  The wgrad K steps B * H * ceil(W / 128) are 6 and
+    12 (fewer than the 17 K slices: empty slices), 102 = 6 * 17, and 20, 72, 120 (uneven slices); H is even, so exactly
+    17 cannot occur."""
     L = _lib.lib()
     g = torch.Generator(device="cpu").manual_seed(B * 100 + H + dil)
     x = round_to_tf32(torch.randn(B, H, W, 64, generator=g)).cuda()
     d = round_to_tf32(torch.randn(B, H, W, 64, generator=g)).cuda()
     w = round_to_tf32(torch.randn(64, 64, 5, 13, generator=g) * 0.05).cuda()            # (co, ci, kh, kw)
     wt = w.permute(2, 3, 0, 1).flip(0, 1).transpose(2, 3).contiguous()                  # [kh][kw][ci][co] flipped
-    dx = torch.empty_like(x)
+    dx = torch.full_like(x, float("nan"))
     _lib.check(L.modfx_cnn_conv_dgrad_tf32_f32(_vp(d), _vp(dx), B, H, W, dil, _vp(wt), _s()))
     ws = torch.empty(L.modfx_cnn_train_workspace_bytes(B, H, W, 1), dtype=torch.uint8, device="cuda")
-    dw = torch.empty(64, 64, 5, 13, device="cuda")
+    dw = torch.full((64, 64, 5, 13), float("nan"), device="cuda")
     _lib.check(L.modfx_cnn_conv_wgrad_tf32_f32(_vp(x), _vp(d), _vp(dw), B, H, W, 64, dil, _vp(ws), _s()))
     x64, d64, w64 = (t.double() for t in (x.permute(0, 3, 1, 2), d.permute(0, 3, 1, 2), w))
     x64.requires_grad_(True)
@@ -192,6 +234,7 @@ def test_dgrad_and_wgrad_kernels_against_float64(dil, B, H, W):
     (y * d64).sum().backward()
     assert rel(dx.permute(0, 3, 1, 2), x64.grad) <= 1e-5
     assert rel(dw, w64.grad) <= 1e-5
+    check_conv_grads(x, d, w, dil, dx, dw)
 
 
 def test_wgrad_first_layer_and_pool_prelu_ties():
@@ -208,26 +251,27 @@ def test_wgrad_first_layer_and_pool_prelu_ties():
     (F.conv2d(x.permute(0, 3, 1, 2).double(), w64, padding="same") * d.permute(0, 3, 1, 2).double()).sum().backward()
     assert rel(dw, w64.grad) <= 1e-5
 
-    # training forward on a constant input: every pooled pair is an exact tie -> argmax 0 (upper row), and the
-    # backward puts the whole gradient on the upper row
-    xin = torch.zeros(1, 4, 8, 64, device="cuda")
-    w = torch.full((5, 13, 64, 64), 0.0, device="cuda")
-    bias = torch.linspace(-1, 1, 64, device="cuda")
-    slope = torch.full((64,), 0.25, device="cuda")
-    y, z = torch.empty(1, 2, 8, 64, device="cuda"), torch.empty(1, 2, 8, 64, device="cuda")
-    am = torch.empty(1, 2, 8, 64, dtype=torch.uint8, device="cuda")
-    _lib.check(L.modfx_cnn_conv_pool_prelu_train_f32(_vp(xin), _vp(y), _vp(z), _vp(am), 1, 4, 8, 64, 1, _vp(w), _vp(bias),
-                                                     _vp(slope), _s()))
-    assert int(am.sum()) == 0 and torch.equal(z, bias.expand_as(z))
-    dy = torch.ones_like(y)
-    dconv = torch.empty(1, 4, 8, 64, device="cuda")
-    db, ds = torch.empty(64, device="cuda"), torch.empty(64, device="cuda")
-    _lib.check(L.modfx_cnn_pool_prelu_bwd_f32(_vp(dy), _vp(z), _vp(am), _vp(slope), _vp(dconv), _vp(db), _vp(ds), 1, 4, 8,
-                                              _vp(ws), _s()))
-    assert torch.all(dconv[:, 1::2] == 0) and torch.all(dconv[:, 0::2] != 0)
-    zz = bias.double()
-    assert torch.allclose(db.double(), torch.where(zz > 0, 1.0, 0.25).double() * 16, rtol=1e-6)
-    assert torch.allclose(ds.double(), torch.where(zz > 0, 0.0, zz) * 16, rtol=1e-5, atol=1e-6)
+    # training forward on a constant input, both kernels (64 channels; 2 channels at dilation 1): every pooled pair is an
+    # exact tie -> argmax 0 (upper row), and the backward puts the whole gradient on the upper row
+    for cin in (64, 2):
+        xin = torch.zeros(1, 4, 8, cin, device="cuda")
+        w = torch.full((5, 13, 64, cin), 0.0, device="cuda")
+        bias = torch.linspace(-1, 1, 64, device="cuda")
+        slope = torch.full((64,), 0.25, device="cuda")
+        y, z = torch.empty(1, 2, 8, 64, device="cuda"), torch.empty(1, 2, 8, 64, device="cuda")
+        am = torch.full((1, 2, 8, 64), 255, dtype=torch.uint8, device="cuda")
+        _lib.check(L.modfx_cnn_conv_pool_prelu_train_f32(_vp(xin), _vp(y), _vp(z), _vp(am), 1, 4, 8, cin, 1, _vp(w),
+                                                         _vp(bias), _vp(slope), _s()))
+        assert int(am.sum()) == 0 and torch.equal(z, bias.expand_as(z)), cin
+        dy = torch.ones_like(y)
+        dconv = torch.empty(1, 4, 8, 64, device="cuda")
+        db, ds = torch.empty(64, device="cuda"), torch.empty(64, device="cuda")
+        _lib.check(L.modfx_cnn_pool_prelu_bwd_f32(_vp(dy), _vp(z), _vp(am), _vp(slope), _vp(dconv), _vp(db), _vp(ds), 1, 4,
+                                                  8, _vp(ws), _s()))
+        assert torch.all(dconv[:, 1::2] == 0) and torch.all(dconv[:, 0::2] != 0)
+        zz = bias.double()
+        assert torch.allclose(db.double(), torch.where(zz > 0, 1.0, 0.25).double() * 16, rtol=1e-6)
+        assert torch.allclose(ds.double(), torch.where(zz > 0, 0.0, zz) * 16, rtol=1e-5, atol=1e-6)
 
 
 def test_layernorm_and_head_backward_against_float64():
